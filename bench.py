@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path of the physics layer on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--dtype f64]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--dtype f64] [--dump-outputs DIR]
     python bench.py --impl reference ...          # the reference's CPU arithmetic (oracle port), host cores
 
 A "step" is one pass of the physics layer over one batch of synthetic log-normal fields (SURVEY.md section 8d):
@@ -72,7 +72,15 @@ def parse():
                     help="SMs the VO kernel leaves to the ROM kernels of the overlapped step (-1 = calibrate during warm-up)")
     ap.add_argument("--log-input", action="store_true", help="VO residual from the log-field (exp inside the kernel) in the step")
     ap.add_argument("--e2e-chunks", type=int, default=4)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (u, dL/dlogX, VO residual of rank 0's "
+                         "batch) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "b200" or args.workload == "cfg5"):
+        ap.error("--dump-outputs writes the outputs of the physics-layer step: --impl b200, workloads cfg1 - cfg4")
+    return args
 
 
 def workload_config(w):
@@ -165,14 +173,10 @@ def run_reference(args):
     ref = CpuReference(full, n)
     for _ in range(max(3, args.warmup)):      # the first calls pay torch's thread-pool start-up (2 s, 0.6 s, 0.04 s measured)
         ref.step()
-    steps, acc, acc_c, acc_v = 0, 0.0, 0.0, 0.0
-    t0 = time.perf_counter()
-    for _ in range(max(1, args.steps)):
+    steps, acc, acc_c, acc_v = args.steps, 0.0, 0.0, 0.0
+    for _ in range(steps):
         c, v = ref.cgm(), ref.vo_cached_gamma()
         acc += c + v; acc_c += c; acc_v += v
-        steps += 1
-        if time.perf_counter() - t0 > 120.0:
-            break
     value = steps * ref.n / acc
     t_asm = ref.vo_assemble(min(ref.n, 32))
     t_vec = ref.vo_vectorised()
@@ -424,6 +428,25 @@ def device_inputs(torch, dev, w, B, tdt, seed):
              y=(torch.tensor(w.y[0], device=dev).expand(B, -1) + 0.01 * rn(B, w.d)).to(tdt),
              g=torch.tensor(w.g_fom[0], device=dev, dtype=tdt), V=torch.tensor(w.V, device=dev, dtype=tdt))
     return d
+
+
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each array of ``outputs`` (name -> [B, ...] device tensor) as out_dir/<name>.npy in its own float dtype.  Above
+    DUMP_MAX_BYTES in all, every array keeps the same fixed, seeded sample of batch rows (in increasing order)."""
+    import numpy as np
+    arrays = {k: t.detach().cpu().numpy() for k, t in outputs.items()}
+    B = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    if B * row_bytes > DUMP_MAX_BYTES:
+        keep = (DUMP_MAX_BYTES - 4096) // row_bytes         # 4096: room for the .npy headers
+        rows = np.sort(np.random.RandomState(0).choice(B, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def nonzero_tile_fraction(w):
@@ -698,9 +721,9 @@ def run_b200(args):
     elif not args.no_overlap and not args.no_graph:
         reserve_ms = calibrate_sm_reserve(torch, hp, max(10, min(K, 30)), [0, 8, 11, 16, 20])
     if args.no_graph:
-        run, mode = (lambda: hp.step(overlap=not args.no_overlap)), "eager"
+        run, keep, mode = (lambda: hp.step(overlap=not args.no_overlap)), None, "eager"
     else:
-        _, _, run, mode = graph_timed(torch, lambda: hp.step(overlap=not args.no_overlap), 3)
+        _, keep, run, mode = graph_timed(torch, lambda: hp.step(overlap=not args.no_overlap), 3)
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
@@ -708,11 +731,14 @@ def run_b200(args):
     t_wall0 = time.perf_counter()
     start.record()
     for k in range(K):
-        run()
+        out = run()      # eager: the step's (u, dL/dlogX, r); a graph replay returns None and refills ``keep``
     end.record()
     torch.cuda.synchronize()
     t_wall1 = time.perf_counter()
     hp.rom.check()
+    if args.dump_outputs is not None and rank == 0:
+        u, gX, r = keep if out is None else out
+        dump_outputs(args.dump_outputs, {"u": u, "grad_logX": gX, "vo_residual": r})
     elapsed_ms = start.elapsed_time(end)
     if world > 1:
         tt = torch.tensor([elapsed_ms], dtype=torch.float64, device=dev)

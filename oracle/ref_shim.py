@@ -1,9 +1,8 @@
 """ORACLE (test infrastructure): import the UNMODIFIED reference hot-path classes from
 /root/reference in this container, with FEniCS/PETSc/matplotlib replaced by empty stand-ins.
 
-Used only by tests/golden/make_golden.py (fixture generation, run in the build container)
-and by tests that skip when /root/reference is absent (it does not exist on the GPU box).
-Nothing under generative-physics-informed-pde_b200/ imports this.
+Used only by tests/golden/make_golden.py, which regenerates the golden fixtures the tests
+compare against.  No test and nothing under generative-physics-informed-pde_b200/ imports this.
 
 Recipe = SURVEY.md Appendix B: the classes on the hot path (bottleneck/ROM.py,
 bottleneck/components.py:260-323, bottleneck/VirtualObservables.py) are pure

@@ -3,10 +3,9 @@
 QuerryPointEnsemble / QuerryEnsemble / VirtualObservablesEnsemble of this package, running the sm_100a kernels -- reproduces
 the value and all parameter gradients that the UNMODIFIED reference classes produced (tests/golden/elbo_4x4_16_ndp.npz).
 
-The reference tree does not exist on the GPU box and its sources may not be copied, so the caller's code is the restatement in
-oracle/elbo_ref.py; tests/test_oracle_golden.py::test_elbo_restatement_matches_reference_generative_model pins that
-restatement to the real GenerativeModel on the CPU with the same fixture.  When a reference tree IS present next to a GPU
-(GPDE_REFERENCE_ROOT), the last test runs the real bottleneck/generative.py on the mirrors."""
+The reference's sources are not part of this repository, so the caller's code is the restatement in oracle/elbo_ref.py;
+tests/test_oracle_golden.py::test_elbo_restatement_matches_reference_generative_model pins that restatement to the values the
+real GenerativeModel stored in the same fixture."""
 import numpy as np
 import pytest
 import torch
@@ -129,42 +128,3 @@ def test_predictive_moments_match_their_definition_and_the_sampled_estimator(dev
         ys = torch.stack([g.propagate_samples(eff[n], F[n].expand(S, -1)) for n in range(N)])
         assert (ys.mean(dim=1) - y_mean).abs().max() < 6 * (y_std / np.sqrt(S)).max()
         assert ((ys.std(dim=1) / y_std) - 1).abs().max() < 0.35
-
-
-def test_real_reference_generative_model_on_the_mirrors_when_available(dev):
-    """Only where a reference tree and a GPU meet (neither the build container nor the GPU box today)."""
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference tree not present on this machine")
-    import importlib
-    ref_shim.load()
-    gen = importlib.import_module("bottleneck.generative")
-    comp = importlib.import_module("bottleneck.components")
-    from oracle import elbo_ref
-    G = load_golden(elbo_fixture.NAME)
-    ph, g, ens = _mirrors(G, torch.double, dev)
-    dim_latent = int(G['dim_latent'])
-    T = lambda a: torch.tensor(a, dtype=torch.double, device=dev)
-    f = elbo_ref.TinyDecoder(dim_latent, G['in_sup_img'][0].size, torch.double, dev)
-    gp = comp.EffectivePropertyMap(dim_latent, g.dim_in, num_hidden_layers=0, independent_X=True, dtype=torch.double, device=dev)
-    model = gen.GenerativeModel(f=f, g=g, gp=gp, dtype=torch.double, device=dev)
-
-    class DS(object):
-        def __init__(self, **t):
-            self._t, self.N = t, next(iter(t.values())).shape[0]
-
-        def get(self, key, random_subset=None):
-            return self._t[key]
-
-    Ns, Nvo = G['in_sup_img'].shape[0], G['in_vo_img'].shape[0]
-    model.register_datasets(dict(supervised=DS(X=T(G['in_sup_img'].reshape(Ns, -1)), Y=T(G['in_sup_Y']), F_ROM_BC=T(G['in_sup_F'])),
-                                 vo=DS(X=T(G['in_vo_img'].reshape(Nvo, -1)), F_ROM_BC=T(G['in_vo_F']))), VO=ens)
-    model.to(dev)
-    params = elbo_ref.named_parameters(f, gp, g, model.q_z, model.q_X)
-    with torch.no_grad():
-        for k, p in params.items():
-            p.copy_(T(G['init_' + k]))
-    with elbo_ref.NoiseTape([G['noise_%d' % i] for i in range(int(G['n_noise']))]):
-        value = model.elbo(step=0)
-    value.backward()
-    elbo_fixture.compare_with_reference(value.item(), {k: p.grad.cpu().numpy() for k, p in params.items()}, G, 1e-9)
