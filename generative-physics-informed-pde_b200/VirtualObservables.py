@@ -237,6 +237,32 @@ class VoPlan(object):
         _lib.check(rc, "gpde_vo_moments_f64")
         return out_r, out_s2
 
+    def energy_step(self, a, V, rho, g, prec, inv_T, mean, info=None):
+        """One subspace-Newton step of the energy-type virtual observables for N data points in ONE launch, matrix-free
+        (gpde_vo_energy_step_f64), in place on ``mean`` [N,d] (contiguous float64 on this device):
+            mean_n <- mean_n - V_n M_n^-1 V_n^T (prec_n (mean_n - g_n) + inv_T[n] rho_n),
+            M_n = V_n^T diag(prec_n) V_n + inv_T[n] V_n^T K_ff(a_n) V_n.
+        a: conductivities [N,n_inputs] (or one shared field), V [d,m] or [N,d,m] (m <= 64), rho [N,d] = K_ff(a_n) mean_n
+        - f_eff (``residual(a, mean, g_bc, None)`` minus the load), g, prec [N,d], inv_T [N].  A data point whose M_n has a
+        non-positive pivot keeps its mean and sets GPDE_INFO_NOT_SPD in ``info``.  Returns ``mean``."""
+        dev = self.device
+        if not (mean.dtype == torch.float64 and mean.dim() == 2 and mean.is_contiguous()):
+            raise ValueError("energy_step updates mean in place: it must be a contiguous float64 [N,d] tensor")
+        N = int(mean.shape[0])
+        a = a.to(torch.float64).contiguous()
+        V, v_stride, m = self._weights_arg(V)
+        rho, g, prec = (t.to(torch.float64).contiguous() for t in (rho, g, prec))
+        inv_T = torch.as_tensor(inv_T, dtype=torch.float64, device=dev).contiguous()
+        if any(t.shape != mean.shape for t in (rho, g, prec)) or mean.shape[1] != self.d or inv_T.shape != (N,) or \
+                (a.dim() == 2 and a.shape[0] != N) or (v_stride and V.shape[0] != N):
+            raise ValueError("energy_step: inconsistent shapes")
+        rc = self._lib.gpde_vo_energy_step_f64(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0,
+                                               _lib.ptr(V, dev), v_stride, m, _lib.ptr(rho, dev), _lib.ptr(g, dev),
+                                               _lib.ptr(prec, dev), _lib.ptr(inv_T, dev), _lib.ptr(mean, dev),
+                                               _lib.ptr(info, dev), N, _lib.stream_of(dev))
+        _lib.check(rc, "gpde_vo_energy_step_f64")
+        return mean
+
 
 class PackedWeights(object):
     """V [d,m] together with its fragment-packed copy (VoPlan.pack_weights); accepted wherever residual() takes V."""
@@ -392,6 +418,15 @@ class BaseSampler(object):
     def sample_V(self):
         return self._sample()
 
+    def sample_V_batch(self, count):
+        """[count, d, m]: ``count`` successive sample_V() draws, stacked in draw order (a numpy array when every draw is
+        one, else a float64 tensor on the draws' device)."""
+        Vs = [self.sample_V() for _ in range(count)]
+        if all(isinstance(v, np.ndarray) for v in Vs):
+            return np.stack(Vs)
+        device = next(v.device for v in Vs if isinstance(v, torch.Tensor))
+        return torch.stack([_as_f64(v, device) for v in Vs])
+
     def sample(self):
         return self.qp.weak_galerkin_on_device(self._sample())
 
@@ -424,11 +459,24 @@ class RadialBasisFunctionSampler(BaseSampler):
         if device is None or torch.device(device).type != "cuda":
             return fem.rbf_weighting(self.qp.physics.mesh, self._rows, centres, self._l)
         # ... evaluated at the fine free nodes on the device (resample() runs at every VO update)
+        return self._evaluate_on_device(centres, device)
+
+    def _evaluate_on_device(self, centres, device):
+        """V [..., d, m] of centres [..., m, 2]."""
         if self._xy_dev is None:
             self._xy_dev = _as_f64(self.qp.physics.mesh.coords[self._rows], device)
         c = _as_f64(centres, device)
-        d2 = (self._xy_dev[:, None, :] - c[None, :, :]).pow(2).sum(-1)
+        d2 = (self._xy_dev[:, None, :] - c[..., None, :, :]).pow(2).sum(-1)
         return torch.exp(-d2 / self._l ** 2)
+
+    def sample_V_batch(self, count):
+        # one vector draw: numpy's legacy RandomState yields the same doubles as the 2 m count scalar draws of count
+        # sample_V() calls, in the same order
+        centres = np.random.uniform(size=(count, self.m, 2))
+        device = self.qp._device
+        if device is None or torch.device(device).type != "cuda":
+            return np.stack([fem.rbf_weighting(self.qp.physics.mesh, self._rows, c, self._l) for c in centres])
+        return self._evaluate_on_device(centres, device)
 
 
 class GaussianSketchingSampler(BaseSampler):
@@ -1071,13 +1119,120 @@ class EnergyVirtualObservable(BaseVirtualObservable):
         return 'Energy virtual Observable | Current temperature = {}'.format(self._temperature)
 
 
+class _ReplaySampler(BaseSampler):
+    """Hands out weighting matrices that were drawn earlier, in their order."""
+
+    def __init__(self, qp, Vs):
+        super().__init__(qp)
+        self._Vs = iter(Vs)
+
+    def _sample(self):
+        return next(self._Vs)
+
+
 class EnergyVirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
-    """VirtualObservables.py:1001-1037."""
+    """VirtualObservables.py:1001-1037 with the loop over the data points replaced by launches over all of them:
+
+      update   per Newton iteration: rho(mean) of all data points (one residual launch) -> gpde_vo_energy_step_f64
+               (one launch); the reference: N x n_it x [dense V^T A V, V^T (A mean - b), solve]
+
+    The weighting matrices are drawn in the member loop's order (data point-major, iteration-minor), with one
+    ``sample_V_batch`` call when the data points share one sampler, so both routes see the same draws.  The member loop
+    (``EnergyVirtualObservable.update`` per data point) runs instead when ``batched_update`` is False, when the drawn m
+    exceeds ``max_kernel_m``, or when the members differ in iterations per update or physics; ``last_update_route`` says
+    which route the last update took ("batched" or "members")."""
+
+    batched_update = True
+    max_kernel_m = 64
+    # per-chunk budget for the drawn weighting matrices V [n, n_it, d, m] of the batched route
+    max_stack_bytes = 1 << 30
 
     def __init__(self, QuerryPointEnsemble, num_iterations_per_update, sampler, dtype, device):
         vos = [EnergyVirtualObservable(qp, num_iterations_per_update, sampler=sampler, dtype=dtype, device=device)
                for qp in QuerryPointEnsemble]
         super().__init__(QuerryPointEnsemble, vos, dtype=dtype, device=device)
+        self._resident = None
+        self._info = None
+        self.last_update_route = None
+
+    def _inputs(self):
+        """(plan, conductivities a [N,n_inputs], Dirichlet values [N,n_bc], diag(K) [N,d], free load [N,d] or None) of
+        all data points, stacked once from the members: their fields, boundary data and diag(K) never change."""
+        if self._resident is None:
+            vos = self._virtual_observables
+            loads = [vo._load_free for vo in vos]
+            load = None
+            if any(f is not None for f in loads):
+                load = torch.stack([f if f is not None else torch.zeros_like(vo._K_diag) for f, vo in zip(loads, vos)])
+            self._resident = (vos[0]._plan, torch.exp(torch.stack([vo._x for vo in vos])),
+                              torch.stack([vo._g_bc for vo in vos]), torch.stack([vo._K_diag for vo in vos]), load)
+        return self._resident
+
+    def _draw(self, chunk, n_it):
+        """V [n, n_it, d, m] of the data points of ``chunk`` in the member loop's order."""
+        s = chunk[0]._sampler
+        if all(vo._sampler is s for vo in chunk):
+            V = _as_f64(s.sample_V_batch(len(chunk) * n_it), self.device)
+        else:
+            V = torch.cat([_as_f64(vo._sampler.sample_V_batch(n_it), self.device) for vo in chunk])
+        return V.view(len(chunk), n_it, *V.shape[1:])
+
+    def _update_members(self, G, PREC, iteration):
+        for n, vo in enumerate(self._virtual_observables):
+            vo.update(G[n, :], PREC[n, :], iteration, ForceUpdate=True)
+        self.flush_cache()
+        self.last_update_route = "members"
+
+    @torch.no_grad()
+    def update(self, G, PREC, iteration, writer=None):
+        self.update_vo_precision(iteration, writer)
+        vos = self._virtual_observables
+        v0 = vos[0]
+        n_it = v0._num_iterations_per_update
+        m_known = [getattr(vo._sampler, "m", None) for vo in vos]
+        if not self.batched_update or any(vo._num_iterations_per_update != n_it or vo._plan is not v0._plan for vo in vos) \
+                or any(m is not None and m > self.max_kernel_m for m in m_known):
+            return self._update_members(G, PREC, iteration)
+        plan, a, gbc, K_diag, load = self._inputs()
+        G64, P64 = _as_f64(G, self.device), _as_f64(PREC, self.device)
+        inv_T = torch.tensor([1.0 / vo.temperature for vo in vos], dtype=_F64, device=self.device)
+        vars_ = 1.0 / (P64 + inv_T.unsqueeze(1) * K_diag)           # the member's expression, row by row
+        mean = torch.stack([vo._mean if vo._mean is not None else torch.zeros_like(vo._K_diag) for vo in vos])
+        if self._info is None:
+            self._info = torch.zeros(1, dtype=torch.int32, device=self.device)
+        # m of samplers that do not announce it is known after the first draw: size the first chunk for the largest m
+        # the kernel takes
+        m = max((m for m in m_known if m is not None), default=self.max_kernel_m)
+        lo = 0
+        while lo < self.N:
+            step = max(1, int(self.max_stack_bytes // (8 * n_it * self.dim_out * m)))
+            chunk = vos[lo:lo + step]
+            V = self._draw(chunk, n_it)
+            m = int(V.shape[-1])
+            if m > self.max_kernel_m:      # only on the first chunk: the member loop, with the draws already made
+                saved = [vo._sampler for vo in chunk]
+                try:
+                    for k, vo in enumerate(chunk):
+                        vo._sampler = _ReplaySampler(vo.querry_point, V[k])
+                    return self._update_members(G, PREC, iteration)
+                finally:
+                    for vo, s in zip(chunk, saved):
+                        vo._sampler = s
+            hi = lo + len(chunk)
+            V = V.transpose(0, 1).contiguous()                          # [n_it, n, d, m]: one contiguous stack per step
+            for it in range(n_it):
+                _, rho = plan.residual(a[lo:hi], mean[lo:hi], gbc[lo:hi], None, a_is_log=False)
+                if load is not None:
+                    rho -= load[lo:hi]
+                plan.energy_step(a[lo:hi], V[it], rho, G64[lo:hi], P64[lo:hi], inv_T[lo:hi], mean[lo:hi], info=self._info)
+            lo = hi
+        if int(self._info.item()):
+            self._info.zero_()
+            raise RuntimeError("energy virtual-observable update: V^T A V is not positive definite for some data point")
+        for k, vo in enumerate(vos):
+            vo._mean, vo._vars = mean[k], vars_[k]
+        self.flush_cache()
+        self.last_update_route = "batched"
 
     def force_temperature(self, value):
         for vo in self:

@@ -57,6 +57,8 @@ SIGNATURES = {
     "gpde_vo_pack_weights_f32": (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_vp]),
     "gpde_vo_posterior_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_vo_moments_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_energy_step_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64,
+                                        c_vp]),
     "gpde_vo_residual_T_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_vo_residual_T_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_cg_init_f64": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_f64, c_i32, c_i64, c_i32, c_vp]),

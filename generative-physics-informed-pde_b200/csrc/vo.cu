@@ -48,6 +48,7 @@ constexpr int kVoThreads = 256;
 #include "vo_gemm.cuh"
 #include "vo_gridgemm.cuh"
 #include "vo_posterior.cuh"
+#include "vo_energy.cuh"
 
 namespace gpde {
 // Experiment switches (A/B runs of the kernel families).  Read from the environment ONCE per plan, in gpde_vo_plan_create,
@@ -1170,6 +1171,20 @@ static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, i
                                        q, B, st);
 }
 
+// gpde_vo_energy_step_f64 for MP = 32 or 64 (vo_energy.cuh)
+template <int MP>
+int vo_energy_step_launch(const gpde_vo_plan *pl, const double *a, int64_t a_stride, const double *V, int64_t v_stride,
+                          int m, const double *rho, const double *g, const double *prec, const double *inv_T,
+                          double *mean, int *info, int64_t N, cudaStream_t st) {
+    auto kern = vo_energy_step_kernel<MP>;
+    const size_t smem = energy_smem_bytes<MP>(pl->csr.max_row);
+    GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(unsigned)N, kPostThreads, smem, st>>>(pl->csr, a, (long long)a_stride, V, (long long)v_stride, m, rho, g, prec,
+                                                  inv_T, mean, info);
+    GPDE_CUDA_OK(cudaGetLastError());
+    return GPDE_OK;
+}
+
 }  // namespace gpde
 
 using namespace gpde;
@@ -1386,6 +1401,22 @@ int gpde_vo_moments_f64(const gpde_vo_plan *pl, const double *a, int64_t a_strid
     }
     GPDE_CUDA_OK(cudaGetLastError());
     return GPDE_OK;
+}
+
+int gpde_vo_energy_step_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, const double *V, int64_t v_stride,
+                            int m, const double *rho, const double *g, const double *prec, const double *inv_T, double *mean,
+                            int *info, int64_t N, gpde_stream_t stream) {
+    if (!pl || N < 0 || m <= 0) return fail(GPDE_ERR_ARG, "vo_energy_step: bad argument");
+    if (m > 64) return fail(GPDE_ERR_SIZE, "vo_energy_step: m = %d > 64 weighting functions per data point", m);
+    if (N == 0) return GPDE_OK;
+    if (!a || !V || !rho || !g || !prec || !inv_T || !mean) return fail(GPDE_ERR_ARG, "vo_energy_step: null argument");
+    if (a_stride != 0 && a_stride != (int64_t)pl->dev.n_inputs)
+        return fail(GPDE_ERR_ARG, "vo_energy_step: a_stride must be 0 or n_inputs");
+    if (v_stride != 0 && v_stride != (int64_t)pl->dev.d * m) return fail(GPDE_ERR_ARG, "vo_energy_step: v_stride must be 0 or d*m");
+    DeviceGuard guard(pl->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (m <= 32) return vo_energy_step_launch<32>(pl, a, a_stride, V, v_stride, m, rho, g, prec, inv_T, mean, info, N, st);
+    return vo_energy_step_launch<64>(pl, a, a_stride, V, v_stride, m, rho, g, prec, inv_T, mean, info, N, st);
 }
 
 int gpde_vo_residual_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *y,

@@ -216,6 +216,21 @@ int gpde_vo_moments_f64(const gpde_vo_plan *plan, const double *a, int64_t a_str
                         int m, const double *rho, const double *v, double *out_r, double *out_s2, int64_t N,
                         gpde_stream_t stream);
 
+/* One subspace-Newton step of the energy-type virtual observables for all data points in ONE launch, matrix-free
+ * (EnergyVirtualObservable.update, bottleneck/VirtualObservables.py:769-788, looped over the data points at :1001-1037):
+ *     M_n    = V_n^T diag(prec_n) V_n + inv_T[n] V_n^T K_ff(a_n) V_n        (= V_n^T A_n V_n, A_n = diag(prec_n) + K/T_n)
+ *     b_n    = V_n^T (prec_n (mean_n - g_n) + inv_T[n] rho_n)                (= V_n^T (A_n mean_n - b))
+ *     mean_n = mean_n - V_n M_n^-1 b_n                                       (Cholesky of M_n, in place on mean)
+ * a [N, n_inputs] conductivities (NOT logs; a_stride = 0: one field shared by all data points, else n_inputs); V [d,m]
+ * shared (v_stride = 0) or [N,d,m] (v_stride = d*m); m <= 64 (else GPDE_ERR_SIZE); rho [N,d] = K_ff(a_n) mean_n - f_eff
+ * (the rho output of gpde_vo_residual with y = mean, minus a load vector the plan does not carry); g, prec, mean [N,d];
+ * inv_T [N] device doubles.  N = 0 is a no-op.
+ * info (device int32, may be NULL) receives GPDE_INFO_NOT_SPD if some M_n has a non-positive pivot; that data point's mean
+ * is left unchanged.                                                                                                   */
+int gpde_vo_energy_step_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, const double *V,
+                            int64_t v_stride, int m, const double *rho, const double *g, const double *prec,
+                            const double *inv_T, double *mean, int *info, int64_t N, gpde_stream_t stream);
+
 /* q[B,d] = K_ff(a_b) (V s_b) = Gamma_b^T s_b  (VirtualObservables.py:663; with s = P r it is the
  * gradient of 1/2 r^T P r w.r.t. y).  With B = m, s = I and a_stride = 0 it yields Gamma itself.
  * On the reference's pixel meshes with m <= 32 this is one kernel (after a small packing launch of V^T): the rows
