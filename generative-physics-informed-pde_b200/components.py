@@ -186,7 +186,9 @@ class ReducedOrderModelOperator(torch.nn.Module):
         what GenerativeModel.update_virtual_observables computes in a Python loop over data points with
         propagate_samples + torch.mean / torch.std (generative.py:198-207).  effprops [N,S,E], F [N,n].  One batched coarse
         solve and one launch; the output noise is integrated out instead of sampled:
-            Y_std^2 = W Cov_s(u) W^T + exp(2 logsigmas_y)  (the expectation of the reference's sample variance)."""
+            Y_std^2 = W Cov_s(u) W^T + exp(2 logsigmas_y)  (the expectation of the reference's sample variance).
+        S = 1 gives Y_std = exp(logsigmas_y) (no sample covariance; torch.std of one sample would be NaN).  S is limited by
+        shared memory: S <= 998 on the 4x4 coarse mesh, S <= 234 on the 8x8 one (GpdeLibraryError beyond)."""
         N, S, E = effprops.shape
         Fx = F.unsqueeze(1).expand(N, S, F.shape[-1]).reshape(N * S, -1)
         u = self.rom.solve_log(effprops.reshape(N * S, E), Fx)

@@ -73,6 +73,8 @@ __global__ void prolong_apply_T_kernel(ProlongDev P, const T *__restrict__ gy, T
 // sample / per node and chunk).
 constexpr int kLlThreads = 256, kLlSamples = 32;
 constexpr double kLog2Pi = 1.8378770664093453;
+// dynamic shared memory the loglik row kernel and the moments kernel may ask for (opted in above the 48 KB default)
+constexpr size_t kMaxSmemBytes = 200 * 1024;
 
 template <typename T>
 __global__ void __launch_bounds__(kLlThreads)
@@ -199,15 +201,21 @@ template <typename T>
 static int prolong_loglik(const gpde_prolong_plan *pl, const T *u, const T *Y, const T *ls, double *L, T *gu, double *gls,
                           int64_t B, gpde_stream_t stream) {
     if (!pl || B < 0) return fail(GPDE_ERR_ARG, "prolong_loglik: bad argument");
-    if (B == 0) return GPDE_OK;
-    if (!u || !Y || !ls || !L) return fail(GPDE_ERR_ARG, "prolong_loglik: null argument");
+    if (B > 0 && (!u || !Y || !ls || !L)) return fail(GPDE_ERR_ARG, "prolong_loglik: null argument");
+    const size_t smem = sizeof(double) * ((size_t)kLlSamples * pl->dev.n + kLlSamples);
+    if (B > 0 && smem > kMaxSmemBytes)
+        return fail(GPDE_ERR_SIZE, "prolong_loglik: %d samples x %d dofs do not fit in shared memory", kLlSamples,
+                    pl->dev.n);
     DeviceGuard guard(pl->device);
     cudaStream_t st = (cudaStream_t)stream;
-    GPDE_CUDA_OK(cudaMemsetAsync(L, 0, sizeof(double) * (size_t)B, st));
+    // gls sums over the batch: an empty batch (a rank without samples) contributes zeros, not whatever gls held
     if (gls) GPDE_CUDA_OK(cudaMemsetAsync(gls, 0, sizeof(double) * (size_t)pl->dev.d, st));
+    if (B == 0) return GPDE_OK;
+    auto rows = prolong_loglik_rows_kernel<T>;
+    if (smem > 48 * 1024) GPDE_CUDA_OK(cudaFuncSetAttribute(rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    GPDE_CUDA_OK(cudaMemsetAsync(L, 0, sizeof(double) * (size_t)B, st));
     const dim3 grid((unsigned)((pl->dev.d + kLlThreads - 1) / kLlThreads), (unsigned)((B + kLlSamples - 1) / kLlSamples));
-    const size_t smem = sizeof(double) * (size_t)(kLlSamples * pl->dev.n + kLlSamples);
-    prolong_loglik_rows_kernel<T><<<grid, kLlThreads, smem, st>>>(pl->dev, u, Y, ls, L, gls, B);
+    rows<<<grid, kLlThreads, smem, st>>>(pl->dev, u, Y, ls, L, gls, B);
     if (gu) {
         const long long total = B * (long long)pl->dev.n;   // warps
         const unsigned g2 = (unsigned)std::min<long long>((total + 7) / 8, (long long)sm_count(pl->device) * 16);
@@ -224,7 +232,7 @@ static int prolong_moments(const gpde_prolong_plan *pl, const T *u, const T *ls,
     if (N == 0) return GPDE_OK;
     if (!u || !ls || !y_mean || !y_std) return fail(GPDE_ERR_ARG, "prolong_moments: null argument");
     const size_t smem = sizeof(double) * ((size_t)pl->dev.n * (1 + pl->dev.n) + (size_t)S * pl->dev.n);
-    if (smem > 200 * 1024) return fail(GPDE_ERR_SIZE, "prolong_moments: %d samples x %d dofs do not fit in shared memory", S, pl->dev.n);
+    if (smem > kMaxSmemBytes) return fail(GPDE_ERR_SIZE, "prolong_moments: %d samples x %d dofs do not fit in shared memory", S, pl->dev.n);
     DeviceGuard guard(pl->device);
     auto kern = prolong_moments_kernel<T>;
     GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

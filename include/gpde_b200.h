@@ -117,7 +117,8 @@ int gpde_prolong_apply_T_f32(const gpde_prolong_plan *plan, const float *gy, flo
  *     L  [B]   L_b   = -1/2 sum_i [2 ls_i + ((Y_bi - (W u_b)_i) / exp(ls_i))^2 + log 2 pi]        (always double)
  *     gu [B,n] dL_b/du_b = W^T ((Y_b - W u_b) exp(-2 ls))                          (may be NULL)
  *     gls[d]   d(sum_b L_b)/dls_i = sum_b (e_bi^2 - 1)                             (always double; may be NULL)
- * u [B,n], Y [B,d], ls [d] (log standard deviations, the operator's logsigmas_y).  L and gls are zeroed by the call. */
+ * u [B,n], Y [B,d], ls [d] (log standard deviations, the operator's logsigmas_y).  L and gls are zeroed by the call, gls
+ * also when B = 0.  The row kernel stages 32 samples of u in shared memory: n <= 799 coarse dofs, else GPDE_ERR_SIZE. */
 int gpde_prolong_loglik_f64(const gpde_prolong_plan *plan, const double *u, const double *Y, const double *ls,
                             double *L, double *gu, double *gls, int64_t B, gpde_stream_t stream);
 int gpde_prolong_loglik_f32(const gpde_prolong_plan *plan, const float *u, const float *Y, const float *ls,
@@ -127,7 +128,10 @@ int gpde_prolong_loglik_f32(const gpde_prolong_plan *plan, const float *u, const
  * torch.mean / torch.std over the S samples) without the [N S, d] samples: with ubar / Cov_u the sample mean / unbiased
  * covariance of the S coarse solutions u[n,s,:],
  *     y_mean[n,i] = W_i . ubar_n,     y_std[n,i] = sqrt(W_i Cov_u,n W_i^T + exp(2 ls_i))
- * (the reference's estimator with the output noise integrated out).  u [N,S,n_coarse], ls [d], y_mean / y_std [N,d]. */
+ * (the reference's estimator with the output noise integrated out).  u [N,S,n_coarse], ls [d], y_mean / y_std [N,d].
+ * S = 1 takes Cov_u as zero: y_std = exp(ls), where torch.std of one sample would give NaN.  ubar, Cov_u and the S
+ * samples live in shared memory: 8 (n (n + 1) + S n) bytes <= 200 KB, i.e. S <= 998 on the 4x4 coarse mesh (n = 25) and
+ * S <= 234 on the 8x8 one (n = 81); larger S returns GPDE_ERR_SIZE. */
 int gpde_prolong_moments_f64(const gpde_prolong_plan *plan, const double *u, const double *ls, double *y_mean,
                              double *y_std, int64_t N, int S, gpde_stream_t stream);
 int gpde_prolong_moments_f32(const gpde_prolong_plan *plan, const float *u, const float *ls, float *y_mean,
