@@ -7,11 +7,12 @@
 //   rho_i = sum_slots a[in] * (c0 * u_i + c1 * u~[j1] + c2 * u~[j2]) - f_i
 //
 // Kernel families, chosen per call (gpde_vo_plan_kernel_path):
-//   vo_grid.cuh   structured pixel grid (verified at plan creation), FP64 I/O: marching flux-form kernel with the
-//                 contraction on the FP64 tensor pipe inside the kernel (m <= 32), or producing rho for ...
-//   vo_gemm.cuh   ... the FP64 tensor-core contraction rho[B,d] V[d,m] for many weighting functions (m > 32);
-//   vo_fused.cuh  any P1 diffusion mesh, m <= 32: edge-form matvec + ring-staged tiles + DMMA contraction;
-//   version 1     (below) any mesh, any m, FP32/FP64: row-cell ELL matvec, then vo_gemm.cuh.
+//   vo_grid2.cuh     the reference's pixel meshes (verified at plan creation), FP32/FP64 I/O: marching flux-form kernel
+//                    with the contraction on the FP64 tensor pipe inside the kernel (m <= 32), or producing rho for ...
+//   vo_gridgemm.cuh  ... one kernel that also contracts rho with many weighting functions (m > 32), or for ...
+//   vo_gemm.cuh      ... the FP64 tensor-core contraction rho[B,d] V[d,m];
+//   vo_fused.cuh     any P1 diffusion mesh, m <= 32: edge-form matvec + ring-staged tiles + DMMA contraction;
+//   version 1        (below) any mesh, any m, FP32/FP64: row-cell ELL matvec, then vo_gemm.cuh.
 #include "common.cuh"
 
 #include <algorithm>
@@ -42,7 +43,6 @@ constexpr int kVoThreads = 256;
 }  // namespace gpde
 
 #include "vo_fused.cuh"
-#include "vo_grid.cuh"
 #include "vo_grid2.cuh"
 #include "vo_expand.cuh"
 #include "vo_gemm.cuh"
@@ -51,19 +51,22 @@ constexpr int kVoThreads = 256;
 #include "vo_energy.cuh"
 
 namespace gpde {
+// A pixel mesh the structured-grid kernels (vo_grid2.cuh) serve, verified by build_grid_plan.
+struct GridDev {
+    int ok;
+    int nx, ny;          // pixels per row, pixel rows; nodes are (nx+1) x (ny+1)
+    int ncol;            // free node columns per row (nx - 1)
+    long long in0, sy;   // conductivity entry of pixel (cx, cy) = in0 + cy * sy + cx
+    double rh, scale;    // rh = chs / cvs, scale = cvs
+    int has_load;
+};
+
 // Experiment switches (A/B runs of the kernel families).  Read from the environment ONCE per plan, in gpde_vo_plan_create,
 // never on a launch path.
 struct VoEnv {
-    int grid_r = 2;           // GPDE_GRID_R: node rows per stage of the general grid kernel (1 or 2)
     bool path_v1 = false;     // GPDE_VO_PATH=v1: version-1 kernels only
     bool path_fused = false;  // GPDE_VO_PATH=fused: no structured-grid kernels
-    bool no_grid2 = false;    // GPDE_GRID_V=1: general grid kernel instead of the lean one
-    int grid2_nvs = 0;        // GPDE_GRID2_NVS: V stages of the lean kernel (2 or 3; 0 = automatic)
-    int grid2_flags = 0;      // GPDE_GRID2_FLAGS
-    bool grid2_pdl = true;    // GPDE_GRID2_PDL=0: no programmatic dependent launch
-    int grid_debug = 0;       // GPDE_GRID_DEBUG
     bool sync_staging = false;   // GPDE_VO_SYNC_STAGING
-    bool expand_gemm = false;    // GPDE_VO_EXPAND=gemm
     int gemm_splits = 0;         // GPDE_GEMM_SPLITS: parts of the contraction length (0 = automatic)
     int grid2_split = 1;         // GPDE_GRID2_SPLIT: 0 = never cut the node rows over a cluster, 1 = automatic, n > 1 = force n
     bool gridgemm = true;        // GPDE_VO_GRIDGEMM=0: rho through HBM + vo_gemm_kernel instead of the one-kernel route (m > 32)
@@ -71,15 +74,8 @@ struct VoEnv {
     int grid2_spc = 0;           // GPDE_GRID2_SPC: samples per CTA of the lean grid kernel (0 = automatic, see grid2_samples_per_cta)
     VoEnv() {
         const char *e;
-        if ((e = getenv("GPDE_GRID_R"))) grid_r = atoi(e);
         if ((e = getenv("GPDE_VO_PATH"))) { path_v1 = strcmp(e, "v1") == 0; path_fused = strcmp(e, "fused") == 0; }
-        if ((e = getenv("GPDE_GRID_V"))) no_grid2 = atoi(e) == 1;
-        if ((e = getenv("GPDE_GRID2_NVS"))) grid2_nvs = atoi(e);
-        if ((e = getenv("GPDE_GRID2_FLAGS"))) grid2_flags = atoi(e);
-        if ((e = getenv("GPDE_GRID2_PDL"))) grid2_pdl = atoi(e) != 0;
-        if ((e = getenv("GPDE_GRID_DEBUG"))) grid_debug = atoi(e);
         sync_staging = getenv("GPDE_VO_SYNC_STAGING") != nullptr;
-        if ((e = getenv("GPDE_VO_EXPAND"))) expand_gemm = strcmp(e, "gemm") == 0;
         if ((e = getenv("GPDE_GEMM_SPLITS"))) gemm_splits = std::max(0, std::min(8, atoi(e)));
         if ((e = getenv("GPDE_GRID2_SPLIT"))) grid2_split = std::max(0, std::min(8, atoi(e)));
         if ((e = getenv("GPDE_VO_GRIDGEMM"))) gridgemm = atoi(e) != 0;
@@ -367,31 +363,30 @@ static cudaError_t build_csr_terms(gpde_vo_plan *pl, int n_cells, const int32_t 
     return e;
 }
 
-// Structured-grid detection for vo_grid.cuh.  Leaves pl->grid.ok = 0 unless the element data is exactly the
-// 5-point pixel operator the grid kernel evaluates (every check below is against the arrays the caller
-// passed, nothing is assumed from names):
-//   nodes (nx+1) x (ny+1) numbered x-fastest; Dirichlet dofs = the columns ix = 0 and ix = nx, listed row by
-//   row (left, right); free dofs = all other nodes ascending; two cells per pixel sharing one input entry
-//   in0 + cy*sy + cx; horizontal / vertical couplings uniform (chs / cvs), hypotenuse couplings zero.
-static cudaError_t build_grid_plan(gpde_vo_plan *pl, int n_nodes, int n_cells, const int32_t *cell_dofs,
-                                   const double *Ke, const int32_t *cell_to_input, int n_inputs,
-                                   const int64_t *free_dofs, int d, const int64_t *bc_dofs, int n_bc,
-                                   const std::vector<double> &f_free) {
+// Structured-grid detection for vo_grid2.cuh.  Leaves pl->grid.ok = 0 unless the element data is exactly the
+// 5-point pixel operator the grid kernel evaluates on a mesh it is built for (every check below is against the
+// arrays the caller passed, nothing is assumed from names):
+//   nodes (nx+1) x (ny+1) numbered x-fastest, nx in {16, 32, 64, 128}, ny even; Dirichlet dofs = the columns ix = 0
+//   and ix = nx, listed row by row (left, right); free dofs = all other nodes ascending; two cells per pixel sharing
+//   one input entry in0 + cy*sy + cx; horizontal / vertical couplings uniform (chs / cvs), hypotenuse couplings zero.
+static void build_grid_plan(gpde_vo_plan *pl, int n_nodes, int n_cells, const int32_t *cell_dofs, const double *Ke,
+                            const int32_t *cell_to_input, int n_inputs, const int64_t *free_dofs, int d,
+                            const int64_t *bc_dofs, int n_bc, const std::vector<double> &f_free) {
     GridDev &G = pl->grid;
     memset(&G, 0, sizeof(G));
-    if (n_bc < 4 || (n_bc & 1) || bc_dofs[0] != 0) return cudaSuccess;
+    if (n_bc < 4 || (n_bc & 1) || bc_dofs[0] != 0) return;
     const long long nxn = bc_dofs[1] + 1;               // nodes per row
-    if (nxn < 3 || n_nodes % nxn != 0) return cudaSuccess;
+    if (nxn < 3 || n_nodes % nxn != 0) return;
     const int nx = (int)nxn - 1, nyn = (int)(n_nodes / nxn), ny = nyn - 1, ncol = nx - 1;
-    if (ny < 1 || n_bc != 2 * nyn || d != ncol * nyn || n_cells != 2 * nx * ny || n_inputs != nx * ny) return cudaSuccess;
-    if ((nx & 1) || ncol > 256) return cudaSuccess;       // pixel rows must be whole 16-byte units
+    if (ny < 1 || n_bc != 2 * nyn || d != ncol * nyn || n_cells != 2 * nx * ny || n_inputs != nx * ny) return;
+    if (!(nx == 16 || nx == 32 || nx == 64 || nx == 128) || ny < 2 || (ny & 1)) return;
     for (int r = 0; r < nyn; ++r)
-        if (bc_dofs[2 * r] != (long long)r * nxn || bc_dofs[2 * r + 1] != (long long)r * nxn + nx) return cudaSuccess;
+        if (bc_dofs[2 * r] != (long long)r * nxn || bc_dofs[2 * r + 1] != (long long)r * nxn + nx) return;
     for (int i = 0; i < d; ++i)
-        if (free_dofs[i] != (long long)(i / ncol) * nxn + 1 + i % ncol) return cudaSuccess;
+        if (free_dofs[i] != (long long)(i / ncol) * nxn + 1 + i % ncol) return;
     double kmax = 0.0;
     for (size_t k = 0; k < (size_t)n_cells * 9; ++k) kmax = std::max(kmax, fabs(Ke[k]));
-    if (!(kmax > 0.0)) return cudaSuccess;
+    if (!(kmax > 0.0)) return;
     const double tol = 1e-13 * kmax;
     std::vector<int> sq_input((size_t)nx * ny, -1), sq_count((size_t)nx * ny, 0);
     // side coverage per square: bottom, top (horizontal), left, right (vertical)
@@ -405,106 +400,55 @@ static cudaError_t build_grid_plan(gpde_vo_plan *pl, int n_nodes, int n_cells, c
             iy[l] = cell_dofs[3 * c + l] / (int)nxn;
         }
         const int cx = std::min(ix[0], std::min(ix[1], ix[2])), cy = std::min(iy[0], std::min(iy[1], iy[2]));
-        if (cx >= nx || cy >= ny) return cudaSuccess;
+        if (cx >= nx || cy >= ny) return;
         for (int l = 0; l < 3; ++l)
-            if (ix[l] - cx > 1 || iy[l] - cy > 1) return cudaSuccess;
+            if (ix[l] - cx > 1 || iy[l] - cy > 1) return;
         const size_t sq = (size_t)cy * nx + cx;
         if (sq_count[sq] == 0) sq_input[sq] = cell_to_input[c];
-        else if (sq_input[sq] != cell_to_input[c]) return cudaSuccess;   // per-cell input: generic kernels
-        if (++sq_count[sq] > 2) return cudaSuccess;
+        else if (sq_input[sq] != cell_to_input[c]) return;   // per-cell input: generic kernels
+        if (++sq_count[sq] > 2) return;
         for (int l = 0; l < 3; ++l) {
             double rs = 0.0;
             for (int l2 = 0; l2 < 3; ++l2) rs += Ke[9 * c + 3 * l + l2];
-            if (fabs(rs) > tol) return cudaSuccess;                     // not a pure diffusion operator
+            if (fabs(rs) > tol) return;                     // not a pure diffusion operator
             for (int l2 = 0; l2 < 3; ++l2) {
                 if (l2 == l) continue;
                 const double v = Ke[9 * c + 3 * l + l2];
-                if (fabs(v - Ke[9 * c + 3 * l2 + l]) > tol) return cudaSuccess;
+                if (fabs(v - Ke[9 * c + 3 * l2 + l]) > tol) return;
                 const int dx = ix[l2] - ix[l], dy = iy[l2] - iy[l];
                 if (dx != 0 && dy != 0) {
-                    if (fabs(v) > tol) return cudaSuccess;               // hypotenuse must not couple
+                    if (fabs(v) > tol) return;               // hypotenuse must not couple
                 } else if (dy == 0) {
                     if (!have_h) { chs = v; have_h = true; }
-                    if (fabs(v - chs) > tol) return cudaSuccess;
+                    if (fabs(v - chs) > tol) return;
                     if (l < l2) side[sq * 4 + (iy[l] == cy ? 0 : 1)]++;
                 } else {
                     if (!have_v) { cvs = v; have_v = true; }
-                    if (fabs(v - cvs) > tol) return cudaSuccess;
+                    if (fabs(v - cvs) > tol) return;
                     if (l < l2) side[sq * 4 + 2 + (ix[l] == cx ? 0 : 1)]++;
                 }
             }
         }
     }
-    if (!have_h || !have_v || chs == 0.0 || cvs == 0.0) return cudaSuccess;
+    if (!have_h || !have_v || chs == 0.0 || cvs == 0.0) return;
     for (size_t k = 0; k < side.size(); ++k)
-        if (side[k] != 1) return cudaSuccess;                          // every pixel side carried by exactly one cell
+        if (side[k] != 1) return;                          // every pixel side carried by exactly one cell
     for (size_t sq = 0; sq < sq_count.size(); ++sq)
-        if (sq_count[sq] != 2) return cudaSuccess;
+        if (sq_count[sq] != 2) return;
     const long long in0 = sq_input[0];
     const long long sy = ny > 1 ? (long long)sq_input[nx] - in0 : nx;
-    if (sy != nx && sy != -nx) return cudaSuccess;
+    if (sy != nx && sy != -nx) return;
     for (int cy = 0; cy < ny; ++cy)
         for (int cx = 0; cx < nx; ++cx)
-            if (sq_input[(size_t)cy * nx + cx] != in0 + cy * sy + cx) return cudaSuccess;
-    if ((in0 & 1) || (sy & 1)) return cudaSuccess;
+            if (sq_input[(size_t)cy * nx + cx] != in0 + cy * sy + cx) return;
+    if ((in0 & 1) || (sy & 1)) return;
 
-    G.nx = nx; G.ny = ny; G.ncol = ncol; G.cols = 4; G.nstrips = 0; G.groups = 0;   // decomposition: grid_pick()
+    G.nx = nx; G.ny = ny; G.ncol = ncol;
     G.in0 = in0; G.sy = sy; G.rh = chs / cvs; G.scale = cvs;
     G.has_load = 0;
-    std::vector<double> f_over(d);
-    for (int i = 0; i < d; ++i) {
-        f_over[i] = f_free[i] / cvs;
+    for (int i = 0; i < d; ++i)
         if (f_free[i] != 0.0) G.has_load = 1;
-    }
-    cudaError_t e = track_vo(pl, &G.f_over, f_over);
-    if (e == cudaSuccess) G.ok = 1;
-    return e;
-}
-
-// Shared-memory layout of one pipeline stage holding R node rows (see vo_grid.cuh): per-sample regions of
-// a_stride / y_stride doubles (pitches chosen so that the 8 samples of a warp hit distinct banks), then the
-// packed V rows.  Returns the stage size in bytes for NT n-tiles (NT = 0: no V in the stage).
-static inline size_t grid_layout(GridDev &G, int R, int NT) {
-    const int S = 8 * G.groups;
-    G.a_stride = std::max(R * G.nx, (R - 1) * G.nx + 4 * G.cols * G.nstrips) + 2;
-    G.y_stride = ((R - 1) * G.ncol + 4 * G.cols * G.nstrips + 4 + 3) & ~3;
-    G.a_off = 0;
-    G.y_off = S * G.a_stride * 8;
-    G.v_off = (G.y_off + S * G.y_stride * 8 + 127) & ~127;
-    return (size_t)G.v_off + (size_t)R * G.nstrips * G.cols * NT * 32 * 8;
-}
-static inline int grid_nstrips(int ncol, int cols) {
-    int n = 1;
-    while (n * 4 * cols < ncol) n *= 2;
-    return n;
-}
-static inline size_t grid_packed_bytes(const GridDev &G, int NT) {
-    return (size_t)(G.ny + 1) * grid_nstrips(G.ncol, 4) * 4 * NT * 32 * 8;
-}
-// rows per stage and ring depth that fit the 227 KB of a CTA: two rows per stage halve the per-row barrier and
-// staging overhead (GPDE_GRID_R forces 1 or 2 for experiments)
-// Decomposition: columns per lane C, warps per CTA W, rows per stage R, ring depth NS.  The kernel is templated on
-// all of them; measured on B200 at cfg 2 (round 1):
-//     C = 4, W = 16, R = 2 : 156 us   <- instantiated (16 warps of 128 registers, one CTA per SM)
-//     C = 4, W = 16, R = 1 : 186 us   <- instantiated (used when two 2-row stages do not fit)
-//     C = 4, W =  8, R = 1 : 174 us   (8 warps per CTA, two CTAs per SM)
-//     C = 8, W =  8, R = 2 : 176 us   (8 fat warps, half the per-step overhead per node)
-// The kernel is latency-bound at 4 warps per scheduler: more resident warps win over less overhead per node.
-// GPDE_GRID_R=1 forces one row per stage (A/B runs).
-static inline bool grid_pick(const VoEnv &env, GridDev &G, int NT, int &R, int &NS, int &W, size_t &stage) {
-    const int C = 4;
-    W = 16;
-    if (grid_nstrips(G.ncol, C) > W) return false;
-    G.cols = C;
-    G.nstrips = grid_nstrips(G.ncol, C);
-    G.groups = W / G.nstrips;
-    const size_t budget = 225 * 1024 - 512;
-    for (R = env.grid_r; R >= 1; --R) {
-        stage = grid_layout(G, R, NT);
-        NS = (int)std::min<size_t>(R == 2 ? 3 : 4, budget / stage);
-        if (NS >= 2) return true;
-    }
-    return false;
+    G.ok = 1;
 }
 
 // GPDE_VO_PATH=v1 forces the unfused version-1 kernels (A/B testing, fallback check)
@@ -517,16 +461,18 @@ static bool use_grid(const gpde_vo_plan *pl) {
     return pl->grid.ok && !pl->env.path_v1 && !pl->env.path_fused;
 }
 
-// Lean structured-grid kernel (vo_grid2.cuh): nx in {16, 32, 64, 128}, even ny, no load vector.  Returns 1 if it
-// served the call, 0 if vo_grid.cuh should.  rho_pitch > 0 selects the rho variant (V, m unused).
-// GPDE_GRID_V=1 keeps it out (A/B runs against the general kernel).
-// mesh-side conditions and the decomposition of the lean kernel for m weighting functions (rho: no V inside)
+// Bytes of one packed V row of the lean grid kernel: NT n-tiles and NX DFMA columns per strip, then the strips' masks.
+static inline int grid2_v_row_bytes(int nstrips, int NT, int NX) {
+    return nstrips * (4 * NT * 32 * 8 + NX * 128) + kGrid2MaskBytes;
+}
+
+// The decomposition of the lean grid kernel (vo_grid2.cuh) for m weighting functions (rho: no V inside); false when it
+// does not apply (no pixel mesh, a load vector to subtract, m > 32, shared memory).
 static bool grid2_setup(const gpde_vo_plan *pl, int m, bool rho, int sub_f, Grid2Dev &G, int &NT, int &NX, size_t &smem,
                         int ea = 8, int ey = 8) {   // ea / ey: bytes per element of a / y (8 or 4)
     const GridDev &G0 = pl->grid;
-    if (pl->env.no_grid2) return false;
     const int nx = G0.nx, ny = G0.ny;
-    if (!G0.ok || !(nx == 16 || nx == 32 || nx == 64 || nx == 128) || ny < 2 || (ny & 1)) return false;
+    if (!G0.ok) return false;
     if (G0.has_load && sub_f) return false;
     NT = 1; NX = 0;
     if (!rho) {
@@ -548,17 +494,20 @@ static bool grid2_setup(const gpde_vo_plan *pl, int m, bool rho, int sub_f, Grid
     G.y_pitch = ey == 8 ? 2 * nx + 8 : 2 * nx + 12;
     G.y_off = S * G.a_pitch * ea;
     G.v_off = 0;
-    G.v_row_bytes = rho ? 0 : G.nstrips * (4 * NT * 32 * 8 + NX * 128) + kGrid2MaskBytes;
+    G.v_row_bytes = rho ? 0 : grid2_v_row_bytes(G.nstrips, NT, NX);
     G.stage_bytes = (G.y_off + S * G.y_pitch * ey + 127) & ~127;
     const size_t fixed = 2 * (size_t)G.stage_bytes + (4 * 16 + 8) * sizeof(unsigned long long) + 258 * sizeof(double);
     // V ring: three 2-row stages when they fit (the sample groups of a CTA may then drift a stage apart), else two
     G.nvs = rho ? 0 : ((fixed + 3 * 2 * (size_t)G.v_row_bytes <= 227 * 1024) ? 3 : 2);
-    if (!rho && (pl->env.grid2_nvs == 2 || pl->env.grid2_nvs == 3)) G.nvs = pl->env.grid2_nvs;
     smem = fixed + (size_t)G.nvs * 2 * G.v_row_bytes;
     if (smem > 227 * 1024) return false;
-    G.flags = pl->env.grid2_flags;
     G.spc = S;
     return true;
+}
+
+// The lean grid kernel stages a in 16-byte pieces: base, sample stride and the plan's pixel offsets must be aligned.
+static bool grid2_a_aligned(const gpde_vo_plan *pl, const void *a, long long a_stride, int ea) {
+    return !((uintptr_t)a & 15) && !((a_stride * ea) & 15) && !((pl->grid.in0 * ea) & 15) && !((pl->grid.sy * ea) & 15);
 }
 
 // Samples per CTA of the lean grid kernel.  A CTA holds S = 8 * groups sample slots and owns a whole SM; with
@@ -595,8 +544,8 @@ static int launch_grid2(const gpde_vo_plan *pl, const TA *a, long long a_stride,
     int NT, NX;
     size_t smem;
     if (!grid2_setup(pl, m, rho, sub_f, G, NT, NX, smem, EA, EY)) return 0;
-    // 16-byte pieces of a: base, sample stride and the plan's pixel offsets; y only needs its natural alignment
-    if (((uintptr_t)a & 15) || ((a_stride * EA) & 15) || ((G.in0 * EA) & 15) || ((G.sy * EA) & 15) || ((uintptr_t)y & (EY - 1))) return 0;
+    // y only needs its natural alignment
+    if (!grid2_a_aligned(pl, a, a_stride, EA) || ((uintptr_t)y & (EY - 1))) return 0;
     if (!rho && ((uintptr_t)workspace & 15)) return 0;
     const int S = 8 * G.groups;
     double *Vp = (double *)workspace;
@@ -618,8 +567,8 @@ static int launch_grid2(const gpde_vo_plan *pl, const TA *a, long long a_stride,
     }
     const unsigned grid = blocks * (unsigned)csize;
     // the residual kernel is launched as a programmatic dependent of the packing kernel (its prologue and first
-    // a / y stages overlap the packing); GPDE_GRID2_PDL=0 keeps the plain stream order
-    const bool pdl = !rho && !prepacked && pl->env.grid2_pdl && csize == 1;
+    // a / y stages overlap the packing)
+    const bool pdl = !rho && !prepacked && csize == 1;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3(grid);
@@ -704,12 +653,11 @@ static int launch_grid2_wt(const gpde_vo_plan *pl, const T *a, long long a_strid
     int NT, NX;
     size_t smem;
     if (!grid2_setup(pl, 0, true, 0, G, NT, NX, smem, EA, 8)) return 0;
-    if (((uintptr_t)a & 15) || ((a_stride * EA) & 15) || ((G.in0 * EA) & 15) || ((G.sy * EA) & 15) || ((uintptr_t)workspace & 15)) return 0;
+    if (!grid2_a_aligned(pl, a, a_stride, EA) || ((uintptr_t)workspace & 15)) return 0;
     const int KS = mw <= 16 ? 4 : (mw <= 28 ? 7 : 8);
     G.v_row_bytes = G.nstrips * 2 * KS * 256 + kGrid2MaskBytes;
     const size_t fixed = smem;                  // (rho variant: no V stages counted yet)
     G.nvs = (fixed + 3 * 2 * (size_t)G.v_row_bytes <= 227 * 1024) ? 3 : 2;
-    if (pl->env.grid2_nvs == 2 || pl->env.grid2_nvs == 3) G.nvs = pl->env.grid2_nvs;
     smem = fixed + (size_t)G.nvs * 2 * G.v_row_bytes;
     if (smem > 227 * 1024) return 0;
     const int S = 8 * G.groups, d = pl->dev.d;
@@ -738,7 +686,7 @@ static int launch_grid2_wt(const gpde_vo_plan *pl, const T *a, long long a_strid
 }
 
 // Structured-grid path.  Returns 1 if it served the call, 0 if the caller should use the generic kernels (alignment /
-// size conditions not met), <0 on error.  FP32 I/O: the lean kernel only.
+// size conditions not met), <0 on error.
 template <typename T>
 static int launch_grid_lean(const gpde_vo_plan *pl, const T *a, long long a_stride, int a_is_log, const T *y,
                             const T *g, long long g_stride, const T *V, int m, T *r, void *workspace,
@@ -752,51 +700,6 @@ static int launch_grid_lean(const gpde_vo_plan *pl, const T *a, long long a_stri
                                   "(16-byte aligned a and sample stride, y given, no load vector)");
     return 0;
 }
-static int launch_grid(const gpde_vo_plan *pl, const double *a, long long a_stride, int a_is_log, const double *y,
-                       const double *g, long long g_stride, const double *V, int m, double *r, void *workspace,
-                       int sub_f, bool prepacked, long long B, cudaStream_t st, int sm_reserve = 0) {
-    GridDev G = pl->grid;
-    if (!y || m < 1 || m > 32) return 0;
-    {
-        const int rc2 = launch_grid_lean<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, m, r, workspace, sub_f, prepacked, B, st,
-                                                 sm_reserve);
-        if (rc2 != 0) return rc2;
-    }
-    if (((uintptr_t)a & 15) || ((uintptr_t)y & 15) || (a_stride & 1) || ((uintptr_t)workspace & 15)) return 0;
-    const int NT = m <= 8 ? 1 : (m <= 16 ? 2 : 4);
-    int R, NS, W;
-    size_t stage;
-    if (!grid_pick(pl->env, G, NT, R, NS, W, stage)) return 0;
-    if (!sub_f) G.has_load = 0;
-    double *Vp = (double *)workspace;
-    {
-        const long long total = (long long)grid_packed_bytes(G, NT) / 8;
-        const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, (long long)pl->n_sm * 8);
-        vo_grid_pack_kernel<<<grid, 256, 0, st>>>(G, V, m, NT, Vp);
-    }
-    const int S = 8 * G.groups;
-    const int dbg = pl->env.grid_debug;   // timing experiments only
-    const unsigned grid = (unsigned)((B + S - 1) / S);
-    const size_t smem = (size_t)NS * stage + 2 * NS * sizeof(unsigned long long) + 16 * sizeof(double);
-#define GPDE_LAUNCH_GRID(NTV, RV, WV, CV)                                                                        \
-    {                                                                                                            \
-        auto kern = vo_grid_kernel<NTV, false, RV, WV, CV>;                                                      \
-        GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));        \
-        kern<<<grid, WV * 32, smem, st>>>(G, a, a_stride, a_is_log, y, g, g_stride, Vp, m, r, B, NS, (int)stage, dbg); \
-    }
-#define GPDE_LAUNCH_GRID_NT(RV, WV, CV)                                                                          \
-    {                                                                                                            \
-        if (NT == 1) GPDE_LAUNCH_GRID(1, RV, WV, CV)                                                             \
-        else if (NT == 2) GPDE_LAUNCH_GRID(2, RV, WV, CV)                                                        \
-        else GPDE_LAUNCH_GRID(4, RV, WV, CV)                                                                     \
-    }
-    if (R == 2) GPDE_LAUNCH_GRID_NT(2, 16, 4)
-    else GPDE_LAUNCH_GRID_NT(1, 16, 4)
-#undef GPDE_LAUNCH_GRID_NT
-#undef GPDE_LAUNCH_GRID
-    GPDE_CUDA_OK(cudaGetLastError());
-    return 1;
-}
 
 // Structured-grid fine residual rho[B][pitch] (pitch >= d, padding zeroed) for the tensor-core contraction.
 // Returns 1 if it served the call, 0 if the generic matvec kernel should (alignment / size), <0 on error.
@@ -807,35 +710,6 @@ static int launch_grid_rho_lean(const gpde_vo_plan *pl, const T *a, long long a_
     return launch_grid2<T, T, TR>(pl, a, a_stride, a_is_log, y, g, g_stride, (const T *)nullptr, 0, rho, nullptr, pitch, sub_f,
                                   false, B, st);
 }
-static int launch_grid_rho(const gpde_vo_plan *pl, const double *a, long long a_stride, int a_is_log, const double *y,
-                           const double *g, long long g_stride, double *rho, int pitch, int sub_f, long long B,
-                           cudaStream_t st) {
-    GridDev G = pl->grid;
-    if (!y) return 0;
-    {
-        const int rc2 = launch_grid_rho_lean<double, double>(pl, a, a_stride, a_is_log, y, g, g_stride, rho, pitch, sub_f, B, st);
-        if (rc2 != 0) return rc2;
-    }
-    if (((uintptr_t)a & 15) || ((uintptr_t)y & 15) || (a_stride & 1)) return 0;
-    int R, NS, W;
-    size_t stage;                                     // no V rows in the stage
-    if (!grid_pick(pl->env, G, 0, R, NS, W, stage)) return 0;
-    if (!sub_f) G.has_load = 0;
-    const int S = 8 * G.groups;
-    const unsigned grid = (unsigned)((B + S - 1) / S);
-    const size_t smem = (size_t)NS * stage + 2 * NS * sizeof(unsigned long long) + 16 * sizeof(double);
-#define GPDE_LAUNCH_RHO(RV, WV, CV)                                                                              \
-    {                                                                                                            \
-        auto kern = vo_grid_kernel<1, true, RV, WV, CV>;                                                         \
-        GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));        \
-        kern<<<grid, WV * 32, smem, st>>>(G, a, a_stride, a_is_log, y, g, g_stride, nullptr, pitch, rho, B, NS, (int)stage, 0); \
-    }
-    if (R == 2) GPDE_LAUNCH_RHO(2, 16, 4) else GPDE_LAUNCH_RHO(1, 16, 4)
-#undef GPDE_LAUNCH_RHO
-    GPDE_CUDA_OK(cudaGetLastError());
-    return 1;
-}
-
 template <typename Ta, typename Ty, typename To>
 static int launch_matvec(const gpde_vo_plan *pl, const Ta *a, long long a_stride, int a_is_log, const Ty *y,
                          const Ta *g, long long g_stride, int sub_f, double *rho_ws, int ws_stride, To *rho_out,
@@ -953,14 +827,8 @@ static int vo_residual(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int
     DeviceGuard guard(pl->device);
     cudaStream_t st = (cudaStream_t)stream;
     if (m > 0 && !rho && use_grid(pl)) {
-        int rc;
-        if constexpr (sizeof(T) == 8)
-            rc = launch_grid(pl, (const double *)a, (long long)a_stride, a_is_log, (const double *)y,
-                             (const double *)g, (long long)g_stride, (const double *)V, m, (double *)r,
-                             workspace, (flags & 1) ? 0 : 1, (flags & 2) != 0, (long long)B, st, (flags >> 8) & 0xff);
-        else
-            rc = launch_grid_lean<T>(pl, a, (long long)a_stride, a_is_log, y, g, (long long)g_stride, V, m, r, workspace,
-                                     (flags & 1) ? 0 : 1, (flags & 2) != 0, (long long)B, st, (flags >> 8) & 0xff);
+        const int rc = launch_grid_lean<T>(pl, a, (long long)a_stride, a_is_log, y, g, (long long)g_stride, V, m, r, workspace,
+                                           (flags & 1) ? 0 : 1, (flags & 2) != 0, (long long)B, st, (flags >> 8) & 0xff);
         if (rc != 0) return rc < 0 ? rc : GPDE_OK;
     }
     if (m == 0 && rho && use_grid(pl)) {   // the fine residual alone: rho rows straight into the caller's [B,d]
@@ -998,12 +866,8 @@ static int vo_residual(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int
     double *ws = m > 0 ? (double *)workspace : nullptr;
     int rc = 0;
     if (m > 0 && !rho && use_grid(pl)) {   // structured pixel grid: the marching kernel produces rho (no V inside)
-        if constexpr (sizeof(T) == 8)
-            rc = launch_grid_rho(pl, (const double *)a, (long long)a_stride, a_is_log, (const double *)y, (const double *)g,
-                                 (long long)g_stride, ws, dp, (flags & 1) ? 0 : 1, (long long)B, st);
-        else
-            rc = launch_grid_rho_lean<T, double>(pl, a, (long long)a_stride, a_is_log, y, g, (long long)g_stride, ws, dp,
-                                                 (flags & 1) ? 0 : 1, (long long)B, st);
+        rc = launch_grid_rho_lean<T, double>(pl, a, (long long)a_stride, a_is_log, y, g, (long long)g_stride, ws, dp,
+                                             (flags & 1) ? 0 : 1, (long long)B, st);
         if (rc < 0) return rc;
     }
     if (rc == 0) {
@@ -1057,87 +921,46 @@ static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, i
         const int rc = launch_grid2_wt<T>(pl, a, (long long)a_stride, a_is_log, V, m, s, q, workspace, (long long)B, st);
         if (rc != 0) return rc < 0 ? rc : GPDE_OK;
     }
-    if constexpr (sizeof(T) == 4) {
-        // FP32 I/O on the reference's pixel meshes, m <= 32: the same two launches as FP64 (s, V converted on load by the
-        // expansion kernel; w stays FP64 workspace; the marching kernel stages a as floats and stores q as floats)
-        Grid2Dev G2;
-        int nt2, nx2;
-        size_t smem2;
-        if (use_grid(pl) && m <= 32 && !((uintptr_t)a & 15) && !((a_stride * 4) & 15) && !((uintptr_t)workspace & 15) &&
-            grid2_setup(pl, 0, true, 0, G2, nt2, nx2, smem2, 4, 8)) {
-            const int d = pl->dev.d;
-            double *w = (double *)workspace;
-            const long long ldw = ((long long)d + 3) & ~3ll;
+    // structured pixel grid: w = s V^T on the FP64 tensor pipe, then q = K_ff w with the marching kernel (rho of u~ = (w, 0)
+    // without the load vector IS K_ff w); FP32 I/O: s and V converted on load, w stays FP64, a staged and q stored as floats
+    Grid2Dev G2;
+    int nt2, nx2;
+    size_t smem2;
+    if (use_grid(pl) && (m <= 32 || sizeof(T) == 8) && grid2_a_aligned(pl, a, (long long)a_stride, (int)sizeof(T)) &&
+        !((uintptr_t)workspace & 15) && grid2_setup(pl, 0, true, 0, G2, nt2, nx2, smem2, (int)sizeof(T), 8)) {
+        const int d = pl->dev.d;
+        double *w = (double *)workspace;
+        long long ldw = d;
+        if (m <= 32) {   // contraction length m <= 32: one launch, operands read in place (vo_expand.cuh)
+            ldw = ((long long)d + 3) & ~3ll;
             const int n_tiles = (d + 7) / 8;
             const unsigned gx = (unsigned)((B + 8 * kExpandMT * kExpandWarps - 1) / (8 * kExpandMT * kExpandWarps));
             const int nch = std::max(1, std::min(n_tiles, (int)(4 * pl->n_sm / gx)));
-            const int tpc = std::min((n_tiles + nch - 1) / nch, 64);
+            const int tpc = std::min((n_tiles + nch - 1) / nch, 64);         // <= 64 n-tiles of V per CTA in shared memory
             const dim3 grid(gx, (unsigned)((n_tiles + tpc - 1) / tpc));
             const size_t smem = (size_t)tpc * 8 * kExpandVPitch * sizeof(double);
-#define GPDE_LAUNCH_EXPAND_F(KSV)                                                                                   \
-    {                                                                                                               \
-        auto kern = vo_expand_dmma_kernel<KSV, float>;                                                              \
-        GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
-        kern<<<grid, kExpandWarps * 32, smem, st>>>((const float *)s, (const float *)V, w, ldw, (long long)B, d, m, tpc); \
-    }
-            if (m <= 8) GPDE_LAUNCH_EXPAND_F(2)
-            else if (m <= 16) GPDE_LAUNCH_EXPAND_F(4)
-            else if (m <= 28) GPDE_LAUNCH_EXPAND_F(7)
-            else GPDE_LAUNCH_EXPAND_F(8)
-#undef GPDE_LAUNCH_EXPAND_F
-            GPDE_CUDA_OK(cudaGetLastError());
-            const int rc2 = launch_grid2<float, double, float>(pl, (const float *)a, (long long)a_stride, a_is_log, w, nullptr, 0,
-                                                               nullptr, 0, (float *)q, nullptr, d, 0, false, (long long)B, st, ldw);
-            if (rc2 != 0) return rc2 < 0 ? rc2 : GPDE_OK;
-        }
-    }
-    if constexpr (sizeof(T) == 8) {
-        // structured pixel grid: w = s V^T on the FP64 tensor pipe, then q = K_ff w with the marching kernel
-        // (rho of u~ = (w, 0) without the load vector IS K_ff w)
-        if (use_grid(pl) && !((uintptr_t)a & 15) && !(a_stride & 1) && !((uintptr_t)workspace & 15)) {
-            const int d = pl->dev.d, mp = gemm_dp(m), bn = 128, ldb = (d + bn - 1) / bn * bn;
-            double *Sp = (double *)workspace, *Vt = Sp + (size_t)B * mp, *w = Vt + (size_t)mp * ldb;
-            if (m <= 32 && !pl->env.expand_gemm) {   // GPDE_VO_EXPAND=gemm: the general GEMM also for m <= 32 (A/B runs)
-                // contraction length m <= 32: one launch, operands read in place (vo_expand.cuh)
-                w = (double *)workspace;
-                Grid2Dev G2;
-                int nt2, nx2;
-                size_t smem2;
-                const bool lean = grid2_setup(pl, 0, true, 0, G2, nt2, nx2, smem2);
-                const long long ldw = lean ? (((long long)d + 3) & ~3ll) : d;   // the general grid kernel wants y contiguous
-                const int n_tiles = (d + 7) / 8;
-                const unsigned gx = (unsigned)((B + 8 * kExpandMT * kExpandWarps - 1) / (8 * kExpandMT * kExpandWarps));
-                const int nch = std::max(1, std::min(n_tiles, (int)(4 * pl->n_sm / gx)));
-                const int tpc = std::min((n_tiles + nch - 1) / nch, 64);         // <= 64 n-tiles of V per CTA in shared memory
-                const dim3 grid(gx, (unsigned)((n_tiles + tpc - 1) / tpc));
-                const size_t smem = (size_t)tpc * 8 * kExpandVPitch * sizeof(double);
-                const double *sd = (const double *)s, *Vd = (const double *)V;
 #define GPDE_LAUNCH_EXPAND(KSV)                                                                                     \
     {                                                                                                               \
-        auto kern = vo_expand_dmma_kernel<KSV>;                                                                     \
+        auto kern = vo_expand_dmma_kernel<KSV, T>;                                                                  \
         GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
-        kern<<<grid, kExpandWarps * 32, smem, st>>>(sd, Vd, w, ldw, (long long)B, d, m, tpc);                       \
+        kern<<<grid, kExpandWarps * 32, smem, st>>>(s, V, w, ldw, (long long)B, d, m, tpc);                         \
     }
-                if (m <= 8) GPDE_LAUNCH_EXPAND(2)
-                else if (m <= 16) GPDE_LAUNCH_EXPAND(4)
-                else if (m <= 28) GPDE_LAUNCH_EXPAND(7)
-                else GPDE_LAUNCH_EXPAND(8)
+            if (m <= 8) GPDE_LAUNCH_EXPAND(2)
+            else if (m <= 16) GPDE_LAUNCH_EXPAND(4)
+            else if (m <= 28) GPDE_LAUNCH_EXPAND(7)
+            else GPDE_LAUNCH_EXPAND(8)
 #undef GPDE_LAUNCH_EXPAND
-                GPDE_CUDA_OK(cudaGetLastError());
-                if (lean) {
-                    const int rc2 = launch_grid2<double, double, double>(pl, (const double *)a, (long long)a_stride, a_is_log, w,
-                                                                         nullptr, 0, nullptr, 0, (double *)q, nullptr, d, 0, false,
-                                                                         (long long)B, st, ldw);
-                    if (rc2 != 0) return rc2 < 0 ? rc2 : GPDE_OK;
-                    return fail(GPDE_ERR_ARG, "vo_residual_T: lean grid kernel declined after setup");
-                }
-            } else {
+            GPDE_CUDA_OK(cudaGetLastError());
+        } else if constexpr (sizeof(T) == 8) {   // m > 32: the general FP64 GEMM, w [B,d] behind the padded operands
+            const int mp = gemm_dp(m), bn = 128, ldb = (d + bn - 1) / bn * bn;
+            double *Sp = (double *)workspace, *Vt = Sp + (size_t)B * mp;
+            w = Vt + (size_t)mp * ldb;
             {
                 const long long total = (long long)B * mp;
                 const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, (long long)pl->n_sm * 8);
-                vo_gemm_pad_rows_kernel<<<grid, 256, 0, st>>>((const double *)s, (long long)B, m, Sp, mp);
+                vo_gemm_pad_rows_kernel<<<grid, 256, 0, st>>>(s, (long long)B, m, Sp, mp);
                 vo_gemm_pack_transposed_kernel<<<dim3((unsigned)(ldb / 32), (unsigned)((mp + 31) / 32)), dim3(32, 8), 0, st>>>(
-                    (const double *)V, d, m, Vt, mp, ldb);
+                    V, d, m, Vt, mp, ldb);
             }
             {
                 auto kern = vo_gemm_kernel<128, double>;
@@ -1147,11 +970,11 @@ static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, i
                 kern<<<grid, kGemmThreads, smem, st>>>(Sp, mp, Vt, ldb, w, d, (long long)B, (double *)nullptr);
                 GPDE_CUDA_OK(cudaGetLastError());
             }
-            }
-            const int rc = launch_grid_rho(pl, (const double *)a, (long long)a_stride, a_is_log, w, nullptr, 0, (double *)q, d,
-                                           0, (long long)B, st);
-            if (rc != 0) return rc < 0 ? rc : GPDE_OK;
         }
+        const int rc = launch_grid2<T, double, T>(pl, a, (long long)a_stride, a_is_log, w, nullptr, 0, nullptr, 0, q, nullptr, d, 0,
+                                                  false, (long long)B, st, ldw);
+        if (rc != 0) return rc < 0 ? rc : GPDE_OK;
+        return fail(GPDE_ERR_ARG, "vo_residual_T: lean grid kernel declined after setup");
     }
     if (use_fused(pl) && sizeof(double) * kFS * (size_t)m <= sizeof(double) * kFS * kRhoPitch) {
         const unsigned grid = (unsigned)((B + kFS - 1) / kFS);
@@ -1261,13 +1084,11 @@ int gpde_vo_plan_create(gpde_vo_plan **plan, int n_nodes, int n_cells, const int
     if (e == cudaSuccess) e = track_vo(pl, &D.f_free, f_free);
     if (e == cudaSuccess) e = build_csr_terms(pl, n_cells, cell_dofs, Ke, cell_to_input, d, src);
     if (e == cudaSuccess) e = build_fused_tiles(pl, n_nodes, n_cells, cell_dofs, Ke, cell_to_input, d, src, f_free);
-    if (e == cudaSuccess)
-        e = build_grid_plan(pl, n_nodes, n_cells, cell_dofs, Ke, cell_to_input, n_inputs, free_dofs, d, bc_dofs, n_bc,
-                            f_free);
     if (e != cudaSuccess) {
         gpde_vo_plan_destroy(pl);
         return fail(GPDE_ERR_CUDA, "vo_plan_create: upload failed: %s", cudaGetErrorString(e));
     }
+    build_grid_plan(pl, n_nodes, n_cells, cell_dofs, Ke, cell_to_input, n_inputs, free_dofs, d, bc_dofs, n_bc, f_free);
     *plan = pl;
     return GPDE_OK;
 }
@@ -1290,15 +1111,12 @@ int gpde_vo_plan_info(const gpde_vo_plan *pl, int64_t out[8]) {
 
 int gpde_vo_plan_kernel_path(const gpde_vo_plan *pl, int m, int elem_bytes) {
     if (!pl) return fail(GPDE_ERR_ARG, "vo_plan_kernel_path: null");
-    if (elem_bytes == 8) {
-        if (m > 0 && m <= 32 && use_grid(pl)) return 2;
-        if (m > 32 && use_grid(pl)) return 3;
-    } else if (use_grid(pl)) {   // FP32 I/O: the lean kernel only (the reference's own meshes)
+    if (use_grid(pl)) {
         Grid2Dev G;
         int NT, NX;
         size_t smem;
-        if (m > 0 && m <= 32 && grid2_setup(pl, m, false, 1, G, NT, NX, smem, 4, 4)) return 2;
-        if (m > 32 && grid2_setup(pl, 0, true, 1, G, NT, NX, smem, 4, 4)) return 3;
+        if (m > 0 && m <= 32 && grid2_setup(pl, m, false, 1, G, NT, NX, smem, elem_bytes, elem_bytes)) return 2;
+        if (m > 32 && grid2_setup(pl, 0, true, 1, G, NT, NX, smem, elem_bytes, elem_bytes)) return 3;
     }
     if (m > 0 && m <= 32 && use_fused(pl)) return 1;
     return 0;
@@ -1316,8 +1134,8 @@ size_t gpde_vo_workspace_bytes(const gpde_vo_plan *pl, int64_t B, int m) {
         need = std::max(need, sizeof(double) * ((size_t)B * mp + mp * ldb + (size_t)B * pl->dev.d));
     }
     if (m > 32) need = std::max(need, gridgemm_workspace_bytes(pl, (long long)B, m));
-    if (pl->grid.ok && m > 0 && m <= 32) {   // packed V (+ the per-row tile masks of the lean kernel)
-        need = std::max(need, grid_packed_bytes(pl->grid, 4) + (size_t)(pl->grid.ny + 1) * kGrid2MaskBytes);
+    if (pl->grid.ok && m > 0 && m <= 32) {   // packed V rows of the lean kernel (NT = 4 n-tiles: the most m <= 32 takes)
+        need = std::max(need, (size_t)(pl->grid.ny + 1) * grid2_v_row_bytes(pl->grid.nx / 16, 4, 0));
         // packed V^T rows of the one-kernel transposed application (launch_grid2_wt): <= 8 k-steps
         need = std::max(need, (size_t)(pl->grid.ny + 1) * ((size_t)((pl->grid.nx + 15) / 16) * 2 * 8 * 256 + kGrid2MaskBytes));
     }

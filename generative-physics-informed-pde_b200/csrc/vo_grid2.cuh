@@ -1,12 +1,22 @@
-// Structured-grid virtual-observable residual kernel, lean variant (sm_100a).  Included by vo.cu after vo_grid.cuh.
+// Structured-grid virtual-observable residual kernel (sm_100a).  Included by vo.cu.
+//
+// When the fine mesh is the reference's own (pixels of two P1 triangles on an nx x ny grid,
+// factories/model.py:130-133; Dirichlet data on the left/right edges, LinearEllipticFactories.py:173-179,
+// 239-281) and the conductivity comes per pixel (bottleneck/utils.py:41-98), K_fom(a) is a 5-point
+// operator: the coupling of two horizontally adjacent nodes is chs * (a[pixel below] + a[pixel above]),
+// of two vertically adjacent ones cvs * (a[pixel left] + a[pixel right]); the hypotenuse couplings of
+// right-angled P1 triangles vanish.  gpde_vo_plan_create verifies this against the element data it is
+// given and otherwise leaves the generic kernels (vo_fused.cuh / version 1) in charge.
 //
 //   r[b,:] = V^T (K_fom(a_b) u~_b - f)_free        (VirtualObservables.py:61-69, 662, 990)
 //
-// Same algorithm and work decomposition as vo_grid.cuh (marching over node rows, flux form, the 4 values a lane
-// produces are its A fragments of mma.sync.m8n8k4.f64), specialised for the reference's own meshes so that the
-// inner loop carries no generality:
-//   * nx in {16, 32, 64, 128} pixels per row and an even number of pixel rows, no load vector
-//     (LinearEllipticFactories.py:165-171 is the zero load); anything else stays with vo_grid.cuh;
+// A CTA of 16 warps marches over the node rows bottom to top; warp (group, strip) = 8 samples x 16 node columns, lane
+// (s = lane/4, k = lane%4) owns 4 columns of sample s and keeps the row below in registers; flux form
+// S_i = rh (Fh_right - Fh_left) + (Fv_up - Fv_down), rho_i = cvs * S_i - f_i; the 4 values a lane produces ARE its A
+// fragments of four mma.sync.m8n8k4.f64 k-steps (M = 8 samples, K = 4 lanes' columns, N = 8 columns of V), the B
+// fragments come from a fragment-packed V row in shared memory.  The inner loop carries no generality:
+//   * nx in {16, 32, 64, 128} pixels per row and an even number of pixel rows (build_grid_plan in vo.cu), no load vector
+//     (LinearEllipticFactories.py:165-171 is the zero load; a plan with one is served here only when the call ignores it);
 //   * exactly one lane per warp row touches the left Dirichlet column and one the right one: two selects per
 //     row instead of per-column category decoding; no column masks; first and last node row peeled;
 //   * a stage = 2 node rows; every thread copies the same 4 + 4 16-byte pieces per stage (one piece position in
@@ -43,8 +53,43 @@ struct Grid2Dev {
     int stage_bytes, v_row_bytes;   // one a/y stage (all samples of the CTA); one packed V row
     int nvs;                        // V stages in the ring (2 or 3)
     int spc;                        // samples a CTA takes (<= 8 groups): group i gets [i spc / groups, (i + 1) spc / groups)
-    int flags;                      // experiment switches (GPDE_GRID2_FLAGS): none in use at present
 };
+
+__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void cp_async16_u32(unsigned smem_dst, const void *gmem_src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gmem_src) : "memory");
+}
+
+__device__ __forceinline__ void mbar_init(unsigned long long *bar, unsigned count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(unsigned long long *bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive_expect_tx(unsigned long long *bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(unsigned long long *bar, unsigned parity) {
+    const unsigned addr = smem_u32(bar);
+    unsigned done;
+    do {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+            "selp.u32 %0, 1, 0, p;\n\t}"
+            : "=r"(done)
+            : "r"(addr), "r"(parity)   // (a suspend-time hint made wake-ups ~10x slower on B200: measured, not used)
+            : "memory");
+        if (!done) __nanosleep(40);
+    } while (!done);
+}
+// global -> shared bulk copy (TMA engine, 1-D); bytes % 16 == 0, both addresses 16-byte aligned
+__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, unsigned bytes, unsigned long long *bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                     smem_u32(dst)),
+                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
+                 : "memory");
+}
 
 __device__ __forceinline__ void cp_async8_u32(unsigned smem_dst, const void *gmem_src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_dst), "l"(gmem_src) : "memory");
@@ -99,27 +144,9 @@ template <typename T> __device__ __forceinline__ double lds_elem(unsigned addr);
 template <> __device__ __forceinline__ double lds_elem<double>(unsigned addr) { return lds64(addr); }
 template <> __device__ __forceinline__ double lds_elem<float>(unsigned addr) { return (double)lds32f(addr); }
 
-// exp_tab16 (vo_grid.cuh) with its nine 64-bit constants read as constant-bank operands of the FP64 instructions instead
-// of being re-materialised into registers (two moves each) for every row
-__constant__ double kExpK[9] = {23.083120654223414, -0.04332169877307024, -1.1926343307941173e-11,
-                                1.38888888888888888889e-03, 8.33333333333333333333e-03, 4.16666666666666666667e-02,
-                                1.66666666666666666667e-01, 0.5, 1.0};
-__device__ __forceinline__ double exp_tab16c(double x, unsigned tab) {   // tab = shared-memory address of the 2^(j/16) table
-    const double t = fma(x, kExpK[0], 6755399441055744.0);   // 1.5*2^52: low word = rint(16 x / ln2)
-    const int ki = __double2loint(t);
-    const double kd = t - 6755399441055744.0;
-    double r = fma(kd, kExpK[1], x);
-    r = fma(kd, kExpK[2], r);
-    double p = kExpK[3];
-    p = fma(p, r, kExpK[4]);
-    p = fma(p, r, kExpK[5]);
-    p = fma(p, r, kExpK[6]);
-    p = fma(p, r, 0.5);
-    p = fma(p, r, 1.0);
-    p = fma(p, r, 1.0);
-    const double v = p * lds64(tab + ((ki << 3) & 0x78));
-    return __hiloint2double(__double2hiint(v) + ((ki << 16) & 0xfff00000), __double2loint(v));
-}
+// |x| <= 700 (false for NaN / inf) from the high word alone: integer pipe, no FP64 compare
+__device__ __forceinline__ int exp_arg_hi(double x) { return __double2hiint(x) & 0x7fffffff; }
+constexpr int kExpHiMax = 0x4085e000;   // high word of 700.0
 
 // V[d,m] row-major -> per node row t: [strip q][n-tile tt < NT][half ph < 2][lane][2], then [strip q][k][4] (NX = 1 only),
 // then one 32-bit mask per strip (8 words, 32 bytes).

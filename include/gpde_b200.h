@@ -159,8 +159,10 @@ int gpde_vo_plan_info(const gpde_vo_plan *plan, int64_t out[8]);
  * 3 = structured pixel grid, m > 32: V packing + ONE kernel that produces the fine residual inside the FP64 tensor-core
  *     contraction (vo_gridgemm.cuh) + the reduction of its partial tiles (three launches),
  * 2 = structured-grid kernel (V packing launch + one fused launch), 1 = generic fused kernel (one launch),
- * 0 = version-1 kernels (generic matvec + V padding + tensor-core contraction; three launches).  Informational (launch counting, tests); calls whose
- * pointers are not 16-byte aligned, that pass y = NULL or that ask for rho fall back from 2 to 1. */
+ * 0 = version-1 kernels (generic matvec + V padding + tensor-core contraction; three launches).  Informational (launch counting, tests).
+ * 2 and 3 need a pixel mesh of the lean grid kernel (nx in {16, 32, 64, 128}, even ny) without a load vector, and shared
+ * memory for the decomposition at elem_bytes; the load vector is assumed subtracted.  Calls whose pointers are not 16-byte
+ * aligned, that pass y = NULL or that ask for rho fall back from 2 to 1. */
 int gpde_vo_plan_kernel_path(const gpde_vo_plan *plan, int m, int elem_bytes);
 
 /* scratch bytes for residual / residual_T on B samples with m weighting functions */

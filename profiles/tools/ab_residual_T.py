@@ -10,7 +10,7 @@ from gpde_b200.VirtualObservables import VoPlan
 from gpde_b200.workloads import Workload
 name = sys.argv[1] if len(sys.argv) > 1 else "cfg2"
 B = int(sys.argv[2]) if len(sys.argv) > 2 else 4096
-extra = [dict(kv.split("=") for kv in spec.split(",")) for spec in sys.argv[3:]]   # e.g. GPDE_GRID2_FLAGS=2 GPDE_GRID2_NVS=2
+extra = [dict(kv.split("=") for kv in spec.split(",")) for spec in sys.argv[3:]]   # e.g. GPDE_GRID2_SPC=24
 dev = torch.device("cuda", 0)
 w = Workload(name, B=min(B, 4096), seed=0)
 base = VoPlan.cached(w.physics["fom"], dev, pixel_input=True)

@@ -1,5 +1,5 @@
 """VO residual at cfg2 with and without the in-kernel exp (a_is_log), and for m = 8 / 16 / 25: how the kernel time
-responds to removing instruction classes (a diagnostic for what bounds vo_grid_kernel)."""
+responds to removing instruction classes (a diagnostic for what bounds vo_grid2_kernel)."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch
