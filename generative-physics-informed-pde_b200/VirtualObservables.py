@@ -77,6 +77,7 @@ class VoPlan(object):
         self.n_nodes, self.n_cells, self.n_inputs, self.d, self.n_bc, self.slots_per_row = (int(v) for v in info[:6])
         self.fused_smem_bytes = int(info[7])   # 0: this mesh only runs on the unfused version-1 kernels
         self._scratch = None
+        self._grad_scratch = None
 
     def __del__(self):
         handle, self.handle = getattr(self, "handle", None), None
@@ -194,6 +195,42 @@ class VoPlan(object):
         _lib.check(rc, "gpde_vo_residual_T_" + sfx)
         return q
 
+    def residual_grad(self, a, y, g, V, gbar_r, *, a_is_log=True, want_grad_a=True, want_grad_g=False):
+        """(grad_a, grad_g): the gradient of L with dL/dr = gbar_r [B,m] through r = residual(a, y, g, V) with respect to
+        the conductivity input a and the Dirichlet values g (gpde_vo_residual_grad_*; r is linear in both, no solve):
+            grad_a[b,p] = sum_{cells c of input p} w~_b[c]^T K_c u~_b[c],   grad_g[b] = K_cf(a_b) w~_b,
+        w~_b = V gbar_r_b on the free dofs (0 on the Dirichlet dofs).  With ``a_is_log`` a = exp(x) and grad_a is the
+        gradient in x.  A gradient that is not wanted is None.  For a shared 1-D ``a`` or ``g`` the per-sample gradients
+        are summed over the batch.  The load vector does not enter."""
+        dt = a.dtype
+        sfx = _lib.suffix(dt)
+        dev = self.device
+        gbar_r = gbar_r.to(dt).contiguous()
+        B, m = int(gbar_r.shape[0]), int(gbar_r.shape[1])
+        sizes = [t.shape[0] for t in (y, a, g) if t is not None and t.dim() == 2]
+        if any(n != B for n in sizes):   # the kernels index every batched argument by the B of gbar_r
+            raise ValueError("inconsistent batch sizes %r among a, y, g and gbar_r (%d)" % (sizes, B))
+        a = a.contiguous()
+        y = None if y is None else y.to(dt).contiguous()
+        g = None if g is None else g.to(dt).contiguous()
+        Vc = V.to(dt).contiguous()
+        grad_a = a.new_empty((B, self.n_inputs)) if want_grad_a else None
+        grad_g = a.new_empty((B, self.n_bc)) if want_grad_g else None
+        if B:
+            need = max(16, int(self._lib.gpde_vo_grad_workspace_bytes(self.handle, B, m)))
+            if self._grad_scratch is None or self._grad_scratch.numel() < need:
+                self._grad_scratch = torch.empty(need, dtype=torch.uint8, device=dev)
+            fn = getattr(self._lib, "gpde_vo_residual_grad_" + sfx)
+            rc = fn(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
+                    _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), m,
+                    _lib.ptr(gbar_r, dev), _lib.ptr(grad_a, dev), _lib.ptr(grad_g, dev), _lib.ptr(self._grad_scratch, dev),
+                    B, _lib.stream_of(dev))
+            _lib.check(rc, "gpde_vo_residual_grad_" + sfx)
+        if grad_a is not None and a.dim() == 1:
+            grad_a = grad_a.sum(0)
+        if grad_g is not None and g is not None and g.dim() == 1:
+            grad_g = grad_g.sum(0)
+        return grad_a, grad_g
 
     def _weights_arg(self, V):
         """(contiguous float64 V, v_stride): [d,m] shared by the data points or [N,d,m] one matrix per data point."""
@@ -276,19 +313,32 @@ class PackedWeights(object):
 
 
 class VoResidualFn(torch.autograd.Function):
-    """r = V^T (K(a) u~ - f), differentiable in y: dL/dy = K_ff(a) V gbar_r (one residual_T launch)."""
+    """r = V^T (K(a) u~ - f), differentiable in y: dL/dy = K_ff(a) V gbar_r (one residual_T launch), in the
+    conductivity input a and in the Dirichlet values g (VoPlan.residual_grad).  V gets no gradient (None)."""
 
     @staticmethod
     def forward(ctx, y, a, g, V, plan, a_is_log):
         ctx.plan, ctx.a_is_log = plan, a_is_log
-        ctx.save_for_backward(a, V)
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            ctx.save_for_backward(a, V, y, g)
+        else:
+            ctx.save_for_backward(a, V)
         return plan.residual(a, y, g, V, a_is_log=a_is_log)
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, gbar_r):
-        a, V = ctx.saved_tensors
-        return ctx.plan.residual_T(a, V, gbar_r.contiguous(), a_is_log=ctx.a_is_log), None, None, None, None, None
+        a, V = ctx.saved_tensors[:2]
+        grad_y = grad_a = grad_g = None
+        if ctx.needs_input_grad[0]:
+            grad_y = ctx.plan.residual_T(a, V, gbar_r.contiguous(), a_is_log=ctx.a_is_log)
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            y, g = ctx.saved_tensors[2:]
+            grad_a, grad_g = ctx.plan.residual_grad(a, y, g, V, gbar_r, a_is_log=ctx.a_is_log,
+                                                    want_grad_a=ctx.needs_input_grad[1], want_grad_g=ctx.needs_input_grad[2])
+            if grad_g is not None:
+                grad_g = grad_g.to(g.dtype)
+        return grad_y, grad_a, grad_g, None, None, None
 
 
 def condition_gaussian(Gamma, alpha, noise_var, g, prec):

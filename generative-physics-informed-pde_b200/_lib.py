@@ -61,6 +61,11 @@ SIGNATURES = {
                                         c_vp]),
     "gpde_vo_residual_T_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_vo_residual_T_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_grad_workspace_bytes": (c_sz, [c_vp, c_i64, c_i32]),
+    "gpde_vo_residual_grad_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp,
+                                          c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_grad_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp,
+                                          c_vp, c_i64, c_vp]),
     "gpde_cg_init_f64": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_f64, c_i32, c_i64, c_i32, c_vp]),
     "gpde_cg_step_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i64, c_i32, c_vp]),
 }

@@ -49,6 +49,7 @@ constexpr int kVoThreads = 256;
 #include "vo_gridgemm.cuh"
 #include "vo_posterior.cuh"
 #include "vo_energy.cuh"
+#include "vo_grad.cuh"
 
 namespace gpde {
 // A pixel mesh the structured-grid kernels (vo_grid2.cuh) serve, verified by build_grid_plan.
@@ -90,6 +91,7 @@ struct gpde_vo_plan {
     gpde::VoTiles tiles;
     gpde::GridDev grid;
     gpde::VoCsrDev csr;     // K_ff as CSR term lists (vo_posterior.cuh)
+    gpde::VoGradDev grad;   // input -> cells lists and the Dirichlet rows of K (vo_grad.cuh)
     size_t fused_smem;
     int device;
     int n_sm;
@@ -313,15 +315,17 @@ static cudaError_t build_fused_tiles(gpde_vo_plan *pl, int n_nodes, int n_cells,
 }
 
 
-// K_ff(a) as CSR over the free dofs with, per stored entry, the list of (conductivity input, element-matrix entry) terms:
-// K_ij(a) = sum_t a[term_in[t]] * term_coef[t].  Used by the batched posterior update (vo_posterior.cuh).
-static cudaError_t build_csr_terms(gpde_vo_plan *pl, int n_cells, const int32_t *cell_dofs, const double *Ke,
-                                   const int32_t *cell_to_input, int d, const std::vector<int> &src) {
+// Rows of K(a) over the free columns as CSR with, per stored entry, the list of (conductivity input, element-matrix entry)
+// terms: K_ij(a) = sum_t a[term_in[t]] * term_coef[t].  row_of[node] = the node's row (< 0: not a row).  The free rows
+// (K_ff) serve the batched posterior update (vo_posterior.cuh), the Dirichlet rows (K_cf) the gradient in g (vo_grad.cuh).
+static cudaError_t build_csr_terms(gpde_vo_plan *pl, VoCsrDev &C, int d, const std::vector<int> &row_of, int n_cells,
+                                   const int32_t *cell_dofs, const double *Ke, const int32_t *cell_to_input,
+                                   const std::vector<int> &src) {
     struct Term { int in; double coef; };
     std::vector<std::vector<std::pair<int, std::vector<Term>>>> rows(d);
     for (int c = 0; c < n_cells; ++c)
         for (int l = 0; l < 3; ++l) {
-            const int i = src[cell_dofs[3 * c + l]];
+            const int i = row_of[cell_dofs[3 * c + l]];
             if (i < 0) continue;
             for (int l2 = 0; l2 < 3; ++l2) {
                 const int j = src[cell_dofs[3 * c + l2]];
@@ -353,13 +357,34 @@ static cudaError_t build_csr_terms(gpde_vo_plan *pl, int n_cells, const int32_t 
         row_ptr[i + 1] = (int)col.size();
         max_row = std::max(max_row, row_ptr[i + 1] - row_ptr[i]);
     }
-    VoCsrDev &C = pl->csr;
     C.d = d; C.nnz = (int)col.size(); C.max_row = max_row;
     cudaError_t e = track_vo(pl, &C.row_ptr, row_ptr);
     if (e == cudaSuccess) e = track_vo(pl, &C.col, col);
     if (e == cudaSuccess) e = track_vo(pl, &C.term_ptr, term_ptr);
     if (e == cudaSuccess) e = track_vo(pl, &C.term_in, term_in);
     if (e == cudaSuccess) e = track_vo(pl, &C.term_coef, term_coef);
+    return e;
+}
+
+// The cells of every conductivity input, ascending, with their dof sources and element matrices (vo_grad_cells_kernel).
+static cudaError_t build_grad_cells(gpde_vo_plan *pl, int n_cells, const int32_t *cell_dofs, const double *Ke,
+                                    const int32_t *cell_to_input, int n_inputs, const std::vector<int> &src) {
+    std::vector<int> in_ptr(n_inputs + 1, 0);
+    for (int c = 0; c < n_cells; ++c) in_ptr[cell_to_input[c] + 1]++;
+    for (int p = 0; p < n_inputs; ++p) in_ptr[p + 1] += in_ptr[p];
+    std::vector<int> next(in_ptr.begin(), in_ptr.end() - 1);
+    std::vector<int4> cell_src(n_cells);
+    std::vector<double> cell_K((size_t)n_cells * 9);
+    for (int c = 0; c < n_cells; ++c) {
+        const int e = next[cell_to_input[c]]++;
+        cell_src[e] = make_int4(src[cell_dofs[3 * c]], src[cell_dofs[3 * c + 1]], src[cell_dofs[3 * c + 2]], 0);
+        for (int k = 0; k < 9; ++k) cell_K[(size_t)e * 9 + k] = Ke[(size_t)c * 9 + k];
+    }
+    VoGradDev &G = pl->grad;
+    G.n_inputs = n_inputs;
+    cudaError_t e = track_vo(pl, &G.in_ptr, in_ptr);
+    if (e == cudaSuccess) e = track_vo(pl, &G.cell_src, cell_src);
+    if (e == cudaSuccess) e = track_vo(pl, &G.cell_K, cell_K);
     return e;
 }
 
@@ -909,6 +934,68 @@ static int vo_residual(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int
     return GPDE_OK;
 }
 
+// w = s V^T [B, ldw] in FP64 into `workspace` (16-byte aligned, >= expand_bytes): the first half of residual_T's two-kernel
+// route on pixel grids and of the residual gradient (vo_grad.cuh).  FP32 I/O: s and V converted on load.
+static size_t expand_bytes(const gpde_vo_plan *pl, long long B, int m) {
+    const size_t d = (size_t)pl->dev.d;
+    if (m <= 32) return sizeof(double) * (size_t)B * ((d + 3) & ~(size_t)3);
+    const size_t mp = (size_t)gemm_dp(m), ldb = (d + 127) / 128 * 128;
+    return sizeof(double) * ((size_t)B * mp + mp * ldb + (size_t)B * d);
+}
+template <typename T>
+static int launch_expand(const gpde_vo_plan *pl, const T *s, const T *V, int m, void *workspace, long long B, cudaStream_t st,
+                         double *&w, long long &ldw) {
+    const int d = pl->dev.d;
+    w = (double *)workspace;
+    ldw = d;
+    if (m <= 32) {   // contraction length m <= 32: one launch, operands read in place (vo_expand.cuh)
+        ldw = ((long long)d + 3) & ~3ll;
+        const int n_tiles = (d + 7) / 8;
+        const unsigned gx = (unsigned)((B + 8 * kExpandMT * kExpandWarps - 1) / (8 * kExpandMT * kExpandWarps));
+        const int nch = std::max(1, std::min(n_tiles, (int)(4 * pl->n_sm / gx)));
+        const int tpc = std::min((n_tiles + nch - 1) / nch, 64);         // <= 64 n-tiles of V per CTA in shared memory
+        const dim3 grid(gx, (unsigned)((n_tiles + tpc - 1) / tpc));
+        const size_t smem = (size_t)tpc * 8 * kExpandVPitch * sizeof(double);
+#define GPDE_LAUNCH_EXPAND(KSV)                                                                                     \
+    {                                                                                                           \
+        auto kern = vo_expand_dmma_kernel<KSV, T>;                                                              \
+        GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));       \
+        kern<<<grid, kExpandWarps * 32, smem, st>>>(s, V, w, ldw, (long long)B, d, m, tpc);                     \
+    }
+        if (m <= 8) GPDE_LAUNCH_EXPAND(2)
+        else if (m <= 16) GPDE_LAUNCH_EXPAND(4)
+        else if (m <= 28) GPDE_LAUNCH_EXPAND(7)
+        else GPDE_LAUNCH_EXPAND(8)
+#undef GPDE_LAUNCH_EXPAND
+        GPDE_CUDA_OK(cudaGetLastError());
+    } else if constexpr (sizeof(T) == 8) {   // m > 32: the general FP64 GEMM, w [B,d] behind the padded operands
+        const int mp = gemm_dp(m), bn = 128, ldb = (d + bn - 1) / bn * bn;
+        double *Sp = (double *)workspace, *Vt = Sp + (size_t)B * mp;
+        w = Vt + (size_t)mp * ldb;
+        {
+            const long long total = (long long)B * mp;
+            const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, (long long)pl->n_sm * 8);
+            vo_gemm_pad_rows_kernel<<<grid, 256, 0, st>>>(s, (long long)B, m, Sp, mp);
+            vo_gemm_pack_transposed_kernel<<<dim3((unsigned)(ldb / 32), (unsigned)((mp + 31) / 32)), dim3(32, 8), 0, st>>>(
+                V, d, m, Vt, mp, ldb);
+        }
+        {
+            auto kern = vo_gemm_kernel<128, double>;
+            const size_t smem = gemm_smem(bn);
+            GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            dim3 grid((unsigned)((B + kGemmBM - 1) / kGemmBM), (unsigned)(ldb / bn));
+            kern<<<grid, kGemmThreads, smem, st>>>(Sp, mp, Vt, ldb, w, d, (long long)B, (double *)nullptr);
+            GPDE_CUDA_OK(cudaGetLastError());
+        }
+    } else {   // m > 32 with FP32 I/O
+        const long long total = B * (long long)d;
+        const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, (long long)pl->n_sm * 16);
+        vo_expand_kernel<T><<<grid, 256, 0, st>>>(s, V, w, B, d, m);
+        GPDE_CUDA_OK(cudaGetLastError());
+    }
+    return GPDE_OK;
+}
+
 template <typename T>
 static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *V, int m,
                          const T *s, T *q, void *workspace, int64_t B, gpde_stream_t stream) {
@@ -929,48 +1016,10 @@ static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, i
     if (use_grid(pl) && (m <= 32 || sizeof(T) == 8) && grid2_a_aligned(pl, a, (long long)a_stride, (int)sizeof(T)) &&
         !((uintptr_t)workspace & 15) && grid2_setup(pl, 0, true, 0, G2, nt2, nx2, smem2, (int)sizeof(T), 8)) {
         const int d = pl->dev.d;
-        double *w = (double *)workspace;
-        long long ldw = d;
-        if (m <= 32) {   // contraction length m <= 32: one launch, operands read in place (vo_expand.cuh)
-            ldw = ((long long)d + 3) & ~3ll;
-            const int n_tiles = (d + 7) / 8;
-            const unsigned gx = (unsigned)((B + 8 * kExpandMT * kExpandWarps - 1) / (8 * kExpandMT * kExpandWarps));
-            const int nch = std::max(1, std::min(n_tiles, (int)(4 * pl->n_sm / gx)));
-            const int tpc = std::min((n_tiles + nch - 1) / nch, 64);         // <= 64 n-tiles of V per CTA in shared memory
-            const dim3 grid(gx, (unsigned)((n_tiles + tpc - 1) / tpc));
-            const size_t smem = (size_t)tpc * 8 * kExpandVPitch * sizeof(double);
-#define GPDE_LAUNCH_EXPAND(KSV)                                                                                     \
-    {                                                                                                               \
-        auto kern = vo_expand_dmma_kernel<KSV, T>;                                                                  \
-        GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
-        kern<<<grid, kExpandWarps * 32, smem, st>>>(s, V, w, ldw, (long long)B, d, m, tpc);                         \
-    }
-            if (m <= 8) GPDE_LAUNCH_EXPAND(2)
-            else if (m <= 16) GPDE_LAUNCH_EXPAND(4)
-            else if (m <= 28) GPDE_LAUNCH_EXPAND(7)
-            else GPDE_LAUNCH_EXPAND(8)
-#undef GPDE_LAUNCH_EXPAND
-            GPDE_CUDA_OK(cudaGetLastError());
-        } else if constexpr (sizeof(T) == 8) {   // m > 32: the general FP64 GEMM, w [B,d] behind the padded operands
-            const int mp = gemm_dp(m), bn = 128, ldb = (d + bn - 1) / bn * bn;
-            double *Sp = (double *)workspace, *Vt = Sp + (size_t)B * mp;
-            w = Vt + (size_t)mp * ldb;
-            {
-                const long long total = (long long)B * mp;
-                const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, (long long)pl->n_sm * 8);
-                vo_gemm_pad_rows_kernel<<<grid, 256, 0, st>>>(s, (long long)B, m, Sp, mp);
-                vo_gemm_pack_transposed_kernel<<<dim3((unsigned)(ldb / 32), (unsigned)((mp + 31) / 32)), dim3(32, 8), 0, st>>>(
-                    V, d, m, Vt, mp, ldb);
-            }
-            {
-                auto kern = vo_gemm_kernel<128, double>;
-                const size_t smem = gemm_smem(bn);
-                GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                dim3 grid((unsigned)((B + kGemmBM - 1) / kGemmBM), (unsigned)(ldb / bn));
-                kern<<<grid, kGemmThreads, smem, st>>>(Sp, mp, Vt, ldb, w, d, (long long)B, (double *)nullptr);
-                GPDE_CUDA_OK(cudaGetLastError());
-            }
-        }
+        double *w;
+        long long ldw;
+        const int rce = launch_expand<T>(pl, s, V, m, workspace, (long long)B, st, w, ldw);
+        if (rce != GPDE_OK) return rce;
         const int rc = launch_grid2<T, double, T>(pl, a, (long long)a_stride, a_is_log, w, nullptr, 0, nullptr, 0, q, nullptr, d, 0,
                                                   false, (long long)B, st, ldw);
         if (rc != 0) return rc < 0 ? rc : GPDE_OK;
@@ -992,6 +1041,57 @@ static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, i
     GPDE_CUDA_OK(cudaGetLastError());
     return launch_matvec<T, double, T>(pl, a, a_stride, a_is_log, w, (const T *)nullptr, 0, 0, (double *)nullptr, 0,
                                        q, B, st);
+}
+
+// gpde_vo_residual_grad_*: w = gbar_r V^T, then grad_a (marching kernel on pixel grids, per-input cell lists otherwise)
+// and grad_g (Dirichlet rows of K(a)).  The kernel choice depends on the plan only.
+template <typename T>
+static int vo_residual_grad(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *y, const T *g,
+                            int64_t g_stride, const T *V, int m, const T *gbar_r, T *grad_a, T *grad_g, void *workspace,
+                            int64_t B, gpde_stream_t stream) {
+    if (!pl || B < 0) return fail(GPDE_ERR_ARG, "vo_residual_grad: bad argument (null plan or B < 0)");
+    if (m <= 0) return fail(GPDE_ERR_ARG, "vo_residual_grad: m = %d weighting functions (must be > 0)", m);
+    if (a_stride != 0 && a_stride != pl->dev.n_inputs)
+        return fail(GPDE_ERR_ARG, "vo_residual_grad: a_stride must be 0 or n_inputs = %d", pl->dev.n_inputs);
+    if (g_stride != 0 && g_stride != pl->dev.n_bc)
+        return fail(GPDE_ERR_ARG, "vo_residual_grad: g_stride must be 0 or n_bc = %d", pl->dev.n_bc);
+    if (B == 0) return GPDE_OK;
+    if (!V || !gbar_r) return fail(GPDE_ERR_ARG, "vo_residual_grad: V and gbar_r are required");
+    if (!a) return fail(GPDE_ERR_ARG, "vo_residual_grad: null conductivity field");
+    if (!workspace || ((uintptr_t)workspace & 15))
+        return fail(GPDE_ERR_ARG, "vo_residual_grad: workspace must be non-NULL and 16-byte aligned "
+                                  "(>= gpde_vo_grad_workspace_bytes)");
+    if (!grad_a && !grad_g) return GPDE_OK;
+    DeviceGuard guard(pl->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    double *w;
+    long long ldw;
+    const int rce = launch_expand<T>(pl, gbar_r, V, m, workspace, (long long)B, st, w, ldw);
+    if (rce != GPDE_OK) return rce;
+    const int d = pl->dev.d;
+    if (grad_a && pl->grid.ok) {
+        const GridDev &G = pl->grid;
+        const long long total = (long long)B * G.nx;
+        const unsigned grid = (unsigned)std::min<long long>((total + kGradThreads - 1) / kGradThreads, (long long)pl->n_sm * 8);
+        vo_grad_grid_kernel<T><<<grid, kGradThreads, 0, st>>>(G.nx, G.ny, G.in0, G.sy, -G.rh * G.scale, -G.scale, a,
+                                                                (long long)a_stride, a_is_log, y, d, g, (long long)g_stride,
+                                                                w, ldw, grad_a, (long long)B);
+        GPDE_CUDA_OK(cudaGetLastError());
+    } else if (grad_a) {
+        const long long total = (long long)B * pl->dev.n_inputs;
+        const unsigned grid = (unsigned)std::min<long long>((total + kGradThreads - 1) / kGradThreads, (long long)pl->n_sm * 16);
+        vo_grad_cells_kernel<T><<<grid, kGradThreads, 0, st>>>(pl->grad, a, (long long)a_stride, a_is_log, y, d, g,
+                                                                 (long long)g_stride, w, ldw, grad_a, (long long)B);
+        GPDE_CUDA_OK(cudaGetLastError());
+    }
+    if (grad_g && pl->dev.n_bc > 0) {
+        const long long total = (long long)B * pl->dev.n_bc;
+        const unsigned grid = (unsigned)std::min<long long>((total + kGradThreads - 1) / kGradThreads, (long long)pl->n_sm * 16);
+        vo_grad_g_kernel<T><<<grid, kGradThreads, 0, st>>>(pl->grad.bc_rows, a, (long long)a_stride, a_is_log, w, ldw, grad_g,
+                                                             (long long)B);
+        GPDE_CUDA_OK(cudaGetLastError());
+    }
+    return GPDE_OK;
 }
 
 // gpde_vo_energy_step_f64 for MP = 32 or 64 (vo_energy.cuh)
@@ -1082,7 +1182,16 @@ int gpde_vo_plan_create(gpde_vo_plan **plan, int n_nodes, int n_cells, const int
     if (e == cudaSuccess) e = track_vo(pl, &D.ell_c1, c1);
     if (e == cudaSuccess) e = track_vo(pl, &D.ell_c2, c2);
     if (e == cudaSuccess) e = track_vo(pl, &D.f_free, f_free);
-    if (e == cudaSuccess) e = build_csr_terms(pl, n_cells, cell_dofs, Ke, cell_to_input, d, src);
+    if (e == cudaSuccess) {
+        std::vector<int> free_row(n_nodes), bc_row(n_nodes);
+        for (int v = 0; v < n_nodes; ++v) {
+            free_row[v] = src[v] >= 0 ? src[v] : -1;
+            bc_row[v] = src[v] < 0 ? -src[v] - 1 : -1;
+        }
+        e = build_csr_terms(pl, pl->csr, d, free_row, n_cells, cell_dofs, Ke, cell_to_input, src);
+        if (e == cudaSuccess) e = build_csr_terms(pl, pl->grad.bc_rows, n_bc, bc_row, n_cells, cell_dofs, Ke, cell_to_input, src);
+    }
+    if (e == cudaSuccess) e = build_grad_cells(pl, n_cells, cell_dofs, Ke, cell_to_input, n_inputs, src);
     if (e == cudaSuccess) e = build_fused_tiles(pl, n_nodes, n_cells, cell_dofs, Ke, cell_to_input, d, src, f_free);
     if (e != cudaSuccess) {
         gpde_vo_plan_destroy(pl);
@@ -1140,6 +1249,11 @@ size_t gpde_vo_workspace_bytes(const gpde_vo_plan *pl, int64_t B, int m) {
         need = std::max(need, (size_t)(pl->grid.ny + 1) * ((size_t)((pl->grid.nx + 15) / 16) * 2 * 8 * 256 + kGrid2MaskBytes));
     }
     return need;
+}
+
+size_t gpde_vo_grad_workspace_bytes(const gpde_vo_plan *pl, int64_t B, int m) {
+    if (!pl || B < 0 || m <= 0) return 0;
+    return expand_bytes(pl, (long long)B, m);
 }
 
 int gpde_vo_pack_weights_f64(const gpde_vo_plan *pl, const double *V, int m, int flags, void *workspace,
@@ -1254,6 +1368,17 @@ int gpde_vo_residual_T_f64(const gpde_vo_plan *pl, const double *a, int64_t a_st
 int gpde_vo_residual_T_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *V,
                            int m, const float *s, float *q, void *workspace, int64_t B, gpde_stream_t stream) {
     return vo_residual_T<float>(pl, a, a_stride, a_is_log, V, m, s, q, workspace, B, stream);
+}
+
+int gpde_vo_residual_grad_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *y,
+                              const double *g, int64_t g_stride, const double *V, int m, const double *gbar_r, double *grad_a,
+                              double *grad_g, void *workspace, int64_t B, gpde_stream_t stream) {
+    return vo_residual_grad<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, m, gbar_r, grad_a, grad_g, workspace, B, stream);
+}
+int gpde_vo_residual_grad_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *y,
+                              const float *g, int64_t g_stride, const float *V, int m, const float *gbar_r, float *grad_a,
+                              float *grad_g, void *workspace, int64_t B, gpde_stream_t stream) {
+    return vo_residual_grad<float>(pl, a, a_stride, a_is_log, y, g, g_stride, V, m, gbar_r, grad_a, grad_g, workspace, B, stream);
 }
 
 }  // extern "C"

@@ -249,6 +249,28 @@ int gpde_vo_residual_T_f32(const gpde_vo_plan *plan, const float *a, int64_t a_s
                            const float *V, int m, const float *s, float *q, void *workspace,
                            int64_t B, gpde_stream_t stream);
 
+/* Gradient of r = gpde_vo_residual_*(a, y, g, V) with respect to the conductivity input and the Dirichlet values, for
+ * an incoming gradient gbar_r [B,m].  With w~_b = V gbar_r_b on the free dofs and 0 on the Dirichlet dofs, and since
+ * K(a) = sum_c a[cell_to_input[c]] K_c is linear in a:
+ *     grad_a[b,p] = sum_{c : cell_to_input[c] = p} w~_b[c]^T K_c u~_b[c]     ([c] = the three dofs of cell c)
+ *     grad_g[b,k] = (K_cf(a_b) w~_b)_k                                       (the Dirichlet rows of K(a) applied to w~)
+ * a_is_log != 0: a holds x with a = exp(x) (no offset), and grad_a is the gradient in x: exp(x) times the above.
+ * The load vector does not enter either gradient.  Arguments as for gpde_vo_residual_*: a [B or 1, n_inputs]
+ * (a_stride = n_inputs or 0), y [B,d] (NULL = zeros), g [B or 1, n_bc] (g_stride = n_bc or 0, NULL = zeros), V [d,m].
+ * Outputs are per sample even when a_stride or g_stride is 0: grad_a [B,n_inputs], grad_g [B,n_bc]; either may be NULL.
+ * workspace: >= gpde_vo_grad_workspace_bytes(plan, B, m), 16-byte aligned (it holds w = gbar_r V^T in FP64; FP32 I/O
+ * computes in FP64 too).  B = 0 is a no-op.  m <= 0, a NULL gbar_r, V or a, a bad stride or a NULL or misaligned
+ * workspace return GPDE_ERR_ARG.  Every output is written by one thread in a fixed order: results are deterministic. */
+size_t gpde_vo_grad_workspace_bytes(const gpde_vo_plan *plan, int64_t B, int m);
+int gpde_vo_residual_grad_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
+                              const double *y, const double *g, int64_t g_stride, const double *V, int m,
+                              const double *gbar_r, double *grad_a, double *grad_g, void *workspace,
+                              int64_t B, gpde_stream_t stream);
+int gpde_vo_residual_grad_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
+                              const float *y, const float *g, int64_t g_stride, const float *V, int m,
+                              const float *gbar_r, float *grad_a, float *grad_g, void *workspace,
+                              int64_t B, gpde_stream_t stream);
+
 /* ---- fine-mesh label solves: batched preconditioned CG (setup-time replacement of the per-sample FEniCS / spsolve calls
  * of physics/LinearElliptic.py:85-101, 120-133 in utils/data.py:96-99).  One iteration = one gpde_vo_residual_f64 call with
  * y = p (rho output, flags bit0, no Dirichlet data: rho = K_ff(a) p for the whole batch) + one gpde_cg_step_f64 call.
