@@ -259,9 +259,32 @@ class VoPlan(object):
         _lib.check(rc, "gpde_vo_posterior_f64")
         return mean, vars_
 
+    def posterior_blocked(self, a, V, rho, noise_var, g, prec, info=None):
+        """``posterior`` for 1 <= m <= 256 (gpde_vo_posterior_blocked_f64): Lambda_n and L_n^-1 live in a workspace this call
+        allocates (about 1 MB per data point at m = 256) instead of shared memory; three launches for all data points."""
+        dev = self.device
+        N = int(g.shape[0])
+        a = a.to(torch.float64).contiguous()
+        V, v_stride, m = self._weights_arg(V)
+        rho, g, prec = (t.to(torch.float64).contiguous() for t in (rho, g, prec))
+        noise_var = noise_var.to(torch.float64).contiguous()
+        mean, vars_ = torch.empty_like(g), torch.empty_like(g)
+        need = int(self._lib.gpde_vo_posterior_blocked_workspace_bytes(self.handle, N, m))
+        ws = torch.empty(max(need, 16), dtype=torch.uint8, device=dev)
+        rc = self._lib.gpde_vo_posterior_blocked_f64(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0,
+                                                     _lib.ptr(V, dev), v_stride, m, _lib.ptr(rho, dev),
+                                                     _lib.ptr(noise_var, dev), _lib.ptr(g, dev), _lib.ptr(prec, dev),
+                                                     _lib.ptr(mean, dev), _lib.ptr(vars_, dev), _lib.ptr(info, dev),
+                                                     _lib.ptr(ws, dev), need, N, _lib.stream_of(dev))
+        _lib.check(rc, "gpde_vo_posterior_blocked_f64")
+        return mean, vars_
+
+    def posterior_blocked_workspace_bytes(self, N, m):
+        return int(self._lib.gpde_vo_posterior_blocked_workspace_bytes(self.handle, int(N), int(m)))
+
     def moments(self, a, V, rho, v):
         """(r [N,m], s2 [N,m]) = (V_n^T rho_n, sum_i Gamma_n[:,i]^2 v[n,i]) for all data points in one launch
-        (gpde_vo_moments_f64): the two terms of the precision hyper-update (VirtualObservables.py:985-990)."""
+        (gpde_vo_moments_f64, m <= 256): the two terms of the precision hyper-update (VirtualObservables.py:985-990)."""
         dev = self.device
         N = int(rho.shape[0])
         a = a.to(torch.float64).contiguous()
@@ -890,13 +913,18 @@ class VirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
       update_vo_precision  rho(mean) -> gpde_vo_moments_f64 -> sum  (2 launches + one [N,m] reduction)
       residuals            one residual launch
 
-    all matrix-free on the samplers' weighting matrices V (no dense Gamma [N,m,d]).  Ensembles that contain samplers
-    without a weighting matrix (flux constraints) or more than 64 virtual observables per data point condition densely
-    (``condition_gaussian``: torch / cuBLAS / cuSOLVER), chunked by ``max_stack_bytes``."""
+    all matrix-free on the samplers' weighting matrices V (no dense Gamma [N,m,d]).  Up to ``max_kernel_m`` = 64 virtual
+    observables per data point the update is one posterior launch; up to ``max_blocked_m`` = 256 it is the blocked route
+    (gpde_vo_posterior_blocked_f64: three launches, Lambda_n in a device workspace, data points chunked so that the
+    workspace stays within ``max_stack_bytes``).  Ensembles that contain samplers without a weighting matrix (flux
+    constraints) or more than 256 virtual observables per data point condition densely (``condition_gaussian``: torch /
+    cuBLAS / cuSOLVER), chunked by ``max_stack_bytes``.  ``last_update_route`` says which route the last update took:
+    "kernel", "blocked" or "dense"."""
 
-    # per-chunk budget for the stacked Gamma [n,m,d] of the dense route
+    # per-chunk budget for the stacked Gamma [n,m,d] of the dense route and the workspace of the blocked route
     max_stack_bytes = 1 << 30
     max_kernel_m = 64
+    max_blocked_m = 256
 
     def __init__(self, QuerryPointEnsemble, QuerryEnsemble, dtype, device):
         vos = [VirtualObservable(q, qp, dtype=dtype, device=device) for q, qp in zip(QuerryEnsemble, QuerryPointEnsemble)]
@@ -913,6 +941,7 @@ class VirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
         self._resident = None
         self._post, self._post_gen, self._members_dirty = None, 0, False
         self._info = None
+        self.last_update_route = None
         for k, vo in enumerate(self._virtual_observables):
             vo._ens, vo._k = self, k
 
@@ -961,12 +990,13 @@ class VirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
             self._resident = (plan, a, qpe.dirichlet_values(_F64, self.device))
         return self._resident
 
-    def _weights(self):
+    def _weights(self, max_m=None):
         """Weighting matrices of the data points for the batched kernels: one shared [d,m] tensor (every LinearQuerry holds
         the SAME tensor: V = W of the coarse-grained-residual sampler) or the stack [N,d,m]; None when some data point has
-        no weighting matrix or m exceeds the kernels' limit (dense route).  The stack is rebuilt after resample()."""
+        no weighting matrix or m exceeds ``max_m`` (default ``max_kernel_m``; dense route).  The stack is rebuilt after
+        resample()."""
         Vs = [vo.querry.V for vo in self._virtual_observables]
-        if any(v is None for v in Vs) or Vs[0].shape[1] > self.max_kernel_m:
+        if any(v is None for v in Vs) or Vs[0].shape[1] > (self.max_kernel_m if max_m is None else max_m):
             return None
         if all(v is Vs[0] for v in Vs):
             return Vs[0]
@@ -1023,15 +1053,22 @@ class VirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
     def update(self, G, PREC, iteration, writer=None):
         self.update_vo_precision(iteration, writer)
         G64, P64 = _as_f64(G, self.device), _as_f64(PREC, self.device)
-        V = self._weights()
+        V = self._weights(max(self.max_kernel_m, self.max_blocked_m))
         if V is not None:
             plan, a, _ = self._inputs()
             if self._info is None:
                 self._info = torch.zeros(1, dtype=torch.int32, device=self.device)
-            mean, vars_ = plan.posterior(a, V, self._fine_residual(G64), self._mean_vo_variances, G64, P64, info=self._info)
+            rho = self._fine_residual(G64)
+            if self.m <= self.max_kernel_m:
+                mean, vars_ = plan.posterior(a, V, rho, self._mean_vo_variances, G64, P64, info=self._info)
+                self.last_update_route = "kernel"
+            else:
+                mean, vars_ = self._posterior_blocked(plan, a, V, rho, G64, P64)
+                self.last_update_route = "blocked"
             self._post, self._members_dirty = (mean, vars_), False
             self._post_gen += 1
         else:
+            self.last_update_route = "dense"
             vos = self._virtual_observables
             per = 8 * self.m * self.dim_out
             step = max(1, int(self.max_stack_bytes // max(per, 1)))
@@ -1045,6 +1082,20 @@ class VirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
                     vo._set_posterior(mean[k], vars_[k])
         self.flush_cache()
 
+    def _posterior_blocked(self, plan, a, V, rho, G64, P64):
+        """The blocked route over chunks of data points whose workspace fits ``max_stack_bytes``."""
+        N = self.N
+        per = max(1, plan.posterior_blocked_workspace_bytes(1, self.m))     # the most bytes per data point (most row segments)
+        step = max(1, int(self.max_stack_bytes // per))
+        if step >= N:
+            return plan.posterior_blocked(a, V, rho, self._mean_vo_variances, G64, P64, info=self._info)
+        mean, vars_ = torch.empty_like(G64), torch.empty_like(G64)
+        for lo in range(0, N, step):
+            sl = slice(lo, lo + step)
+            mean[sl], vars_[sl] = plan.posterior_blocked(a[sl] if a.dim() == 2 else a, V[sl] if V.dim() == 3 else V, rho[sl],
+                                                         self._mean_vo_variances, G64[sl], P64[sl], info=self._info)
+        return mean, vars_
+
     @torch.no_grad()
     def update_vo_precision(self, iteration, writer=None):
         if not self._precision_initialized:
@@ -1054,7 +1105,7 @@ class VirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
             raise RuntimeError
         if self.fixed_precision:
             return
-        V = self._weights()
+        V = self._weights(max(self.max_kernel_m, self.max_blocked_m))
         if V is not None:     # VirtualObservables.py:985-990 for all data points: two launches and one reduction
             plan, a, _ = self._inputs()
             mean, vars_ = _as_f64(self._stacked("mean"), self.device), _as_f64(self._stacked("vars"), self.device)

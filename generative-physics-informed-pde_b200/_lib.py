@@ -56,6 +56,9 @@ SIGNATURES = {
     "gpde_vo_pack_weights_f64": (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_vp]),
     "gpde_vo_pack_weights_f32": (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_vp]),
     "gpde_vo_posterior_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_posterior_blocked_workspace_bytes": (c_sz, [c_vp, c_i64, c_i32]),
+    "gpde_vo_posterior_blocked_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                              c_vp, c_vp, c_sz, c_i64, c_vp]),
     "gpde_vo_moments_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_vo_energy_step_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64,
                                         c_vp]),

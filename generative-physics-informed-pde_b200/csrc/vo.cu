@@ -48,6 +48,7 @@ constexpr int kVoThreads = 256;
 #include "vo_gemm.cuh"
 #include "vo_gridgemm.cuh"
 #include "vo_posterior.cuh"
+#include "vo_posterior_blocked.cuh"
 #include "vo_energy.cuh"
 #include "vo_grad.cuh"
 
@@ -1311,10 +1312,66 @@ int gpde_vo_posterior_f64(const gpde_vo_plan *pl, const double *a, int64_t a_str
     return GPDE_OK;
 }
 
+// Layout of the blocked posterior's workspace (vo_posterior_blocked.cuh) for N data points: row segments S of the gram pass
+// so that about two waves of CTAs run (at most 8, at least 8 row tiles per segment), the same S for every data point.
+static gpde::BlkLayout blocked_layout(const gpde_vo_plan *pl, long long N, int m) {
+    using namespace gpde;
+    BlkLayout L;
+    L.mp = (m + kBlkTile - 1) / kBlkTile * kBlkTile;
+    L.nb = L.mp / kBlkTile;
+    L.nbt = L.nb * (L.nb + 1) / 2;
+    const long long ctas = std::max(1LL, N) * L.nbt, want = 2LL * pl->n_sm;
+    const int tiles = (pl->csr.d + kBlkRows - 1) / kBlkRows;
+    int S = ctas >= want ? 1 : (int)((want + ctas - 1) / ctas);
+    S = std::max(1, std::min({S, 8, tiles / 8}));
+    L.S = S;
+    L.seg = (long long)L.nbt * kBlkTile * kBlkTile + L.mp;
+    L.pa = std::max((long long)S * L.seg, (long long)L.mp * L.mp);
+    L.stride = L.pa + (long long)L.mp * L.mp + L.mp;
+    return L;
+}
+
+size_t gpde_vo_posterior_blocked_workspace_bytes(const gpde_vo_plan *pl, int64_t N, int m) {
+    if (!pl || N <= 0 || m <= 0 || m > 256) return 0;
+    return sizeof(double) * (size_t)blocked_layout(pl, (long long)N, m).stride * (size_t)N;
+}
+
+int gpde_vo_posterior_blocked_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, const double *V,
+                                  int64_t v_stride, int m, const double *rho, const double *noise_var, const double *g,
+                                  const double *prec, double *mean, double *vars, int *info, void *workspace,
+                                  size_t workspace_bytes, int64_t N, gpde_stream_t stream) {
+    if (!pl || N < 0 || m <= 0) return fail(GPDE_ERR_ARG, "vo_posterior_blocked: bad argument");
+    if (m > 256) return fail(GPDE_ERR_SIZE, "vo_posterior_blocked: m = %d > 256 weighting functions per data point", m);
+    if (N == 0) return GPDE_OK;
+    if (!a || !V || !rho || !noise_var || !g || !prec || !mean || !vars)
+        return fail(GPDE_ERR_ARG, "vo_posterior_blocked: null argument");
+    if (v_stride != 0 && v_stride != (int64_t)pl->dev.d * m)
+        return fail(GPDE_ERR_ARG, "vo_posterior_blocked: v_stride must be 0 or d*m");
+    const size_t need = gpde_vo_posterior_blocked_workspace_bytes(pl, N, m);
+    if (!workspace || ((uintptr_t)workspace & 15) || workspace_bytes < need)
+        return fail(GPDE_ERR_ARG, "vo_posterior_blocked: workspace must be 16-byte aligned and hold %zu bytes", need);
+    DeviceGuard guard(pl->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const BlkLayout Lo = blocked_layout(pl, (long long)N, m);
+    double *ws = (double *)workspace;
+    const size_t sm_gram = blk_gram_smem(pl->csr.max_row), sm_factor = blk_factor_smem(Lo.mp),
+                 sm_apply = blk_apply_smem(Lo.mp, pl->csr.max_row);
+    GPDE_CUDA_OK(cudaFuncSetAttribute(vo_post_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_gram));
+    GPDE_CUDA_OK(cudaFuncSetAttribute(vo_post_factor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_factor));
+    GPDE_CUDA_OK(cudaFuncSetAttribute(vo_post_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_apply));
+    vo_post_gram_kernel<<<dim3((unsigned)(Lo.nbt * Lo.S), (unsigned)N), kPostThreads, sm_gram, st>>>(
+        pl->csr, a, (long long)a_stride, V, (long long)v_stride, m, rho, prec, ws, Lo);
+    vo_post_factor_kernel<<<(unsigned)N, kPostThreads, sm_factor, st>>>(m, noise_var, ws, Lo, info);
+    vo_post_apply_kernel<<<dim3((unsigned)((pl->csr.d + kBlkRows - 1) / kBlkRows), (unsigned)N), kPostThreads, sm_apply, st>>>(
+        pl->csr, a, (long long)a_stride, V, (long long)v_stride, m, g, prec, ws, Lo, mean, vars);
+    GPDE_CUDA_OK(cudaGetLastError());
+    return GPDE_OK;
+}
+
 int gpde_vo_moments_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, const double *V, int64_t v_stride, int m,
                         const double *rho, const double *v, double *out_r, double *out_s2, int64_t N, gpde_stream_t stream) {
     if (!pl || N < 0 || m <= 0) return fail(GPDE_ERR_ARG, "vo_moments: bad argument");
-    if (m > 64) return fail(GPDE_ERR_SIZE, "vo_moments: m = %d > 64 weighting functions per data point", m);
+    if (m > 256) return fail(GPDE_ERR_SIZE, "vo_moments: m = %d > 256 weighting functions per data point", m);
     if (N == 0) return GPDE_OK;
     if (!a || !V || !rho || !v || !out_r || !out_s2) return fail(GPDE_ERR_ARG, "vo_moments: null argument");
     if (v_stride != 0 && v_stride != (int64_t)pl->dev.d * m) return fail(GPDE_ERR_ARG, "vo_moments: v_stride must be 0 or d*m");
@@ -1325,11 +1382,16 @@ int gpde_vo_moments_f64(const gpde_vo_plan *pl, const double *a, int64_t a_strid
         const size_t smem = moments_smem_bytes<32>(pl->csr.max_row);
         GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<(unsigned)N, kPostThreads, smem, st>>>(pl->csr, a, (long long)a_stride, V, (long long)v_stride, m, rho, v, out_r, out_s2);
-    } else {
+    } else if (m <= 64) {
         auto kern = vo_moments_kernel<64>;
         const size_t smem = moments_smem_bytes<64>(pl->csr.max_row);
         GPDE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<(unsigned)N, kPostThreads, smem, st>>>(pl->csr, a, (long long)a_stride, V, (long long)v_stride, m, rho, v, out_r, out_s2);
+    } else {     // one CTA per (64-column panel, data point)
+        const size_t smem = blk_moments_smem(pl->csr.max_row);
+        GPDE_CUDA_OK(cudaFuncSetAttribute(vo_moments_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        vo_moments_panel_kernel<<<dim3((unsigned)((m + kBlkTile - 1) / kBlkTile), (unsigned)N), kPostThreads, smem, st>>>(
+            pl->csr, a, (long long)a_stride, V, (long long)v_stride, m, rho, v, out_r, out_s2);
     }
     GPDE_CUDA_OK(cudaGetLastError());
     return GPDE_OK;

@@ -214,10 +214,23 @@ int gpde_vo_posterior_f64(const gpde_vo_plan *plan, const double *a, int64_t a_s
                           int64_t v_stride, int m, const double *rho, const double *noise_var, const double *g,
                           const double *prec, double *mean, double *vars, int *info, int64_t N, gpde_stream_t stream);
 
+/* The same conditioning for 1 <= m <= 256 (m > 256: GPDE_ERR_SIZE), blocked: Lambda_n and L_n^-1 (m x m, m padded to a
+ * multiple of 64) live in the caller's workspace instead of shared memory.  Three launches: the Gram blocks of Lambda_n
+ * over row tiles (DMMA), one Cholesky / triangular-inverse CTA per data point, and the mean / variance rows.  Arguments
+ * as gpde_vo_posterior_f64, plus workspace (16-byte aligned, device) of workspace_bytes >=
+ * gpde_vo_posterior_blocked_workspace_bytes(plan, N, m); a null, misaligned or smaller workspace returns GPDE_ERR_ARG.
+ * N = 0 is a no-op.  Results are deterministic for a given (plan, N, m): the row split of the Gram pass depends on N. */
+size_t gpde_vo_posterior_blocked_workspace_bytes(const gpde_vo_plan *plan, int64_t N, int m);
+int gpde_vo_posterior_blocked_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, const double *V,
+                                  int64_t v_stride, int m, const double *rho, const double *noise_var, const double *g,
+                                  const double *prec, double *mean, double *vars, int *info, void *workspace,
+                                  size_t workspace_bytes, int64_t N, gpde_stream_t stream);
+
 /* The two per-data-point terms of the precision hyper-update (VirtualObservablesEnsemble.update_vo_precision,
  * bottleneck/VirtualObservables.py:985-990), all data points at once:
  *     out_r [n,j] = (V_n^T rho_n)_j          = (Gamma_n mean_n - alpha_n)_j  for rho_n = rho(mean_n)
- *     out_s2[n,j] = sum_i Gamma_n[j,i]^2 v[n,i]                                                                  */
+ *     out_s2[n,j] = sum_i Gamma_n[j,i]^2 v[n,i]
+ * m <= 256 (else GPDE_ERR_SIZE); m > 64 runs one CTA per (64-column panel, data point).                           */
 int gpde_vo_moments_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, const double *V, int64_t v_stride,
                         int m, const double *rho, const double *v, double *out_r, double *out_s2, int64_t N,
                         gpde_stream_t stream);
