@@ -131,7 +131,8 @@ __device__ __forceinline__ int factor_band(const RomDev &P, int gl, double *Ab, 
             const int si = P.pair_si[q], sj = P.pair_sj[q];
             const double ci = Ab[(k + si) * bw1 + si];
             const double cj = Ab[(k + sj) * bw1 + sj];
-            Ab[(k + si) * bw1 + (si - sj)] -= ci * cj * invd;
+            // scaled before the product: ci * cj overflows once the entries pass ~1e154 (conductivities up to exp(709))
+            Ab[(k + si) * bw1 + (si - sj)] -= ci * (cj * invd);
         }
         if (z) {
             const double wk = z[k] * invd;

@@ -55,7 +55,11 @@ const char *gpde_last_error(void);
  * the device, in the sparse/banded form the kernels use.
  *   M_host   [n,n,E] row-major, M[:,:,e] = unit-conductivity stiffness of coarse cell e (ROM.py:46-53)
  *   bc_dofs  [n_bc]  constrained dofs (physics.constrained_dofs, ROM.py:14)
- * Free dofs are the remaining ones, ascending (optionally reordered to shrink the band). */
+ * Free dofs are the remaining ones, ascending and never reordered: the half bandwidth of K_ff is that of this order
+ * (an unsorted or duplicated bc_dofs list gives the same plan).  Returns GPDE_ERR_ARG when no dof is free, and
+ * GPDE_ERR_SIZE when the half bandwidth exceeds 255 or the cooperative kernels would need more than 227 KB of shared
+ * memory per CTA: some meshes under ROM.FromPhysics's 290-cell cap are refused (the unit square with 36x4 or 52x1 cells
+ * and left-right Dirichlet dofs; 51x1, half bandwidth 50, is accepted). */
 int gpde_rom_plan_create(gpde_rom_plan **plan, int n, int E, const double *M_host,
                          const int64_t *bc_dofs, int n_bc, int device);
 int gpde_rom_plan_destroy(gpde_rom_plan *plan);
