@@ -126,6 +126,9 @@ class VoPlan(object):
         coarse-grained-residual sampler only changes at resample()).  Returns a PackedWeights to pass as ``V``,
         or V itself when this plan / m has no packed layout.  B = the largest batch it will be used with;
         ``out`` = an earlier PackedWeights whose buffer is reused."""
+        if V.dim() != 2:
+            raise ValueError("pack_weights packs one weighting matrix [d,m] shared by the batch, got V of shape %r"
+                             % (tuple(V.shape),))
         dt = V.dtype if V.dtype in (torch.float32, torch.float64) else torch.float64
         Vc = V.to(dt).contiguous()
         sfx = _lib.suffix(dt)
@@ -146,16 +149,33 @@ class VoPlan(object):
         """r[B,m] = V^T (K(a_b) u~_b - f)_free with u~ = (y on free dofs, g on Dirichlet dofs).
 
         a [B,n_inputs] or [n_inputs] (shared); y [B,d] or None (zeros); g [B,n_bc], [n_bc] or None;
-        V [d,m] or None (then only rho[B,d], the fine residual itself, is produced).
+        V [d,m] shared by the batch, [B,d,m] one matrix per sample (r_b = V_b^T rho_b), or None (then only rho[B,d], the
+        fine residual itself, is produced).
         Returns r, or (r, rho) when want_rho / V is None.
         ``sm_reserve``: SMs to leave to kernels the caller runs beside this call on other streams (the structured-grid
-        kernel sizes its last wave of CTAs for the remaining SMs)."""
+        kernel sizes its last wave of CTAs for the remaining SMs; a [B,d,m] V has no such kernel and ignores it)."""
         dt = a.dtype
         sfx = _lib.suffix(dt)
+        per_sample = V is not None and not isinstance(V, PackedWeights) and V.dim() == 3
         sizes = [t.shape[0] for t in (y, a, g) if t is not None and t.dim() == 2]
-        B = sizes[0] if sizes else 1
+        B = sizes[0] if sizes else (int(V.shape[0]) if per_sample else 1)
         if any(n != B for n in sizes):   # e.g. a shared 1-D field with y = None and a batched g: every batched argument counts
             raise ValueError("inconsistent batch sizes %r among a, y, g" % (sizes,))
+        if per_sample:
+            Vc, v_stride, m = self._per_sample_weights(V, B, dt)
+            r = a.new_empty((B, m))
+            rho = a.new_empty((B, self.d)) if want_rho else None
+            a = a.contiguous()
+            y = None if y is None else y.to(dt).contiguous()
+            g = None if g is None else g.to(dt).contiguous()
+            dev = self.device
+            rc = getattr(self._lib, "gpde_vo_residual_vb_" + sfx)(
+                self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
+                _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), v_stride, m,
+                _lib.ptr(r, dev), _lib.ptr(rho, dev), _lib.ptr(self._vb_workspace(B, m), dev), 1 if ignore_load else 0, B,
+                _lib.stream_of(dev))
+            _lib.check(rc, "gpde_vo_residual_vb_" + sfx)
+            return (r, rho) if rho is not None else r
         a = a.contiguous()
         packed = None
         if isinstance(V, PackedWeights):
@@ -181,15 +201,43 @@ class VoPlan(object):
         _lib.check(rc, "gpde_vo_residual_" + sfx)
         return (r, rho) if rho is not None else r
 
+    def _vb_workspace(self, B, m):
+        need = max(16, int(self._lib.gpde_vo_vb_workspace_bytes(self.handle, B, m)))
+        if self._scratch is None or self._scratch.numel() < need:
+            self._scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
+        return self._scratch
+
+    def _per_sample_weights(self, V, B, dt):
+        """(contiguous V [B,d,m] in dt, v_stride, m) for the per-sample entry points; ValueError unless V matches the batch
+        and the plan."""
+        if V.dim() != 3 or V.shape[0] != B or V.shape[1] != self.d or V.shape[2] < 1:
+            raise ValueError("per-sample weighting matrices must be [B=%d, d=%d, m>=1], got %r" % (B, self.d, tuple(V.shape)))
+        return V.to(dt).contiguous(), int(V.shape[1] * V.shape[2]), int(V.shape[2])
+
     def residual_T(self, a, V, s, *, a_is_log=True):
-        """q[B,d] = K_ff(a_b) (V s_b)  (= Gamma_b^T s_b)."""
+        """q[B,d] = K_ff(a_b) (V s_b)  (= Gamma_b^T s_b); V [d,m] shared by the batch or [B,d,m] one matrix per sample
+        (q_b = K_ff(a_b) (V_b s_b))."""
         dt = a.dtype
         sfx = _lib.suffix(dt)
+        dev = self.device
+        if V.dim() == 3:
+            a, s = a.contiguous(), s.to(dt).contiguous()
+            B = int(s.shape[0])
+            if a.dim() == 2 and a.shape[0] != B:
+                raise ValueError("inconsistent batch sizes: a has %d rows, s %d" % (a.shape[0], B))
+            Vc, v_stride, m = self._per_sample_weights(V, B, dt)
+            if s.shape[1] != m:
+                raise ValueError("s has %d columns, V_b %d" % (s.shape[1], m))
+            q = a.new_empty((B, self.d))
+            rc = getattr(self._lib, "gpde_vo_residual_T_vb_" + sfx)(
+                self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(Vc, dev),
+                v_stride, m, _lib.ptr(s, dev), _lib.ptr(q, dev), _lib.ptr(self._vb_workspace(B, m), dev), B, _lib.stream_of(dev))
+            _lib.check(rc, "gpde_vo_residual_T_vb_" + sfx)
+            return q
         a, s, Vc = a.contiguous(), s.to(dt).contiguous(), V.to(dt).contiguous()
         B, m = s.shape
         q = a.new_empty((B, self.d))
         fn = getattr(self._lib, "gpde_vo_residual_T_" + sfx)
-        dev = self.device
         rc = fn(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(Vc, dev), m,
                 _lib.ptr(s, dev), _lib.ptr(q, dev), _lib.ptr(self._workspace(B, m), dev), B, _lib.stream_of(dev))
         _lib.check(rc, "gpde_vo_residual_T_" + sfx)
@@ -199,9 +247,10 @@ class VoPlan(object):
         """(grad_a, grad_g): the gradient of L with dL/dr = gbar_r [B,m] through r = residual(a, y, g, V) with respect to
         the conductivity input a and the Dirichlet values g (gpde_vo_residual_grad_*; r is linear in both, no solve):
             grad_a[b,p] = sum_{cells c of input p} w~_b[c]^T K_c u~_b[c],   grad_g[b] = K_cf(a_b) w~_b,
-        w~_b = V gbar_r_b on the free dofs (0 on the Dirichlet dofs).  With ``a_is_log`` a = exp(x) and grad_a is the
-        gradient in x.  A gradient that is not wanted is None.  For a shared 1-D ``a`` or ``g`` the per-sample gradients
-        are summed over the batch.  The load vector does not enter."""
+        w~_b = V gbar_r_b on the free dofs (0 on the Dirichlet dofs); V [d,m] shared by the batch or [B,d,m] one matrix per
+        sample (w~_b = V_b gbar_r_b).  With ``a_is_log`` a = exp(x) and grad_a is the gradient in x.  A gradient that is not
+        wanted is None.  For a shared 1-D ``a`` or ``g`` the per-sample gradients are summed over the batch.  The load
+        vector does not enter."""
         dt = a.dtype
         sfx = _lib.suffix(dt)
         dev = self.device
@@ -213,10 +262,23 @@ class VoPlan(object):
         a = a.contiguous()
         y = None if y is None else y.to(dt).contiguous()
         g = None if g is None else g.to(dt).contiguous()
-        Vc = V.to(dt).contiguous()
+        per_sample = V.dim() == 3
+        if per_sample:
+            Vc, v_stride, _ = self._per_sample_weights(V, B, dt)
+            if V.shape[2] != m:
+                raise ValueError("gbar_r has %d columns, V_b %d" % (m, V.shape[2]))
+        else:
+            Vc = V.to(dt).contiguous()
         grad_a = a.new_empty((B, self.n_inputs)) if want_grad_a else None
         grad_g = a.new_empty((B, self.n_bc)) if want_grad_g else None
-        if B:
+        if B and per_sample:
+            rc = getattr(self._lib, "gpde_vo_residual_grad_vb_" + sfx)(
+                self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
+                _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), v_stride, m,
+                _lib.ptr(gbar_r, dev), _lib.ptr(grad_a, dev), _lib.ptr(grad_g, dev), _lib.ptr(self._vb_workspace(B, m), dev),
+                B, _lib.stream_of(dev))
+            _lib.check(rc, "gpde_vo_residual_grad_vb_" + sfx)
+        elif B:
             need = max(16, int(self._lib.gpde_vo_grad_workspace_bytes(self.handle, B, m)))
             if self._grad_scratch is None or self._grad_scratch.numel() < need:
                 self._grad_scratch = torch.empty(need, dtype=torch.uint8, device=dev)
@@ -336,8 +398,9 @@ class PackedWeights(object):
 
 
 class VoResidualFn(torch.autograd.Function):
-    """r = V^T (K(a) u~ - f), differentiable in y: dL/dy = K_ff(a) V gbar_r (one residual_T launch), in the
-    conductivity input a and in the Dirichlet values g (VoPlan.residual_grad).  V gets no gradient (None)."""
+    """r = V^T (K(a) u~ - f), differentiable in y: dL/dy = K_ff(a) V gbar_r (one residual_T call), in the
+    conductivity input a and in the Dirichlet values g (VoPlan.residual_grad).  V [d,m] shared by the batch or [B,d,m]
+    one matrix per sample (passed through to every call as it is).  V gets no gradient (None)."""
 
     @staticmethod
     def forward(ctx, y, a, g, V, plan, a_is_log):
@@ -1023,15 +1086,31 @@ class VirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
             self._packed_weights = cached
         return cached[2]
 
-    def residuals(self, Y, V):
-        """r[N,m] = V^T (K_fom(x_n) y~_n - f) for all data points in ONE launch; V [d,m] is a weighting
-        matrix shared by the ensemble (e.g. V = W of the coarse-grained-residual sampler)."""
-        plan, a, G = self._inputs()
-        return plan.residual(a, _as_f64(Y, self.device), G, self._shared_weights(V, Y.shape[0]), a_is_log=False)
+    def _own_weights(self):
+        """The querries' own weighting matrices for residuals / residual_gradients without V: the shared [d,m] tensor or
+        the stack [N,d,m]."""
+        V = self._weights(max_m=float("inf"))
+        if V is None:
+            raise RuntimeError("residuals / residual_gradients without V need every data point's weighting matrix; some "
+                             "sampler of this ensemble provides only (Gamma, alpha) (flux constraints): pass V explicitly")
+        return V
 
-    def residual_gradients(self, S, V):
-        """q[N,d] = K_ff(x_n) V s_n for all data points in one launch (S [N,m])."""
+    def residuals(self, Y, V=None):
+        """r[N,m] = V_n^T (K_fom(x_n) y~_n - f) for all data points in one call.  V [d,m] is a weighting matrix shared by
+        the ensemble (e.g. V = W of the coarse-grained-residual sampler); without V the querries' own weighting matrices
+        are used (shared, or one per data point as with Gaussian-sketch and RBF samplers), so that r[n] = Gamma_n Y[n] -
+        alpha_n."""
+        plan, a, G = self._inputs()
+        if V is None:
+            V = self._own_weights()
+        V = V if isinstance(V, torch.Tensor) and V.dim() == 3 else self._shared_weights(V, Y.shape[0])
+        return plan.residual(a, _as_f64(Y, self.device), G, V, a_is_log=False)
+
+    def residual_gradients(self, S, V=None):
+        """q[N,d] = K_ff(x_n) V_n s_n = Gamma_n^T S[n] for all data points in one call (S [N,m]); V as for residuals."""
         plan, a, _ = self._inputs()
+        if V is None:
+            V = self._own_weights()
         return plan.residual_T(a, _as_f64(V, self.device), _as_f64(S, self.device), a_is_log=False)
 
     def _fine_residual(self, Y):

@@ -69,6 +69,17 @@ SIGNATURES = {
                                           c_vp, c_i64, c_vp]),
     "gpde_vo_residual_grad_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp,
                                           c_vp, c_i64, c_vp]),
+    "gpde_vo_vb_workspace_bytes": (c_sz, [c_vp, c_i64, c_i32]),
+    "gpde_vo_residual_vb_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
+                                        c_vp, c_i32, c_i64, c_vp]),
+    "gpde_vo_residual_vb_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
+                                        c_vp, c_i32, c_i64, c_vp]),
+    "gpde_vo_residual_T_vb_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_T_vb_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_grad_vb_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
+                                             c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_grad_vb_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
+                                             c_vp, c_vp, c_i64, c_vp]),
     "gpde_cg_init_f64": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_f64, c_i32, c_i64, c_i32, c_vp]),
     "gpde_cg_step_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i64, c_i32, c_vp]),
 }

@@ -288,6 +288,42 @@ int gpde_vo_residual_grad_f32(const gpde_vo_plan *plan, const float *a, int64_t 
                               const float *gbar_r, float *grad_a, float *grad_g, void *workspace,
                               int64_t B, gpde_stream_t stream);
 
+/* ---- the residual family with one weighting matrix per sample: V [B,d,m] row-major, V_b = V + b*v_stride, and v_stride
+ * must be d*m (for one matrix shared by the batch use the entry points above).  Same definitions with V indexed by sample:
+ *     gpde_vo_residual_vb_*       r[b,:] = V_b^T rho_b,   rho_b = (K_fom(a_b) u~_b - f)_free
+ *     gpde_vo_residual_T_vb_*     q[b,:] = K_ff(a_b) (V_b s_b)
+ *     gpde_vo_residual_grad_vb_*  grad_a, grad_g as gpde_vo_residual_grad_* with w~_b = V_b gbar_r_b
+ * Other arguments as for the shared-V versions.  rho: the fine residual comes from the rho-only route of gpde_vo_residual_*
+ * (the kernel the plan picks for it), then one contraction kernel streams V_b once; the transposed application and the
+ * gradient first form the FP64 rows V_b s_b in the workspace with one expansion kernel, then run the K_ff application of
+ * gpde_vo_residual_T_* (strided-y marching kernel on pixel grids, generic matvec otherwise) or the gradient kernels.  Any
+ * m >= 1.  FP32 I/O reads V, rho and s as floats and accumulates in FP64 (rho itself is held as floats).  flags: bit0 =
+ * ignore the load vector f; bit1 (packed weights) returns GPDE_ERR_ARG.  workspace: >= gpde_vo_vb_workspace_bytes(plan, B,
+ * m), 16-byte aligned (it holds rho [B,d] when the caller passes no rho output, or V_b s_b).  B = 0 is a no-op.  m <= 0,
+ * v_stride != d*m, a NULL or misaligned workspace or a NULL operand return GPDE_ERR_ARG.  Every output is summed in a fixed
+ * order: results are deterministic. */
+size_t gpde_vo_vb_workspace_bytes(const gpde_vo_plan *plan, int64_t B, int m);
+int gpde_vo_residual_vb_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
+                            const double *y, const double *g, int64_t g_stride, const double *V, int64_t v_stride,
+                            int m, double *r, double *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream);
+int gpde_vo_residual_vb_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
+                            const float *y, const float *g, int64_t g_stride, const float *V, int64_t v_stride,
+                            int m, float *r, float *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream);
+int gpde_vo_residual_T_vb_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
+                              const double *V, int64_t v_stride, int m, const double *s, double *q, void *workspace,
+                              int64_t B, gpde_stream_t stream);
+int gpde_vo_residual_T_vb_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
+                              const float *V, int64_t v_stride, int m, const float *s, float *q, void *workspace,
+                              int64_t B, gpde_stream_t stream);
+int gpde_vo_residual_grad_vb_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
+                                 const double *y, const double *g, int64_t g_stride, const double *V, int64_t v_stride,
+                                 int m, const double *gbar_r, double *grad_a, double *grad_g, void *workspace,
+                                 int64_t B, gpde_stream_t stream);
+int gpde_vo_residual_grad_vb_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
+                                 const float *y, const float *g, int64_t g_stride, const float *V, int64_t v_stride,
+                                 int m, const float *gbar_r, float *grad_a, float *grad_g, void *workspace,
+                                 int64_t B, gpde_stream_t stream);
+
 /* ---- fine-mesh label solves: batched preconditioned CG (setup-time replacement of the per-sample FEniCS / spsolve calls
  * of physics/LinearElliptic.py:85-101, 120-133 in utils/data.py:96-99).  One iteration = one gpde_vo_residual_f64 call with
  * y = p (rho output, flags bit0, no Dirichlet data: rho = K_ff(a) p for the whole batch) + one gpde_cg_step_f64 call.
