@@ -368,22 +368,44 @@ class VoPlan(object):
         - f_eff (``residual(a, mean, g_bc, None)`` minus the load), g, prec [N,d], inv_T [N].  A data point whose M_n has a
         non-positive pivot keeps its mean and sets GPDE_INFO_NOT_SPD in ``info``.  Returns ``mean``."""
         dev = self.device
-        if not (mean.dtype == torch.float64 and mean.dim() == 2 and mean.is_contiguous()):
-            raise ValueError("energy_step updates mean in place: it must be a contiguous float64 [N,d] tensor")
-        N = int(mean.shape[0])
-        a = a.to(torch.float64).contiguous()
-        V, v_stride, m = self._weights_arg(V)
-        rho, g, prec = (t.to(torch.float64).contiguous() for t in (rho, g, prec))
-        inv_T = torch.as_tensor(inv_T, dtype=torch.float64, device=dev).contiguous()
-        if any(t.shape != mean.shape for t in (rho, g, prec)) or mean.shape[1] != self.d or inv_T.shape != (N,) or \
-                (a.dim() == 2 and a.shape[0] != N) or (v_stride and V.shape[0] != N):
-            raise ValueError("energy_step: inconsistent shapes")
+        N, a, V, v_stride, m, rho, g, prec, inv_T = self._energy_operands("energy_step", a, V, rho, g, prec, inv_T, mean)
         rc = self._lib.gpde_vo_energy_step_f64(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0,
                                                _lib.ptr(V, dev), v_stride, m, _lib.ptr(rho, dev), _lib.ptr(g, dev),
                                                _lib.ptr(prec, dev), _lib.ptr(inv_T, dev), _lib.ptr(mean, dev),
                                                _lib.ptr(info, dev), N, _lib.stream_of(dev))
         _lib.check(rc, "gpde_vo_energy_step_f64")
         return mean
+
+    def energy_step_blocked(self, a, V, rho, g, prec, inv_T, mean, info=None):
+        """``energy_step`` for 1 <= m <= 256 (gpde_vo_energy_step_blocked_f64): M_n lives in a workspace this call
+        allocates (the blocked posterior's, about 1 MB per data point at m = 256) instead of shared memory; three launches
+        for all data points.  Same arguments, checks and in-place update of ``mean``; returns ``mean``."""
+        dev = self.device
+        N, a, V, v_stride, m, rho, g, prec, inv_T = self._energy_operands("energy_step_blocked", a, V, rho, g, prec, inv_T,
+                                                                          mean)
+        need = int(self._lib.gpde_vo_posterior_blocked_workspace_bytes(self.handle, N, m))
+        ws = torch.empty(max(need, 16), dtype=torch.uint8, device=dev)
+        rc = self._lib.gpde_vo_energy_step_blocked_f64(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0,
+                                                       _lib.ptr(V, dev), v_stride, m, _lib.ptr(rho, dev), _lib.ptr(g, dev),
+                                                       _lib.ptr(prec, dev), _lib.ptr(inv_T, dev), _lib.ptr(mean, dev),
+                                                       _lib.ptr(info, dev), _lib.ptr(ws, dev), need, N,
+                                                       _lib.stream_of(dev))
+        _lib.check(rc, "gpde_vo_energy_step_blocked_f64")
+        return mean
+
+    def _energy_operands(self, name, a, V, rho, g, prec, inv_T, mean):
+        """(N, a, V, v_stride, m, rho, g, prec, inv_T) of an energy step, as contiguous float64, with the shape checks."""
+        if not (mean.dtype == torch.float64 and mean.dim() == 2 and mean.is_contiguous()):
+            raise ValueError("%s updates mean in place: it must be a contiguous float64 [N,d] tensor" % name)
+        N = int(mean.shape[0])
+        a = a.to(torch.float64).contiguous()
+        V, v_stride, m = self._weights_arg(V)
+        rho, g, prec = (t.to(torch.float64).contiguous() for t in (rho, g, prec))
+        inv_T = torch.as_tensor(inv_T, dtype=torch.float64, device=self.device).contiguous()
+        if any(t.shape != mean.shape for t in (rho, g, prec)) or mean.shape[1] != self.d or inv_T.shape != (N,) or \
+                (a.dim() == 2 and a.shape[0] != N) or (v_stride and V.shape[0] != N):
+            raise ValueError("%s: inconsistent shapes" % name)
+        return N, a, V, v_stride, m, rho, g, prec, inv_T
 
 
 class PackedWeights(object):
@@ -1317,14 +1339,19 @@ class EnergyVirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
                (one launch); the reference: N x n_it x [dense V^T A V, V^T (A mean - b), solve]
 
     The weighting matrices are drawn in the member loop's order (data point-major, iteration-minor), with one
-    ``sample_V_batch`` call when the data points share one sampler, so both routes see the same draws.  The member loop
-    (``EnergyVirtualObservable.update`` per data point) runs instead when ``batched_update`` is False, when the drawn m
-    exceeds ``max_kernel_m``, or when the members differ in iterations per update or physics; ``last_update_route`` says
-    which route the last update took ("batched" or "members")."""
+    ``sample_V_batch`` call when the data points share one sampler, so both routes see the same draws.  Up to
+    ``max_kernel_m`` = 64 weighting functions the step is gpde_vo_energy_step_f64; for ``max_kernel_m`` < m <=
+    ``max_blocked_m`` it is the blocked gpde_vo_energy_step_blocked_f64 (three launches, M_n in a workspace).  The member
+    loop (``EnergyVirtualObservable.update`` per data point) runs instead when ``batched_update`` is False, when the m
+    announced by the samplers or drawn exceeds both limits, or when the members differ in iterations per update or
+    physics; ``last_update_route`` says which route the last update took ("batched", "blocked" or "members")."""
 
     batched_update = True
     max_kernel_m = 64
-    # per-chunk budget for the drawn weighting matrices V [n, n_it, d, m] of the batched route
+    # the blocked route takes max_kernel_m < m <= max_blocked_m (at most 256, the kernels' limit); at 64 it is off and
+    # such m take the member loop
+    max_blocked_m = 64
+    # per-chunk budget for the drawn weighting matrices V [n, n_it, d, m] (and the blocked route's workspace)
     max_stack_bytes = 1 << 30
 
     def __init__(self, QuerryPointEnsemble, num_iterations_per_update, sampler, dtype, device):
@@ -1370,8 +1397,9 @@ class EnergyVirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
         v0 = vos[0]
         n_it = v0._num_iterations_per_update
         m_known = [getattr(vo._sampler, "m", None) for vo in vos]
+        max_m = max(self.max_kernel_m, self.max_blocked_m)
         if not self.batched_update or any(vo._num_iterations_per_update != n_it or vo._plan is not v0._plan for vo in vos) \
-                or any(m is not None and m > self.max_kernel_m for m in m_known):
+                or any(m is not None and m > max_m for m in m_known):
             return self._update_members(G, PREC, iteration)
         plan, a, gbc, K_diag, load = self._inputs()
         G64, P64 = _as_f64(G, self.device), _as_f64(PREC, self.device)
@@ -1381,15 +1409,16 @@ class EnergyVirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
         if self._info is None:
             self._info = torch.zeros(1, dtype=torch.int32, device=self.device)
         # m of samplers that do not announce it is known after the first draw: size the first chunk for the largest m
-        # the kernel takes
-        m = max((m for m in m_known if m is not None), default=self.max_kernel_m)
+        # the batched routes take
+        m = max((m for m in m_known if m is not None), default=max_m)
+        route = "batched"
         lo = 0
         while lo < self.N:
-            step = max(1, int(self.max_stack_bytes // (8 * n_it * self.dim_out * m)))
+            step = max(1, int(self.max_stack_bytes // self._chunk_bytes_per_point(plan, n_it, m)))
             chunk = vos[lo:lo + step]
             V = self._draw(chunk, n_it)
             m = int(V.shape[-1])
-            if m > self.max_kernel_m:      # only on the first chunk: the member loop, with the draws already made
+            if m > max_m:                  # only on the first chunk: the member loop, with the draws already made
                 saved = [vo._sampler for vo in chunk]
                 try:
                     for k, vo in enumerate(chunk):
@@ -1398,13 +1427,16 @@ class EnergyVirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
                 finally:
                     for vo, s in zip(chunk, saved):
                         vo._sampler = s
+            energy_step = plan.energy_step
+            if m > self.max_kernel_m:
+                energy_step, route = plan.energy_step_blocked, "blocked"
             hi = lo + len(chunk)
             V = V.transpose(0, 1).contiguous()                          # [n_it, n, d, m]: one contiguous stack per step
             for it in range(n_it):
                 _, rho = plan.residual(a[lo:hi], mean[lo:hi], gbc[lo:hi], None, a_is_log=False)
                 if load is not None:
                     rho -= load[lo:hi]
-                plan.energy_step(a[lo:hi], V[it], rho, G64[lo:hi], P64[lo:hi], inv_T[lo:hi], mean[lo:hi], info=self._info)
+                energy_step(a[lo:hi], V[it], rho, G64[lo:hi], P64[lo:hi], inv_T[lo:hi], mean[lo:hi], info=self._info)
             lo = hi
         if int(self._info.item()):
             self._info.zero_()
@@ -1412,7 +1444,13 @@ class EnergyVirtualObservablesEnsemble(BaseVirtualObservablesEnsemble):
         for k, vo in enumerate(vos):
             vo._mean, vo._vars = mean[k], vars_[k]
         self.flush_cache()
-        self.last_update_route = "batched"
+        self.last_update_route = route
+
+    def _chunk_bytes_per_point(self, plan, n_it, m):
+        """Device bytes a data point adds to a chunk: its drawn V [n_it, d, m] and, on the blocked route, its workspace
+        (sized for a chunk of one data point, which has the most row segments)."""
+        ws = plan.posterior_blocked_workspace_bytes(1, m) if m > self.max_kernel_m else 0
+        return 8 * n_it * self.dim_out * m + ws
 
     def force_temperature(self, value):
         for vo in self:

@@ -62,6 +62,8 @@ SIGNATURES = {
     "gpde_vo_moments_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_vo_energy_step_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64,
                                         c_vp]),
+    "gpde_vo_energy_step_blocked_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                                c_vp, c_sz, c_i64, c_vp]),
     "gpde_vo_residual_T_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_vo_residual_T_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gpde_vo_grad_workspace_bytes": (c_sz, [c_vp, c_i64, c_i32]),

@@ -49,6 +49,7 @@ constexpr int kVoThreads = 256;
 #include "vo_gridgemm.cuh"
 #include "vo_posterior.cuh"
 #include "vo_posterior_blocked.cuh"
+#include "vo_energy_blocked.cuh"
 #include "vo_energy.cuh"
 #include "vo_grad.cuh"
 #include "vo_vb.cuh"
@@ -1519,6 +1520,40 @@ int gpde_vo_energy_step_f64(const gpde_vo_plan *pl, const double *a, int64_t a_s
     cudaStream_t st = (cudaStream_t)stream;
     if (m <= 32) return vo_energy_step_launch<32>(pl, a, a_stride, V, v_stride, m, rho, g, prec, inv_T, mean, info, N, st);
     return vo_energy_step_launch<64>(pl, a, a_stride, V, v_stride, m, rho, g, prec, inv_T, mean, info, N, st);
+}
+
+int gpde_vo_energy_step_blocked_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, const double *V,
+                                    int64_t v_stride, int m, const double *rho, const double *g, const double *prec,
+                                    const double *inv_T, double *mean, int *info, void *workspace, size_t workspace_bytes,
+                                    int64_t N, gpde_stream_t stream) {
+    if (!pl || N < 0 || m <= 0) return fail(GPDE_ERR_ARG, "vo_energy_step_blocked: bad argument");
+    if (m > 256) return fail(GPDE_ERR_SIZE, "vo_energy_step_blocked: m = %d > 256 weighting functions per data point", m);
+    if (N == 0) return GPDE_OK;
+    if (!a || !V || !rho || !g || !prec || !inv_T || !mean)
+        return fail(GPDE_ERR_ARG, "vo_energy_step_blocked: null argument");
+    if (a_stride != 0 && a_stride != (int64_t)pl->dev.n_inputs)
+        return fail(GPDE_ERR_ARG, "vo_energy_step_blocked: a_stride must be 0 or n_inputs");
+    if (v_stride != 0 && v_stride != (int64_t)pl->dev.d * m)
+        return fail(GPDE_ERR_ARG, "vo_energy_step_blocked: v_stride must be 0 or d*m");
+    const size_t need = gpde_vo_posterior_blocked_workspace_bytes(pl, N, m);
+    if (!workspace || ((uintptr_t)workspace & 15) || workspace_bytes < need)
+        return fail(GPDE_ERR_ARG, "vo_energy_step_blocked: workspace must be 16-byte aligned and hold %zu bytes", need);
+    DeviceGuard guard(pl->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const BlkLayout Lo = blocked_layout(pl, (long long)N, m);
+    double *ws = (double *)workspace;
+    void *zero_noise = nullptr;
+    GPDE_CUDA_OK(cudaGetSymbolAddress(&zero_noise, energy_zero_noise));
+    const size_t sm_gram = blk_gram_smem(pl->csr.max_row), sm_factor = blk_factor_smem(Lo.mp);
+    GPDE_CUDA_OK(cudaFuncSetAttribute(vo_energy_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_gram));
+    GPDE_CUDA_OK(cudaFuncSetAttribute(vo_post_factor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_factor));
+    vo_energy_gram_kernel<<<dim3((unsigned)(Lo.nbt * Lo.S), (unsigned)N), kPostThreads, sm_gram, st>>>(
+        pl->csr, a, (long long)a_stride, V, (long long)v_stride, m, rho, g, prec, inv_T, mean, ws, Lo);
+    vo_post_factor_kernel<<<(unsigned)N, kPostThreads, sm_factor, st>>>(m, (const double *)zero_noise, ws, Lo, info);
+    vo_energy_apply_kernel<<<dim3((unsigned)((pl->csr.d + kEnergyApplyRows - 1) / kEnergyApplyRows), (unsigned)N),
+                             kPostThreads, 0, st>>>(pl->csr.d, V, (long long)v_stride, m, ws, Lo, mean);
+    GPDE_CUDA_OK(cudaGetLastError());
+    return GPDE_OK;
 }
 
 int gpde_vo_residual_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *y,

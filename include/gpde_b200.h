@@ -254,6 +254,20 @@ int gpde_vo_energy_step_f64(const gpde_vo_plan *plan, const double *a, int64_t a
                             int64_t v_stride, int m, const double *rho, const double *g, const double *prec,
                             const double *inv_T, double *mean, int *info, int64_t N, gpde_stream_t stream);
 
+/* The same step for 1 <= m <= 256 (m > 256: GPDE_ERR_SIZE), blocked: M_n (m x m, m padded to a multiple of 64) lives in
+ * the caller's workspace instead of shared memory.  Three launches: the Gram blocks of M_n and b_n over row tiles (DMMA),
+ * one Cholesky CTA per data point (the blocked posterior's factor kernel, no noise term), and mean_n -= V_n sol_n on the
+ * rows of V_n.  Arguments as gpde_vo_energy_step_f64, plus workspace (16-byte aligned, device) of workspace_bytes >=
+ * gpde_vo_posterior_blocked_workspace_bytes(plan, N, m): the layout is the blocked posterior's.  m <= 0, an a_stride
+ * other than 0 or n_inputs, a v_stride other than 0 or d*m, a null operand, or a null, misaligned or smaller workspace
+ * returns GPDE_ERR_ARG.  N = 0 is a no-op.  A data point whose M_n has a non-positive pivot ORs GPDE_INFO_NOT_SPD into
+ * info and keeps its mean bitwise.  Results are deterministic for a given (plan, N, m): the row split of the Gram pass
+ * depends on N.                                                                                                        */
+int gpde_vo_energy_step_blocked_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, const double *V,
+                                    int64_t v_stride, int m, const double *rho, const double *g, const double *prec,
+                                    const double *inv_T, double *mean, int *info, void *workspace,
+                                    size_t workspace_bytes, int64_t N, gpde_stream_t stream);
+
 /* q[B,d] = K_ff(a_b) (V s_b) = Gamma_b^T s_b  (VirtualObservables.py:663; with s = P r it is the
  * gradient of 1/2 r^T P r w.r.t. y).  With B = m, s = I and a_stride = 0 it yields Gamma itself.
  * On the reference's pixel meshes with m <= 32 this is one kernel (after a small packing launch of V^T): the rows
