@@ -77,7 +77,6 @@ class VoPlan(object):
         self.n_nodes, self.n_cells, self.n_inputs, self.d, self.n_bc, self.slots_per_row = (int(v) for v in info[:6])
         self.fused_smem_bytes = int(info[7])   # 0: this mesh only runs on the unfused version-1 kernels
         self._scratch = None
-        self._grad_scratch = None
 
     def __del__(self):
         handle, self.handle = getattr(self, "handle", None), None
@@ -116,7 +115,7 @@ class VoPlan(object):
         return {3: 3, 2: 2, 1: 1}.get(path, 3 if m > 0 else 1)
 
     def _workspace(self, B, m):
-        need = max(8, int(self._lib.gpde_vo_workspace_bytes(self.handle, B, m)))
+        need = max(16, int(self._lib.gpde_vo_workspace_bytes(self.handle, B, m)))
         if self._scratch is None or self._scratch.numel() < need:
             self._scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
         return self._scratch
@@ -161,21 +160,6 @@ class VoPlan(object):
         B = sizes[0] if sizes else (int(V.shape[0]) if per_sample else 1)
         if any(n != B for n in sizes):   # e.g. a shared 1-D field with y = None and a batched g: every batched argument counts
             raise ValueError("inconsistent batch sizes %r among a, y, g" % (sizes,))
-        if per_sample:
-            Vc, v_stride, m = self._per_sample_weights(V, B, dt)
-            r = a.new_empty((B, m))
-            rho = a.new_empty((B, self.d)) if want_rho else None
-            a = a.contiguous()
-            y = None if y is None else y.to(dt).contiguous()
-            g = None if g is None else g.to(dt).contiguous()
-            dev = self.device
-            rc = getattr(self._lib, "gpde_vo_residual_vb_" + sfx)(
-                self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
-                _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), v_stride, m,
-                _lib.ptr(r, dev), _lib.ptr(rho, dev), _lib.ptr(self._vb_workspace(B, m), dev), 1 if ignore_load else 0, B,
-                _lib.stream_of(dev))
-            _lib.check(rc, "gpde_vo_residual_vb_" + sfx)
-            return (r, rho) if rho is not None else r
         a = a.contiguous()
         packed = None
         if isinstance(V, PackedWeights):
@@ -186,30 +170,25 @@ class VoPlan(object):
             V = V.V
         y = None if y is None else y.to(dt).contiguous()
         g = None if g is None else g.to(dt).contiguous()
-        m = 0 if V is None else int(V.shape[1])
-        Vc = None if V is None else V.to(dt).contiguous()
+        Vc, v_stride, m = (None, 0, 0) if V is None else self._weights_arg(V, dt, B)
         r = a.new_empty((B, m)) if m else None
         rho = a.new_empty((B, self.d)) if (want_rho or not m) else None
         fn = getattr(self._lib, "gpde_vo_residual_" + sfx)
         ws = packed.buf if packed is not None else (self._workspace(B, m) if m else None)
         dev = self.device
         rc = fn(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
-                _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), m,
+                _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), v_stride, m,
                 _lib.ptr(r, dev), _lib.ptr(rho, dev), _lib.ptr(ws, dev) if m else None,
                 (1 if ignore_load else 0) | (2 if packed is not None else 0) | (max(0, min(255, int(sm_reserve))) << 8), B,
                 _lib.stream_of(dev))
         _lib.check(rc, "gpde_vo_residual_" + sfx)
         return (r, rho) if rho is not None else r
 
-    def _vb_workspace(self, B, m):
-        need = max(16, int(self._lib.gpde_vo_vb_workspace_bytes(self.handle, B, m)))
-        if self._scratch is None or self._scratch.numel() < need:
-            self._scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
-        return self._scratch
-
-    def _per_sample_weights(self, V, B, dt):
-        """(contiguous V [B,d,m] in dt, v_stride, m) for the per-sample entry points; ValueError unless V matches the batch
-        and the plan."""
+    def _weights_arg(self, V, dt, B):
+        """(contiguous V in dt, v_stride, m): V [d,m] shared by the batch (v_stride = 0) or [B,d,m] one matrix per sample
+        (v_stride = d*m); ValueError unless a [B,d,m] V matches the batch size B and the plan."""
+        if V.dim() == 2:
+            return V.to(dt).contiguous(), 0, int(V.shape[1])
         if V.dim() != 3 or V.shape[0] != B or V.shape[1] != self.d or V.shape[2] < 1:
             raise ValueError("per-sample weighting matrices must be [B=%d, d=%d, m>=1], got %r" % (B, self.d, tuple(V.shape)))
         return V.to(dt).contiguous(), int(V.shape[1] * V.shape[2]), int(V.shape[2])
@@ -220,26 +199,15 @@ class VoPlan(object):
         dt = a.dtype
         sfx = _lib.suffix(dt)
         dev = self.device
-        if V.dim() == 3:
-            a, s = a.contiguous(), s.to(dt).contiguous()
-            B = int(s.shape[0])
-            if a.dim() == 2 and a.shape[0] != B:
-                raise ValueError("inconsistent batch sizes: a has %d rows, s %d" % (a.shape[0], B))
-            Vc, v_stride, m = self._per_sample_weights(V, B, dt)
-            if s.shape[1] != m:
-                raise ValueError("s has %d columns, V_b %d" % (s.shape[1], m))
-            q = a.new_empty((B, self.d))
-            rc = getattr(self._lib, "gpde_vo_residual_T_vb_" + sfx)(
-                self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(Vc, dev),
-                v_stride, m, _lib.ptr(s, dev), _lib.ptr(q, dev), _lib.ptr(self._vb_workspace(B, m), dev), B, _lib.stream_of(dev))
-            _lib.check(rc, "gpde_vo_residual_T_vb_" + sfx)
-            return q
-        a, s, Vc = a.contiguous(), s.to(dt).contiguous(), V.to(dt).contiguous()
-        B, m = s.shape
+        a, s = a.contiguous(), s.to(dt).contiguous()
+        B, m = int(s.shape[0]), int(s.shape[1])
+        Vc, v_stride, mv = self._weights_arg(V, dt, B)
+        if v_stride and ((a.dim() == 2 and a.shape[0] != B) or mv != m):
+            raise ValueError("inconsistent shapes: a %r, V %r, s %r" % (tuple(a.shape), tuple(V.shape), tuple(s.shape)))
         q = a.new_empty((B, self.d))
         fn = getattr(self._lib, "gpde_vo_residual_T_" + sfx)
-        rc = fn(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(Vc, dev), m,
-                _lib.ptr(s, dev), _lib.ptr(q, dev), _lib.ptr(self._workspace(B, m), dev), B, _lib.stream_of(dev))
+        rc = fn(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(Vc, dev),
+                v_stride, m, _lib.ptr(s, dev), _lib.ptr(q, dev), _lib.ptr(self._workspace(B, m), dev), B, _lib.stream_of(dev))
         _lib.check(rc, "gpde_vo_residual_T_" + sfx)
         return q
 
@@ -262,45 +230,22 @@ class VoPlan(object):
         a = a.contiguous()
         y = None if y is None else y.to(dt).contiguous()
         g = None if g is None else g.to(dt).contiguous()
-        per_sample = V.dim() == 3
-        if per_sample:
-            Vc, v_stride, _ = self._per_sample_weights(V, B, dt)
-            if V.shape[2] != m:
-                raise ValueError("gbar_r has %d columns, V_b %d" % (m, V.shape[2]))
-        else:
-            Vc = V.to(dt).contiguous()
+        Vc, v_stride, mv = self._weights_arg(V, dt, B)
+        if v_stride and mv != m:
+            raise ValueError("gbar_r has %d columns, V_b %d" % (m, mv))
         grad_a = a.new_empty((B, self.n_inputs)) if want_grad_a else None
         grad_g = a.new_empty((B, self.n_bc)) if want_grad_g else None
-        if B and per_sample:
-            rc = getattr(self._lib, "gpde_vo_residual_grad_vb_" + sfx)(
-                self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
+        fn = getattr(self._lib, "gpde_vo_residual_grad_" + sfx)
+        rc = fn(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
                 _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), v_stride, m,
-                _lib.ptr(gbar_r, dev), _lib.ptr(grad_a, dev), _lib.ptr(grad_g, dev), _lib.ptr(self._vb_workspace(B, m), dev),
+                _lib.ptr(gbar_r, dev), _lib.ptr(grad_a, dev), _lib.ptr(grad_g, dev), _lib.ptr(self._workspace(B, m), dev),
                 B, _lib.stream_of(dev))
-            _lib.check(rc, "gpde_vo_residual_grad_vb_" + sfx)
-        elif B:
-            need = max(16, int(self._lib.gpde_vo_grad_workspace_bytes(self.handle, B, m)))
-            if self._grad_scratch is None or self._grad_scratch.numel() < need:
-                self._grad_scratch = torch.empty(need, dtype=torch.uint8, device=dev)
-            fn = getattr(self._lib, "gpde_vo_residual_grad_" + sfx)
-            rc = fn(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0, int(bool(a_is_log)), _lib.ptr(y, dev),
-                    _lib.ptr(g, dev), (self.n_bc if g.dim() == 2 else 0) if g is not None else 0, _lib.ptr(Vc, dev), m,
-                    _lib.ptr(gbar_r, dev), _lib.ptr(grad_a, dev), _lib.ptr(grad_g, dev), _lib.ptr(self._grad_scratch, dev),
-                    B, _lib.stream_of(dev))
-            _lib.check(rc, "gpde_vo_residual_grad_" + sfx)
+        _lib.check(rc, "gpde_vo_residual_grad_" + sfx)
         if grad_a is not None and a.dim() == 1:
             grad_a = grad_a.sum(0)
         if grad_g is not None and g is not None and g.dim() == 1:
             grad_g = grad_g.sum(0)
         return grad_a, grad_g
-
-    def _weights_arg(self, V):
-        """(contiguous float64 V, v_stride): [d,m] shared by the data points or [N,d,m] one matrix per data point."""
-        V = V.to(torch.float64).contiguous()
-        if V.dim() == 2:
-            return V, 0, int(V.shape[1])
-        assert V.dim() == 3 and V.shape[1] == self.d
-        return V, int(V.shape[1] * V.shape[2]), int(V.shape[2])
 
     def posterior(self, a, V, rho, noise_var, g, prec, info=None):
         """Gaussian conditioning of N data points in ONE launch, matrix-free (gpde_vo_posterior_f64):
@@ -310,7 +255,7 @@ class VoPlan(object):
         dev = self.device
         N = int(g.shape[0])
         a = a.to(torch.float64).contiguous()
-        V, v_stride, m = self._weights_arg(V)
+        V, v_stride, m = self._weights_arg(V, torch.float64, N)
         rho, g, prec = (t.to(torch.float64).contiguous() for t in (rho, g, prec))
         noise_var = noise_var.to(torch.float64).contiguous()
         mean, vars_ = torch.empty_like(g), torch.empty_like(g)
@@ -327,7 +272,7 @@ class VoPlan(object):
         dev = self.device
         N = int(g.shape[0])
         a = a.to(torch.float64).contiguous()
-        V, v_stride, m = self._weights_arg(V)
+        V, v_stride, m = self._weights_arg(V, torch.float64, N)
         rho, g, prec = (t.to(torch.float64).contiguous() for t in (rho, g, prec))
         noise_var = noise_var.to(torch.float64).contiguous()
         mean, vars_ = torch.empty_like(g), torch.empty_like(g)
@@ -350,7 +295,7 @@ class VoPlan(object):
         dev = self.device
         N = int(rho.shape[0])
         a = a.to(torch.float64).contiguous()
-        V, v_stride, m = self._weights_arg(V)
+        V, v_stride, m = self._weights_arg(V, torch.float64, N)
         rho, v = rho.to(torch.float64).contiguous(), v.to(torch.float64).contiguous()
         out_r, out_s2 = rho.new_empty((N, m)), rho.new_empty((N, m))
         rc = self._lib.gpde_vo_moments_f64(self.handle, _lib.ptr(a, dev), self.n_inputs if a.dim() == 2 else 0,
@@ -399,11 +344,11 @@ class VoPlan(object):
             raise ValueError("%s updates mean in place: it must be a contiguous float64 [N,d] tensor" % name)
         N = int(mean.shape[0])
         a = a.to(torch.float64).contiguous()
-        V, v_stride, m = self._weights_arg(V)
+        V, v_stride, m = self._weights_arg(V, torch.float64, N)
         rho, g, prec = (t.to(torch.float64).contiguous() for t in (rho, g, prec))
         inv_T = torch.as_tensor(inv_T, dtype=torch.float64, device=self.device).contiguous()
         if any(t.shape != mean.shape for t in (rho, g, prec)) or mean.shape[1] != self.d or inv_T.shape != (N,) or \
-                (a.dim() == 2 and a.shape[0] != N) or (v_stride and V.shape[0] != N):
+                (a.dim() == 2 and a.shape[0] != N):
             raise ValueError("%s: inconsistent shapes" % name)
         return N, a, V, v_stride, m, rho, g, prec, inv_T
 

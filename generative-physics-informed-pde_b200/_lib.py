@@ -49,9 +49,9 @@ SIGNATURES = {
     "gpde_vo_plan_info": (c_i32, [c_vp, c_vp]),
     "gpde_vo_plan_kernel_path": (c_i32, [c_vp, c_i32, c_i32]),
     "gpde_vo_workspace_bytes": (c_sz, [c_vp, c_i64, c_i32]),
-    "gpde_vo_residual_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp,
+    "gpde_vo_residual_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
                                      c_vp, c_i32, c_i64, c_vp]),
-    "gpde_vo_residual_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp,
+    "gpde_vo_residual_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
                                      c_vp, c_i32, c_i64, c_vp]),
     "gpde_vo_pack_weights_f64": (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_vp]),
     "gpde_vo_pack_weights_f32": (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_vp]),
@@ -64,24 +64,12 @@ SIGNATURES = {
                                         c_vp]),
     "gpde_vo_energy_step_blocked_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                                 c_vp, c_sz, c_i64, c_vp]),
-    "gpde_vo_residual_T_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
-    "gpde_vo_residual_T_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
-    "gpde_vo_grad_workspace_bytes": (c_sz, [c_vp, c_i64, c_i32]),
-    "gpde_vo_residual_grad_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp,
-                                          c_vp, c_i64, c_vp]),
-    "gpde_vo_residual_grad_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp,
-                                          c_vp, c_i64, c_vp]),
-    "gpde_vo_vb_workspace_bytes": (c_sz, [c_vp, c_i64, c_i32]),
-    "gpde_vo_residual_vb_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
-                                        c_vp, c_i32, c_i64, c_vp]),
-    "gpde_vo_residual_vb_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
-                                        c_vp, c_i32, c_i64, c_vp]),
-    "gpde_vo_residual_T_vb_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
-    "gpde_vo_residual_T_vb_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
-    "gpde_vo_residual_grad_vb_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
-                                             c_vp, c_vp, c_i64, c_vp]),
-    "gpde_vo_residual_grad_vb_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
-                                             c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_T_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_T_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_grad_f64": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
+                                          c_vp, c_vp, c_i64, c_vp]),
+    "gpde_vo_residual_grad_f32": (c_i32, [c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp,
+                                          c_vp, c_vp, c_i64, c_vp]),
     "gpde_cg_init_f64": (c_i32, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_f64, c_i32, c_i64, c_i32, c_vp]),
     "gpde_cg_step_f64": (c_i32, [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i64, c_i32, c_vp]),
 }

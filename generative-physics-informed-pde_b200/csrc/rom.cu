@@ -635,7 +635,7 @@ using namespace gpde;
 
 extern "C" {
 
-int gpde_version(void) { return 100; }
+int gpde_version(void) { return 101; }
 const char *gpde_last_error(void) { return gpde::g_last_error; }
 
 int gpde_rom_plan_create(gpde_rom_plan **plan, int n, int E, const double *M, const int64_t *bc_dofs, int n_bc,

@@ -843,15 +843,30 @@ static int launch_gridgemm(const gpde_vo_plan *pl, const T *a, long long a_strid
 
 template <typename T>
 static int vo_residual(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *y, const T *g,
-                       int64_t g_stride, const T *V, int m, T *r, T *rho, void *workspace, int flags, int64_t B,
-                       gpde_stream_t stream) {
+                       int64_t g_stride, const T *V, int64_t v_stride, int m, T *r, T *rho, void *workspace, int flags,
+                       int64_t B, gpde_stream_t stream) {
     if (!pl || B < 0 || m < 0) return fail(GPDE_ERR_ARG, "vo_residual: bad argument");
+    if (v_stride != 0 && (m == 0 || v_stride != (int64_t)pl->dev.d * m))
+        return fail(GPDE_ERR_ARG, "vo_residual: v_stride must be 0, or d*m with m > 0");
     if (B == 0) return GPDE_OK;
     if (!a) return fail(GPDE_ERR_ARG, "vo_residual: null conductivity field");
     if (m > 0 && (!V || !r)) return fail(GPDE_ERR_ARG, "vo_residual: V and r are required when m > 0");
     if (m > 0 && !workspace) return fail(GPDE_ERR_ARG, "vo_residual: workspace required");
     if (m == 0 && !rho) return fail(GPDE_ERR_ARG, "vo_residual: nothing to compute");
-    if (B == 0) return GPDE_OK;
+    if (v_stride) {   // r_b = V_b^T rho_b: the rho-only residual (whichever kernel the plan picks for it), then the contraction
+        if ((uintptr_t)workspace & 15) return fail(GPDE_ERR_ARG, "vo_residual: a per-sample V needs a 16-byte aligned workspace");
+        if (flags & 2) return fail(GPDE_ERR_ARG, "vo_residual: packed weights (flags bit1) are a shared-V layout");
+        T *rb = rho ? rho : (T *)workspace;   // rho [B,d]: the caller's, else the workspace
+        const int rc = vo_residual<T>(pl, a, a_stride, a_is_log, y, g, g_stride, nullptr, 0, 0, nullptr, rb, nullptr, flags & 1,
+                                      B, stream);
+        if (rc != GPDE_OK) return rc;
+        DeviceGuard guard(pl->device);
+        const int npan = (m + kVbPanel - 1) / kVbPanel;
+        const unsigned grid = (unsigned)std::min<long long>((long long)B * npan, (long long)pl->n_sm * 64);
+        vo_vb_contract_kernel<T><<<grid, kVbThreads, 0, (cudaStream_t)stream>>>(V, rb, r, pl->dev.d, m, (long long)B);
+        GPDE_CUDA_OK(cudaGetLastError());
+        return GPDE_OK;
+    }
     DeviceGuard guard(pl->device);
     cudaStream_t st = (cudaStream_t)stream;
     if (m > 0 && !rho && use_grid(pl)) {
@@ -999,36 +1014,44 @@ static int launch_expand(const gpde_vo_plan *pl, const T *s, const T *V, int m, 
     return GPDE_OK;
 }
 
+// One weighting matrix per sample (vo_vb.cuh): w_b = V_b s_b, FP64 rows of pitch ldw.  The rows are padded to 4 doubles
+// (vb_ldw) for the strided-y marching kernel, as launch_expand pads them.
+static long long vb_ldw(const gpde_vo_plan *pl) { return ((long long)pl->dev.d + 3) & ~3ll; }
 template <typename T>
-static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *V, int m,
-                         const T *s, T *q, void *workspace, int64_t B, gpde_stream_t stream) {
+static int launch_vb_expand(const gpde_vo_plan *pl, const T *V, const T *s, int m, double *w, long long ldw, long long B,
+                            cudaStream_t st) {
+    const long long jobs = B * ((pl->dev.d + kVbRows - 1) / kVbRows);
+    const unsigned grid = (unsigned)std::min<long long>(jobs, (long long)pl->n_sm * 64);
+    vo_vb_expand_kernel<T><<<grid, kVbExpThreads, 0, st>>>(V, s, w, ldw, pl->dev.d, m, B);
+    GPDE_CUDA_OK(cudaGetLastError());
+    return GPDE_OK;
+}
+
+template <typename T>
+static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *V, int64_t v_stride,
+                         int m, const T *s, T *q, void *workspace, int64_t B, gpde_stream_t stream) {
     if (!pl || m <= 0 || B < 0) return fail(GPDE_ERR_ARG, "vo_residual_T: bad argument");
+    if (v_stride != 0 && v_stride != (int64_t)pl->dev.d * m) return fail(GPDE_ERR_ARG, "vo_residual_T: v_stride must be 0 or d*m");
     if (B == 0) return GPDE_OK;
     if (!a || !V || !s || !q || !workspace) return fail(GPDE_ERR_ARG, "vo_residual_T: null argument");
+    if (v_stride && ((uintptr_t)workspace & 15))
+        return fail(GPDE_ERR_ARG, "vo_residual_T: a per-sample V needs a 16-byte aligned workspace");
     DeviceGuard guard(pl->device);
     cudaStream_t st = (cudaStream_t)stream;
-    if (use_grid(pl) && m <= 32) {   // one kernel: w = s V^T never leaves the SM
+    if (!v_stride && use_grid(pl) && m <= 32) {   // one kernel: w = s V^T never leaves the SM
         const int rc = launch_grid2_wt<T>(pl, a, (long long)a_stride, a_is_log, V, m, s, q, workspace, (long long)B, st);
         if (rc != 0) return rc < 0 ? rc : GPDE_OK;
     }
-    // structured pixel grid: w = s V^T on the FP64 tensor pipe, then q = K_ff w with the marching kernel (rho of u~ = (w, 0)
-    // without the load vector IS K_ff w); FP32 I/O: s and V converted on load, w stays FP64, a staged and q stored as floats
+    // structured pixel grid: w = s V^T on the FP64 tensor pipe (per-sample V: the expansion kernel), then q = K_ff w with the
+    // marching kernel (rho of u~ = (w, 0) without the load vector IS K_ff w); FP32 I/O: s and V converted on load, w stays
+    // FP64, a staged and q stored as floats
     Grid2Dev G2;
     int nt2, nx2;
     size_t smem2;
-    if (use_grid(pl) && (m <= 32 || sizeof(T) == 8) && grid2_a_aligned(pl, a, (long long)a_stride, (int)sizeof(T)) &&
-        !((uintptr_t)workspace & 15) && grid2_setup(pl, 0, true, 0, G2, nt2, nx2, smem2, (int)sizeof(T), 8)) {
-        const int d = pl->dev.d;
-        double *w;
-        long long ldw;
-        const int rce = launch_expand<T>(pl, s, V, m, workspace, (long long)B, st, w, ldw);
-        if (rce != GPDE_OK) return rce;
-        const int rc = launch_grid2<T, double, T>(pl, a, (long long)a_stride, a_is_log, w, nullptr, 0, nullptr, 0, q, nullptr, d, 0,
-                                                  false, (long long)B, st, ldw);
-        if (rc != 0) return rc < 0 ? rc : GPDE_OK;
-        return fail(GPDE_ERR_ARG, "vo_residual_T: lean grid kernel declined after setup");
-    }
-    if (use_fused(pl) && sizeof(double) * kFS * (size_t)m <= sizeof(double) * kFS * kRhoPitch) {
+    const bool on_grid = use_grid(pl) && (v_stride || m <= 32 || sizeof(T) == 8) &&
+                         grid2_a_aligned(pl, a, (long long)a_stride, (int)sizeof(T)) && !((uintptr_t)workspace & 15) &&
+                         grid2_setup(pl, 0, true, 0, G2, nt2, nx2, smem2, (int)sizeof(T), 8);
+    if (!on_grid && !v_stride && use_fused(pl) && sizeof(double) * kFS * (size_t)m <= sizeof(double) * kFS * kRhoPitch) {
         const unsigned grid = (unsigned)((B + kFS - 1) / kFS);
         const size_t smem = pl->fused_smem;   // the coefficient vectors live in the (unused) rho tile
         auto kern = vo_fused_T_kernel<T>;
@@ -1037,13 +1060,29 @@ static int vo_residual_T(const gpde_vo_plan *pl, const T *a, int64_t a_stride, i
         GPDE_CUDA_OK(cudaGetLastError());
         return GPDE_OK;
     }
+    const int d = pl->dev.d;
     double *w = (double *)workspace;
-    const long long total = B * (long long)pl->dev.d;
-    const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, (long long)pl->n_sm * 16);
-    vo_expand_kernel<T><<<grid, 256, 0, st>>>(s, V, w, B, pl->dev.d, m);
-    GPDE_CUDA_OK(cudaGetLastError());
-    return launch_matvec<T, double, T>(pl, a, a_stride, a_is_log, w, (const T *)nullptr, 0, 0, (double *)nullptr, 0,
-                                       q, B, st);
+    long long ldw = d;   // the generic matvec reads w with pitch d
+    if (v_stride) {
+        if (on_grid) ldw = vb_ldw(pl);
+        const int rce = launch_vb_expand<T>(pl, V, s, m, w, ldw, (long long)B, st);
+        if (rce != GPDE_OK) return rce;
+    } else if (on_grid) {
+        const int rce = launch_expand<T>(pl, s, V, m, workspace, (long long)B, st, w, ldw);
+        if (rce != GPDE_OK) return rce;
+    } else {
+        const long long total = B * (long long)d;
+        const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, (long long)pl->n_sm * 16);
+        vo_expand_kernel<T><<<grid, 256, 0, st>>>(s, V, w, B, d, m);
+        GPDE_CUDA_OK(cudaGetLastError());
+    }
+    if (on_grid) {
+        const int rc = launch_grid2<T, double, T>(pl, a, (long long)a_stride, a_is_log, w, nullptr, 0, nullptr, 0, q, nullptr, d, 0,
+                                                  false, (long long)B, st, ldw);
+        if (rc != 0) return rc < 0 ? rc : GPDE_OK;
+        return fail(GPDE_ERR_ARG, "vo_residual_T: lean grid kernel declined after setup");
+    }
+    return launch_matvec<T, double, T>(pl, a, a_stride, a_is_log, w, (const T *)nullptr, 0, 0, (double *)nullptr, 0, q, B, st);
 }
 
 // grad_a (marching kernel on pixel grids, per-input cell lists otherwise) and grad_g (Dirichlet rows of K(a)) from
@@ -1077,129 +1116,32 @@ static int launch_grad(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int
     return GPDE_OK;
 }
 
-// gpde_vo_residual_grad_*: w = gbar_r V^T, then launch_grad.
+// gpde_vo_residual_grad_*: w = gbar_r V^T (per-sample V: w_b = V_b gbar_r_b), then launch_grad.
 template <typename T>
 static int vo_residual_grad(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *y, const T *g,
-                            int64_t g_stride, const T *V, int m, const T *gbar_r, T *grad_a, T *grad_g, void *workspace,
-                            int64_t B, gpde_stream_t stream) {
+                            int64_t g_stride, const T *V, int64_t v_stride, int m, const T *gbar_r, T *grad_a, T *grad_g,
+                            void *workspace, int64_t B, gpde_stream_t stream) {
     if (!pl || B < 0) return fail(GPDE_ERR_ARG, "vo_residual_grad: bad argument (null plan or B < 0)");
     if (m <= 0) return fail(GPDE_ERR_ARG, "vo_residual_grad: m = %d weighting functions (must be > 0)", m);
     if (a_stride != 0 && a_stride != pl->dev.n_inputs)
         return fail(GPDE_ERR_ARG, "vo_residual_grad: a_stride must be 0 or n_inputs = %d", pl->dev.n_inputs);
     if (g_stride != 0 && g_stride != pl->dev.n_bc)
         return fail(GPDE_ERR_ARG, "vo_residual_grad: g_stride must be 0 or n_bc = %d", pl->dev.n_bc);
+    if (v_stride != 0 && v_stride != (int64_t)pl->dev.d * m)
+        return fail(GPDE_ERR_ARG, "vo_residual_grad: v_stride must be 0 or d*m");
     if (B == 0) return GPDE_OK;
     if (!V || !gbar_r) return fail(GPDE_ERR_ARG, "vo_residual_grad: V and gbar_r are required");
     if (!a) return fail(GPDE_ERR_ARG, "vo_residual_grad: null conductivity field");
     if (!workspace || ((uintptr_t)workspace & 15))
         return fail(GPDE_ERR_ARG, "vo_residual_grad: workspace must be non-NULL and 16-byte aligned "
-                                  "(>= gpde_vo_grad_workspace_bytes)");
-    if (!grad_a && !grad_g) return GPDE_OK;
-    DeviceGuard guard(pl->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    double *w;
-    long long ldw;
-    const int rce = launch_expand<T>(pl, gbar_r, V, m, workspace, (long long)B, st, w, ldw);
-    if (rce != GPDE_OK) return rce;
-    return launch_grad<T>(pl, a, a_stride, a_is_log, y, g, g_stride, w, ldw, grad_a, grad_g, B, st);
-}
-
-// ---- one weighting matrix per sample (vo_vb.cuh): V [B,d,m], v_stride = d*m
-// Row pitch of the FP64 rows w = V_b s_b: padded to 4 doubles for the strided-y marching kernel (as launch_expand does).
-static long long vb_ldw(const gpde_vo_plan *pl) { return ((long long)pl->dev.d + 3) & ~3ll; }
-
-// The argument checks common to the three per-sample entry points; 1 = go on, 0 = B == 0 (no-op), < 0 = error.
-static int vb_check(const gpde_vo_plan *pl, const char *what, int m, int64_t v_stride, int64_t B, const void *V,
-                    const void *workspace) {
-    if (!pl || B < 0) return fail(GPDE_ERR_ARG, "%s: bad argument (null plan or B < 0)", what);
-    if (m <= 0) return fail(GPDE_ERR_ARG, "%s: m = %d weighting functions (must be > 0)", what, m);
-    if (v_stride != (int64_t)pl->dev.d * m)
-        return fail(GPDE_ERR_ARG, "%s: v_stride = %lld must be d*m = %lld", what, (long long)v_stride, (long long)pl->dev.d * m);
-    if (B == 0) return 0;
-    if (!V) return fail(GPDE_ERR_ARG, "%s: null V", what);
-    if (!workspace || ((uintptr_t)workspace & 15))
-        return fail(GPDE_ERR_ARG, "%s: workspace must be non-NULL and 16-byte aligned (>= gpde_vo_vb_workspace_bytes)", what);
-    return 1;
-}
-
-template <typename T>
-static int launch_vb_expand(const gpde_vo_plan *pl, const T *V, const T *s, int m, double *w, long long ldw, long long B,
-                            cudaStream_t st) {
-    const long long jobs = B * ((pl->dev.d + kVbRows - 1) / kVbRows);
-    const unsigned grid = (unsigned)std::min<long long>(jobs, (long long)pl->n_sm * 64);
-    vo_vb_expand_kernel<T><<<grid, kVbExpThreads, 0, st>>>(V, s, w, ldw, pl->dev.d, m, B);
-    GPDE_CUDA_OK(cudaGetLastError());
-    return GPDE_OK;
-}
-
-// r_b = V_b^T rho_b: the rho-only residual (whichever kernel the plan picks for it), then the contraction.
-template <typename T>
-static int vo_residual_vb(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *y, const T *g,
-                          int64_t g_stride, const T *V, int64_t v_stride, int m, T *r, T *rho, void *workspace, int flags,
-                          int64_t B, gpde_stream_t stream) {
-    const int ck = vb_check(pl, "vo_residual_vb", m, v_stride, B, V, workspace);
-    if (ck <= 0) return ck;
-    if (!a || !r) return fail(GPDE_ERR_ARG, "vo_residual_vb: a and r are required");
-    if (flags & 2) return fail(GPDE_ERR_ARG, "vo_residual_vb: packed weights (flags bit1) are a shared-V layout");
-    T *rb = rho ? rho : (T *)workspace;   // rho [B,d]: the caller's, else the workspace
-    const int rc = vo_residual<T>(pl, a, a_stride, a_is_log, y, g, g_stride, nullptr, 0, nullptr, rb, nullptr, flags & 1, B,
-                                  stream);
-    if (rc != GPDE_OK) return rc;
-    DeviceGuard guard(pl->device);
-    const int npan = (m + kVbPanel - 1) / kVbPanel;
-    const unsigned grid = (unsigned)std::min<long long>((long long)B * npan, (long long)pl->n_sm * 64);
-    vo_vb_contract_kernel<T><<<grid, kVbThreads, 0, (cudaStream_t)stream>>>(V, rb, r, pl->dev.d, m, (long long)B);
-    GPDE_CUDA_OK(cudaGetLastError());
-    return GPDE_OK;
-}
-
-// q_b = K_ff(a_b) (V_b s_b): the expansion into the workspace, then the K_ff application of residual_T's two-kernel
-// route (strided-y marching kernel on pixel grids, the generic matvec otherwise).
-template <typename T>
-static int vo_residual_T_vb(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *V, int64_t v_stride,
-                            int m, const T *s, T *q, void *workspace, int64_t B, gpde_stream_t stream) {
-    const int ck = vb_check(pl, "vo_residual_T_vb", m, v_stride, B, V, workspace);
-    if (ck <= 0) return ck;
-    if (!a || !s || !q) return fail(GPDE_ERR_ARG, "vo_residual_T_vb: null argument");
-    DeviceGuard guard(pl->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    const int d = pl->dev.d;
-    Grid2Dev G2;
-    int nt2, nx2;
-    size_t smem2;
-    const bool grid = use_grid(pl) && grid2_a_aligned(pl, a, (long long)a_stride, (int)sizeof(T)) &&
-                      grid2_setup(pl, 0, true, 0, G2, nt2, nx2, smem2, (int)sizeof(T), 8);
-    const long long ldw = grid ? vb_ldw(pl) : d;   // the generic matvec reads y with pitch d
-    double *w = (double *)workspace;
-    const int rce = launch_vb_expand<T>(pl, V, s, m, w, ldw, (long long)B, st);
-    if (rce != GPDE_OK) return rce;
-    if (grid) {
-        const int rc = launch_grid2<T, double, T>(pl, a, (long long)a_stride, a_is_log, w, nullptr, 0, nullptr, 0, q, nullptr, d, 0,
-                                                  false, (long long)B, st, ldw);
-        if (rc != 0) return rc < 0 ? rc : GPDE_OK;
-        return fail(GPDE_ERR_ARG, "vo_residual_T_vb: lean grid kernel declined after setup");
-    }
-    return launch_matvec<T, double, T>(pl, a, a_stride, a_is_log, w, (const T *)nullptr, 0, 0, (double *)nullptr, 0, q, B, st);
-}
-
-// grad_a / grad_g of r_b = V_b^T rho_b: the expansion w_b = V_b gbar_r_b, then launch_grad.
-template <typename T>
-static int vo_residual_grad_vb(const gpde_vo_plan *pl, const T *a, int64_t a_stride, int a_is_log, const T *y, const T *g,
-                               int64_t g_stride, const T *V, int64_t v_stride, int m, const T *gbar_r, T *grad_a, T *grad_g,
-                               void *workspace, int64_t B, gpde_stream_t stream) {
-    if (pl && a_stride != 0 && a_stride != pl->dev.n_inputs)
-        return fail(GPDE_ERR_ARG, "vo_residual_grad_vb: a_stride must be 0 or n_inputs = %d", pl->dev.n_inputs);
-    if (pl && g_stride != 0 && g_stride != pl->dev.n_bc)
-        return fail(GPDE_ERR_ARG, "vo_residual_grad_vb: g_stride must be 0 or n_bc = %d", pl->dev.n_bc);
-    const int ck = vb_check(pl, "vo_residual_grad_vb", m, v_stride, B, V, workspace);
-    if (ck <= 0) return ck;
-    if (!a || !gbar_r) return fail(GPDE_ERR_ARG, "vo_residual_grad_vb: a and gbar_r are required");
+                                  "(>= gpde_vo_workspace_bytes)");
     if (!grad_a && !grad_g) return GPDE_OK;
     DeviceGuard guard(pl->device);
     cudaStream_t st = (cudaStream_t)stream;
     double *w = (double *)workspace;
-    const long long ldw = vb_ldw(pl);
-    const int rce = launch_vb_expand<T>(pl, V, gbar_r, m, w, ldw, (long long)B, st);
+    long long ldw = vb_ldw(pl);
+    const int rce = v_stride ? launch_vb_expand<T>(pl, V, gbar_r, m, w, ldw, (long long)B, st)
+                             : launch_expand<T>(pl, gbar_r, V, m, workspace, (long long)B, st, w, ldw);
     if (rce != GPDE_OK) return rce;
     return launch_grad<T>(pl, a, a_stride, a_is_log, y, g, g_stride, w, ldw, grad_a, grad_g, B, st);
 }
@@ -1358,12 +1300,9 @@ size_t gpde_vo_workspace_bytes(const gpde_vo_plan *pl, int64_t B, int m) {
         // packed V^T rows of the one-kernel transposed application (launch_grid2_wt): <= 8 k-steps
         need = std::max(need, (size_t)(pl->grid.ny + 1) * ((size_t)((pl->grid.nx + 15) / 16) * 2 * 8 * 256 + kGrid2MaskBytes));
     }
+    // w = gbar_r V^T of residual_grad; a per-sample V's rho [B,d] or rows V_b s_b [B][vb_ldw] take no more than this
+    if (m > 0) need = std::max(need, expand_bytes(pl, (long long)B, m));
     return need;
-}
-
-size_t gpde_vo_grad_workspace_bytes(const gpde_vo_plan *pl, int64_t B, int m) {
-    if (!pl || B < 0 || m <= 0) return 0;
-    return expand_bytes(pl, (long long)B, m);
 }
 
 int gpde_vo_pack_weights_f64(const gpde_vo_plan *pl, const double *V, int m, int flags, void *workspace,
@@ -1557,73 +1496,39 @@ int gpde_vo_energy_step_blocked_f64(const gpde_vo_plan *pl, const double *a, int
 }
 
 int gpde_vo_residual_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *y,
-                         const double *g, int64_t g_stride, const double *V, int m, double *r, double *rho,
-                         void *workspace, int flags, int64_t B, gpde_stream_t stream) {
-    return vo_residual<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, m, r, rho, workspace, flags, B, stream);
+                         const double *g, int64_t g_stride, const double *V, int64_t v_stride, int m, double *r,
+                         double *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream) {
+    return vo_residual<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, r, rho, workspace, flags, B, stream);
 }
 int gpde_vo_residual_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *y,
-                         const float *g, int64_t g_stride, const float *V, int m, float *r, float *rho,
-                         void *workspace, int flags, int64_t B, gpde_stream_t stream) {
-    return vo_residual<float>(pl, a, a_stride, a_is_log, y, g, g_stride, V, m, r, rho, workspace, flags, B, stream);
+                         const float *g, int64_t g_stride, const float *V, int64_t v_stride, int m, float *r,
+                         float *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream) {
+    return vo_residual<float>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, r, rho, workspace, flags, B, stream);
 }
 int gpde_vo_residual_T_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *V,
-                           int m, const double *s, double *q, void *workspace, int64_t B, gpde_stream_t stream) {
-    return vo_residual_T<double>(pl, a, a_stride, a_is_log, V, m, s, q, workspace, B, stream);
+                           int64_t v_stride, int m, const double *s, double *q, void *workspace, int64_t B,
+                           gpde_stream_t stream) {
+    return vo_residual_T<double>(pl, a, a_stride, a_is_log, V, v_stride, m, s, q, workspace, B, stream);
 }
 int gpde_vo_residual_T_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *V,
-                           int m, const float *s, float *q, void *workspace, int64_t B, gpde_stream_t stream) {
-    return vo_residual_T<float>(pl, a, a_stride, a_is_log, V, m, s, q, workspace, B, stream);
+                           int64_t v_stride, int m, const float *s, float *q, void *workspace, int64_t B,
+                           gpde_stream_t stream) {
+    return vo_residual_T<float>(pl, a, a_stride, a_is_log, V, v_stride, m, s, q, workspace, B, stream);
 }
 
 int gpde_vo_residual_grad_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *y,
-                              const double *g, int64_t g_stride, const double *V, int m, const double *gbar_r, double *grad_a,
-                              double *grad_g, void *workspace, int64_t B, gpde_stream_t stream) {
-    return vo_residual_grad<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, m, gbar_r, grad_a, grad_g, workspace, B, stream);
+                              const double *g, int64_t g_stride, const double *V, int64_t v_stride, int m,
+                              const double *gbar_r, double *grad_a, double *grad_g, void *workspace, int64_t B,
+                              gpde_stream_t stream) {
+    return vo_residual_grad<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, gbar_r, grad_a, grad_g,
+                                    workspace, B, stream);
 }
 int gpde_vo_residual_grad_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *y,
-                              const float *g, int64_t g_stride, const float *V, int m, const float *gbar_r, float *grad_a,
-                              float *grad_g, void *workspace, int64_t B, gpde_stream_t stream) {
-    return vo_residual_grad<float>(pl, a, a_stride, a_is_log, y, g, g_stride, V, m, gbar_r, grad_a, grad_g, workspace, B, stream);
-}
-
-size_t gpde_vo_vb_workspace_bytes(const gpde_vo_plan *pl, int64_t B, int m) {
-    if (!pl || B < 0 || m <= 0) return 0;
-    return sizeof(double) * (size_t)B * (size_t)vb_ldw(pl);
-}
-
-int gpde_vo_residual_vb_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *y,
-                            const double *g, int64_t g_stride, const double *V, int64_t v_stride, int m, double *r,
-                            double *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream) {
-    return vo_residual_vb<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, r, rho, workspace, flags, B, stream);
-}
-int gpde_vo_residual_vb_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *y,
-                            const float *g, int64_t g_stride, const float *V, int64_t v_stride, int m, float *r,
-                            float *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream) {
-    return vo_residual_vb<float>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, r, rho, workspace, flags, B, stream);
-}
-int gpde_vo_residual_T_vb_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *V,
-                              int64_t v_stride, int m, const double *s, double *q, void *workspace, int64_t B,
+                              const float *g, int64_t g_stride, const float *V, int64_t v_stride, int m,
+                              const float *gbar_r, float *grad_a, float *grad_g, void *workspace, int64_t B,
                               gpde_stream_t stream) {
-    return vo_residual_T_vb<double>(pl, a, a_stride, a_is_log, V, v_stride, m, s, q, workspace, B, stream);
-}
-int gpde_vo_residual_T_vb_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *V,
-                              int64_t v_stride, int m, const float *s, float *q, void *workspace, int64_t B,
-                              gpde_stream_t stream) {
-    return vo_residual_T_vb<float>(pl, a, a_stride, a_is_log, V, v_stride, m, s, q, workspace, B, stream);
-}
-int gpde_vo_residual_grad_vb_f64(const gpde_vo_plan *pl, const double *a, int64_t a_stride, int a_is_log, const double *y,
-                                 const double *g, int64_t g_stride, const double *V, int64_t v_stride, int m,
-                                 const double *gbar_r, double *grad_a, double *grad_g, void *workspace, int64_t B,
-                                 gpde_stream_t stream) {
-    return vo_residual_grad_vb<double>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, gbar_r, grad_a, grad_g,
-                                       workspace, B, stream);
-}
-int gpde_vo_residual_grad_vb_f32(const gpde_vo_plan *pl, const float *a, int64_t a_stride, int a_is_log, const float *y,
-                                 const float *g, int64_t g_stride, const float *V, int64_t v_stride, int m,
-                                 const float *gbar_r, float *grad_a, float *grad_g, void *workspace, int64_t B,
-                                 gpde_stream_t stream) {
-    return vo_residual_grad_vb<float>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, gbar_r, grad_a, grad_g,
-                                      workspace, B, stream);
+    return vo_residual_grad<float>(pl, a, a_stride, a_is_log, y, g, g_stride, V, v_stride, m, gbar_r, grad_a, grad_g,
+                                   workspace, B, stream);
 }
 
 }  // extern "C"

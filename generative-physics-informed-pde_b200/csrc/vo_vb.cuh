@@ -1,8 +1,8 @@
 // One weighting matrix per sample: V [B,d,m] (V_b = V + b d m).  Included by vo.cu.
 //
-// The per-sample residual family (gpde_vo_residual_vb_*, _T_vb_*, _grad_vb_*) reuses the launches of the shared-V
-// routes for everything that involves K(a): the rho-only residual, the K_ff application of residual_T and the gradient
-// kernels of vo_grad.cuh.  What changes with a per-sample V is the contraction with V, which these two kernels do:
+// The residual family with a per-sample V (gpde_vo_residual_*, _T_*, _grad_* with v_stride = d*m) reuses the shared-V
+// routes' launches for everything that involves K(a): the rho-only residual, the K_ff application of residual_T and the
+// gradient kernels of vo_grad.cuh.  What changes with a per-sample V is the contraction with V, which these kernels do:
 //   vo_vb_contract_kernel   r[b,:] = V_b^T rho_b
 //   vo_vb_expand_kernel     w[b,:] = V_b s_b          (FP64 rows of pitch ldw, the input of the K_ff application)
 // Both stream V_b once (8 d m bytes per sample in FP64, against 8 d for rho_b or w_b): they are bound by HBM bandwidth,

@@ -46,7 +46,7 @@ typedef struct gpde_rom_plan gpde_rom_plan;
 typedef struct gpde_vo_plan gpde_vo_plan;
 typedef void *gpde_stream_t; /* cudaStream_t */
 
-int gpde_version(void);
+int gpde_version(void); /* 101: the residual family takes v_stride after V */
 const char *gpde_last_error(void);
 
 /* ------------------------------------------------------------------ coarse-grained model */
@@ -169,29 +169,43 @@ int gpde_vo_plan_info(const gpde_vo_plan *plan, int64_t out[8]);
  * aligned, that pass y = NULL or that ask for rho fall back from 2 to 1. */
 int gpde_vo_plan_kernel_path(const gpde_vo_plan *plan, int m, int elem_bytes);
 
-/* scratch bytes for residual / residual_T on B samples with m weighting functions */
+/* scratch bytes for any residual / residual_T / residual_grad call on B samples with m weighting functions, either
+ * layout of V (v_stride = 0 or d*m) */
 size_t gpde_vo_workspace_bytes(const gpde_vo_plan *plan, int64_t B, int m);
 
-/* r[B,m] = V^T (K_fom(a_b) u~_b - f)_free ,  u~ = y on free dofs, g on constrained dofs
+/* The residual family (gpde_vo_residual_*, gpde_vo_residual_T_*, gpde_vo_residual_grad_*) takes V row-major with
+ * V_b = V + b*v_stride: v_stride = 0 shares one V [d,m] across the batch, v_stride = d*m gives one matrix per sample,
+ * V [B,d,m]; any other value returns GPDE_ERR_ARG.  With one matrix per sample the fine residual comes from the rho-only
+ * route of gpde_vo_residual_* (the kernel the plan picks for it), then one contraction kernel streams V_b once; the
+ * transposed application and the gradient first form the FP64 rows V_b s_b in the workspace with one expansion kernel,
+ * then run the K_ff application of gpde_vo_residual_T_* (strided-y marching kernel on pixel grids, generic matvec
+ * otherwise) or the gradient kernels.  Any m >= 1; FP32 I/O reads V, rho and s as floats and accumulates in FP64 (rho
+ * itself is held as floats); the workspace must be 16-byte aligned; sums run in a fixed order, so results are
+ * deterministic.  B = 0 is a no-op in either layout.
+ *
+ * r[B,m] = V^T (K_fom(a_b) u~_b - f)_free ,  u~ = y on free dofs, g on constrained dofs
  *        = Gamma_b y_b - alpha_b   (VirtualObservables.py:61-69, 662, 990).
  *   a   [B or 1, n_inputs]  (a_stride = n_inputs, or 0 to share one field across the batch)
  *   a_is_log != 0: a holds log-conductivities (QuerryPoint.x), exp() applied inside
  *   y   [B,d]   (NULL = zeros);  g [B or 1, n_bc] with g_stride = n_bc or 0 (NULL = zeros)
- *   V   [d,m] row-major weighting matrix (NULL with m=0: only rho is produced)
+ *   V   [d,m] or [B,d,m] (v_stride) weighting matrices (NULL with m=0 and v_stride=0: only rho is produced)
  *   rho [B,d] optional output of the fine residual itself (may be NULL)
  *   flags: bit0 = ignore the load vector f
  *          bit1 = `workspace` already holds V packed by gpde_vo_pack_weights_f64 (same plan, m, bit0):
  *                 the call skips its packing launch; it fails with GPDE_ERR_ARG instead of falling
- *                 back when the lean structured-grid kernel cannot serve it (V must still be passed)
+ *                 back when the lean structured-grid kernel cannot serve it (V must still be passed);
+ *                 packing is for a shared V only: bit1 with v_stride != 0 returns GPDE_ERR_ARG
  *          bits 8-15 = number of SMs to leave to kernels the caller runs beside this call on other streams
- *                 (the structured-grid kernel sizes its last wave for the remaining SMs; 0 = all SMs)  */
+ *                 (the structured-grid kernel sizes its last wave for the remaining SMs; 0 = all SMs)
+ *   workspace: >= gpde_vo_workspace_bytes(plan, B, m) when m > 0 (per-sample V: it holds rho [B,d] when the caller
+ *                 passes no rho output) */
 int gpde_vo_residual_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
-                         const double *y, const double *g, int64_t g_stride, const double *V, int m,
-                         double *r, double *rho, void *workspace, int flags, int64_t B,
+                         const double *y, const double *g, int64_t g_stride, const double *V, int64_t v_stride,
+                         int m, double *r, double *rho, void *workspace, int flags, int64_t B,
                          gpde_stream_t stream);
 int gpde_vo_residual_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
-                         const float *y, const float *g, int64_t g_stride, const float *V, int m,
-                         float *r, float *rho, void *workspace, int flags, int64_t B,
+                         const float *y, const float *g, int64_t g_stride, const float *V, int64_t v_stride,
+                         int m, float *r, float *rho, void *workspace, int flags, int64_t B,
                          gpde_stream_t stream);
 
 /* Packs V[d,m] once into `workspace` (>= gpde_vo_workspace_bytes(plan, B, m), 16-byte aligned) in the
@@ -268,75 +282,40 @@ int gpde_vo_energy_step_blocked_f64(const gpde_vo_plan *plan, const double *a, i
                                     const double *inv_T, double *mean, int *info, void *workspace,
                                     size_t workspace_bytes, int64_t N, gpde_stream_t stream);
 
-/* q[B,d] = K_ff(a_b) (V s_b) = Gamma_b^T s_b  (VirtualObservables.py:663; with s = P r it is the
- * gradient of 1/2 r^T P r w.r.t. y).  With B = m, s = I and a_stride = 0 it yields Gamma itself.
- * On the reference's pixel meshes with m <= 32 this is one kernel (after a small packing launch of V^T): the rows
- * of V s are produced inside the marching kernel and never reach global memory; `workspace` holds the packed V^T
- * (or, on the other routes, V s [B,d]): >= gpde_vo_workspace_bytes(plan, B, m), 16-byte aligned. */
+/* q[B,d] = K_ff(a_b) (V_b s_b) = Gamma_b^T s_b  (VirtualObservables.py:663; with s = P r it is the
+ * gradient of 1/2 r^T P r w.r.t. y).  With B = m, s = I, a_stride = 0 and a shared V it yields Gamma itself.
+ * On the reference's pixel meshes with m <= 32 and a shared V this is one kernel (after a small packing launch of V^T):
+ * the rows of V s are produced inside the marching kernel and never reach global memory; `workspace` holds the packed
+ * V^T (or, on the other routes, V s [B,d]): >= gpde_vo_workspace_bytes(plan, B, m), 16-byte aligned.  V, v_stride as
+ * for gpde_vo_residual_*. */
 int gpde_vo_residual_T_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
-                           const double *V, int m, const double *s, double *q, void *workspace,
+                           const double *V, int64_t v_stride, int m, const double *s, double *q, void *workspace,
                            int64_t B, gpde_stream_t stream);
 int gpde_vo_residual_T_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
-                           const float *V, int m, const float *s, float *q, void *workspace,
+                           const float *V, int64_t v_stride, int m, const float *s, float *q, void *workspace,
                            int64_t B, gpde_stream_t stream);
 
 /* Gradient of r = gpde_vo_residual_*(a, y, g, V) with respect to the conductivity input and the Dirichlet values, for
- * an incoming gradient gbar_r [B,m].  With w~_b = V gbar_r_b on the free dofs and 0 on the Dirichlet dofs, and since
+ * an incoming gradient gbar_r [B,m].  With w~_b = V_b gbar_r_b on the free dofs and 0 on the Dirichlet dofs, and since
  * K(a) = sum_c a[cell_to_input[c]] K_c is linear in a:
  *     grad_a[b,p] = sum_{c : cell_to_input[c] = p} w~_b[c]^T K_c u~_b[c]     ([c] = the three dofs of cell c)
  *     grad_g[b,k] = (K_cf(a_b) w~_b)_k                                       (the Dirichlet rows of K(a) applied to w~)
  * a_is_log != 0: a holds x with a = exp(x) (no offset), and grad_a is the gradient in x: exp(x) times the above.
  * The load vector does not enter either gradient.  Arguments as for gpde_vo_residual_*: a [B or 1, n_inputs]
- * (a_stride = n_inputs or 0), y [B,d] (NULL = zeros), g [B or 1, n_bc] (g_stride = n_bc or 0, NULL = zeros), V [d,m].
- * Outputs are per sample even when a_stride or g_stride is 0: grad_a [B,n_inputs], grad_g [B,n_bc]; either may be NULL.
- * workspace: >= gpde_vo_grad_workspace_bytes(plan, B, m), 16-byte aligned (it holds w = gbar_r V^T in FP64; FP32 I/O
- * computes in FP64 too).  B = 0 is a no-op.  m <= 0, a NULL gbar_r, V or a, a bad stride or a NULL or misaligned
- * workspace return GPDE_ERR_ARG.  Every output is written by one thread in a fixed order: results are deterministic. */
-size_t gpde_vo_grad_workspace_bytes(const gpde_vo_plan *plan, int64_t B, int m);
+ * (a_stride = n_inputs or 0), y [B,d] (NULL = zeros), g [B or 1, n_bc] (g_stride = n_bc or 0, NULL = zeros), V and
+ * v_stride.  Outputs are per sample even when a_stride or g_stride is 0: grad_a [B,n_inputs], grad_g [B,n_bc]; either
+ * may be NULL.  workspace: >= gpde_vo_workspace_bytes(plan, B, m), 16-byte aligned (it holds w = gbar_r V^T in FP64;
+ * FP32 I/O computes in FP64 too).  B = 0 is a no-op.  m <= 0, a NULL gbar_r, V or a, a bad stride or a NULL or
+ * misaligned workspace return GPDE_ERR_ARG.  Every output is written by one thread in a fixed order: results are
+ * deterministic. */
 int gpde_vo_residual_grad_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
-                              const double *y, const double *g, int64_t g_stride, const double *V, int m,
-                              const double *gbar_r, double *grad_a, double *grad_g, void *workspace,
+                              const double *y, const double *g, int64_t g_stride, const double *V, int64_t v_stride,
+                              int m, const double *gbar_r, double *grad_a, double *grad_g, void *workspace,
                               int64_t B, gpde_stream_t stream);
 int gpde_vo_residual_grad_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
-                              const float *y, const float *g, int64_t g_stride, const float *V, int m,
-                              const float *gbar_r, float *grad_a, float *grad_g, void *workspace,
+                              const float *y, const float *g, int64_t g_stride, const float *V, int64_t v_stride,
+                              int m, const float *gbar_r, float *grad_a, float *grad_g, void *workspace,
                               int64_t B, gpde_stream_t stream);
-
-/* ---- the residual family with one weighting matrix per sample: V [B,d,m] row-major, V_b = V + b*v_stride, and v_stride
- * must be d*m (for one matrix shared by the batch use the entry points above).  Same definitions with V indexed by sample:
- *     gpde_vo_residual_vb_*       r[b,:] = V_b^T rho_b,   rho_b = (K_fom(a_b) u~_b - f)_free
- *     gpde_vo_residual_T_vb_*     q[b,:] = K_ff(a_b) (V_b s_b)
- *     gpde_vo_residual_grad_vb_*  grad_a, grad_g as gpde_vo_residual_grad_* with w~_b = V_b gbar_r_b
- * Other arguments as for the shared-V versions.  rho: the fine residual comes from the rho-only route of gpde_vo_residual_*
- * (the kernel the plan picks for it), then one contraction kernel streams V_b once; the transposed application and the
- * gradient first form the FP64 rows V_b s_b in the workspace with one expansion kernel, then run the K_ff application of
- * gpde_vo_residual_T_* (strided-y marching kernel on pixel grids, generic matvec otherwise) or the gradient kernels.  Any
- * m >= 1.  FP32 I/O reads V, rho and s as floats and accumulates in FP64 (rho itself is held as floats).  flags: bit0 =
- * ignore the load vector f; bit1 (packed weights) returns GPDE_ERR_ARG.  workspace: >= gpde_vo_vb_workspace_bytes(plan, B,
- * m), 16-byte aligned (it holds rho [B,d] when the caller passes no rho output, or V_b s_b).  B = 0 is a no-op.  m <= 0,
- * v_stride != d*m, a NULL or misaligned workspace or a NULL operand return GPDE_ERR_ARG.  Every output is summed in a fixed
- * order: results are deterministic. */
-size_t gpde_vo_vb_workspace_bytes(const gpde_vo_plan *plan, int64_t B, int m);
-int gpde_vo_residual_vb_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
-                            const double *y, const double *g, int64_t g_stride, const double *V, int64_t v_stride,
-                            int m, double *r, double *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream);
-int gpde_vo_residual_vb_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
-                            const float *y, const float *g, int64_t g_stride, const float *V, int64_t v_stride,
-                            int m, float *r, float *rho, void *workspace, int flags, int64_t B, gpde_stream_t stream);
-int gpde_vo_residual_T_vb_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
-                              const double *V, int64_t v_stride, int m, const double *s, double *q, void *workspace,
-                              int64_t B, gpde_stream_t stream);
-int gpde_vo_residual_T_vb_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
-                              const float *V, int64_t v_stride, int m, const float *s, float *q, void *workspace,
-                              int64_t B, gpde_stream_t stream);
-int gpde_vo_residual_grad_vb_f64(const gpde_vo_plan *plan, const double *a, int64_t a_stride, int a_is_log,
-                                 const double *y, const double *g, int64_t g_stride, const double *V, int64_t v_stride,
-                                 int m, const double *gbar_r, double *grad_a, double *grad_g, void *workspace,
-                                 int64_t B, gpde_stream_t stream);
-int gpde_vo_residual_grad_vb_f32(const gpde_vo_plan *plan, const float *a, int64_t a_stride, int a_is_log,
-                                 const float *y, const float *g, int64_t g_stride, const float *V, int64_t v_stride,
-                                 int m, const float *gbar_r, float *grad_a, float *grad_g, void *workspace,
-                                 int64_t B, gpde_stream_t stream);
 
 /* ---- fine-mesh label solves: batched preconditioned CG (setup-time replacement of the per-sample FEniCS / spsolve calls
  * of physics/LinearElliptic.py:85-101, 120-133 in utils/data.py:96-99).  One iteration = one gpde_vo_residual_f64 call with

@@ -1,6 +1,6 @@
 """Times the residual family with one weighting matrix per sample (VoPlan.residual / residual_T / residual_grad with V
-[B,d,m] -> gpde_vo_residual_vb_*, gpde_vo_residual_T_vb_*, gpde_vo_residual_grad_vb_*, csrc/vo_vb.cuh) against the same
-quantities through torch.bmm on the same rho and V.
+[B,d,m] -> gpde_vo_residual_*, gpde_vo_residual_T_*, gpde_vo_residual_grad_* with v_stride = d*m, csrc/vo_vb.cuh)
+against the same quantities through torch.bmm on the same rho and V.
 
     python profiles/tools/time_vo_residual_vb.py --out DIR [--reps R] [--warmup W]
 

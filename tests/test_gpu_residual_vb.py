@@ -1,6 +1,7 @@
-"""The virtual-observable residual family with one weighting matrix per sample, V [B,d,m] (gpde_vo_residual_vb_*,
-gpde_vo_residual_T_vb_*, gpde_vo_residual_grad_vb_*, csrc/vo_vb.cuh): against oracle/vo_ref.py per sample with K and f
-from oracle/fem_p1.py, against the shared-V entry points, through VoResidualFn and through the ensemble API."""
+"""The virtual-observable residual family with one weighting matrix per sample, V [B,d,m] (gpde_vo_residual_*,
+gpde_vo_residual_T_*, gpde_vo_residual_grad_* with v_stride = d*m, csrc/vo_vb.cuh): against oracle/vo_ref.py per sample
+with K and f from oracle/fem_p1.py, against a shared V, through VoResidualFn and through the ensemble API; and the one
+workspace query of the family, for either layout."""
 import ctypes
 
 import numpy as np
@@ -224,7 +225,7 @@ def test_ensemble_without_weighting_matrices_raises(dev):
         ens.residual_gradients(torch.zeros(Y.shape[0], qe[0].m, dtype=torch.double, device=dev))
 
 
-def test_empty_batch(dev):
+def test_empty_batch_in_either_layout(dev):
     plan, ref = _case(16, 8, True, False, dev)
     x, y, g, V, s = (torch.tensor(t, device=dev) for t in _inputs(plan, ref, 2, 5, "NDP", seed=2))
     assert plan.residual(x[:0], y[:0], g[:0], V[:0]).shape == (0, 5)
@@ -232,12 +233,16 @@ def test_empty_batch(dev):
     ga, _ = plan.residual_grad(x[:0], y[:0], g[:0], V[:0], s[:0])
     assert ga.shape == (0, plan.n_inputs)
     lib = plan._lib
-    # B = 0 through the C ABI: no-op even with NULL operands
-    assert lib.gpde_vo_residual_vb_f64(plan.handle, None, 0, 1, None, None, 0, None, plan.d * 5, 5, None, None, None, 0, 0,
-                                       None) == 0
+    # B = 0 through the C ABI: no-op even with NULL operands, in either layout
+    for v_stride in (plan.d * 5, 0):
+        assert lib.gpde_vo_residual_f64(plan.handle, None, 0, 1, None, None, 0, None, v_stride, 5, None, None, None, 0, 0,
+                                        None) == 0
+        assert lib.gpde_vo_residual_T_f64(plan.handle, None, 0, 1, None, v_stride, 5, None, None, None, 0, None) == 0
+        assert lib.gpde_vo_residual_grad_f64(plan.handle, None, 0, 1, None, None, 0, None, v_stride, 5, None, None, None,
+                                             None, 0, None) == 0
 
 
-def test_bad_arguments(dev):
+def test_bad_arguments_through_v_stride(dev):
     from gpde_b200 import _lib
     plan, ref = _case(16, 8, True, False, dev)
     B, m = 3, 5
@@ -246,25 +251,28 @@ def test_bad_arguments(dev):
     r = torch.empty(B, m, dtype=torch.float64, device=dev)
     q = torch.empty(B, plan.d, dtype=torch.float64, device=dev)
     ga = torch.empty(B, plan.n_inputs, dtype=torch.float64, device=dev)
-    ws = torch.empty(int(lib.gpde_vo_vb_workspace_bytes(plan.handle, B, m)) + 64, dtype=torch.uint8, device=dev)
+    ws = torch.empty(int(lib.gpde_vo_workspace_bytes(plan.handle, B, m)) + 64, dtype=torch.uint8, device=dev)
     wsp, mis = P(ws), ctypes.c_void_p(ws.data_ptr() + 8)
     st = _lib.stream_of(dev)
-    res = lambda Vp, stride, w, rr=P(r), mm=m: lib.gpde_vo_residual_vb_f64(plan.handle, P(x), plan.n_inputs, 1, P(y), P(g),
-                                                                           plan.n_bc, Vp, stride, mm, rr, None, w, 0, B, st)
-    resT = lambda Vp, stride, w, qq=P(q): lib.gpde_vo_residual_T_vb_f64(plan.handle, P(x), plan.n_inputs, 1, Vp, stride, m,
-                                                                        P(s), qq, w, B, st)
-    grad = lambda Vp, stride, w, gg=P(s): lib.gpde_vo_residual_grad_vb_f64(plan.handle, P(x), plan.n_inputs, 1, P(y), P(g),
-                                                                           plan.n_bc, Vp, stride, m, gg, P(ga), None, w, B, st)
+    res = lambda Vp, stride, w, rr=P(r), mm=m, fl=0: lib.gpde_vo_residual_f64(plan.handle, P(x), plan.n_inputs, 1, P(y), P(g),
+                                                                              plan.n_bc, Vp, stride, mm, rr, None, w, fl, B, st)
+    resT = lambda Vp, stride, w, qq=P(q): lib.gpde_vo_residual_T_f64(plan.handle, P(x), plan.n_inputs, 1, Vp, stride, m,
+                                                                     P(s), qq, w, B, st)
+    grad = lambda Vp, stride, w, gg=P(s): lib.gpde_vo_residual_grad_f64(plan.handle, P(x), plan.n_inputs, 1, P(y), P(g),
+                                                                        plan.n_bc, Vp, stride, m, gg, P(ga), None, w, B, st)
     good = plan.d * m
     for call in (res, resT, grad):
         assert call(P(V), good, wsp) == 0
-        assert call(P(V), good + 1, wsp) == GPDE_ERR_ARG       # v_stride != d*m
-        assert call(P(V), 0, wsp) == GPDE_ERR_ARG              # no shared route here
+        assert call(P(V), good + 1, wsp) == GPDE_ERR_ARG       # v_stride neither 0 nor d*m
+        assert call(P(V), 1, wsp) == GPDE_ERR_ARG
+        assert call(P(V), -good, wsp) == GPDE_ERR_ARG
         assert call(P(V), good, mis) == GPDE_ERR_ARG           # misaligned workspace
         assert call(P(V), good, None) == GPDE_ERR_ARG          # no workspace
         assert call(None, good, wsp) == GPDE_ERR_ARG           # no V
     assert res(P(V), good, wsp, rr=None) == GPDE_ERR_ARG
     assert res(P(V), 0, wsp, mm=0) == GPDE_ERR_ARG
+    assert res(P(V), good, wsp, mm=0) == GPDE_ERR_ARG          # m = 0 (rho only) takes no V
+    assert res(P(V), good, wsp, fl=2) == GPDE_ERR_ARG          # packed weights are a shared-V layout
     assert resT(P(V), good, wsp, qq=None) == GPDE_ERR_ARG
     assert grad(P(V), good, wsp, gg=None) == GPDE_ERR_ARG
     torch.cuda.synchronize()
@@ -302,3 +310,51 @@ def test_repeated_calls_are_bitwise_identical(dev):
                 for _ in range(2)]
         assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
         assert torch.equal(outs[0][2][0], outs[1][2][0]) and torch.equal(outs[0][2][1], outs[1][2][1])
+
+
+@pytest.mark.parametrize("B", [1, 5, 300])
+@pytest.mark.parametrize("m", [1, 25, 32, 33, 100, 256])
+@pytest.mark.parametrize("per_sample", [False, True], ids=["shared", "per_sample"])
+@pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
+@pytest.mark.parametrize("mesh", MESHES, ids=["pixel", "cell"])
+def test_one_workspace_query_covers_the_family(mesh, dtype, per_sample, m, B, dev):
+    """gpde_vo_workspace_bytes(plan, B, m) is enough for residual, residual_T and residual_grad in either layout: each call
+    gets exactly that many bytes at the start of a larger buffer, must leave the sentinel bytes behind them as they were,
+    and must give what it gives with a generous workspace."""
+    from gpde_b200 import _lib
+    nx, ny, pixel = mesh
+    plan, _ = _case(nx, ny, pixel, not pixel, dev)
+    lib, P, st, sfx = plan._lib, (lambda t: _lib.ptr(t, dev)), _lib.stream_of(dev), _lib.suffix(dtype)
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(1000 * B + m)
+    R = lambda *shape: torch.randn(*shape, generator=gen, device=dev, dtype=torch.float64).to(dtype)
+    x, y, g, s = 0.6 * R(B, plan.n_inputs), R(B, plan.d), R(B, plan.n_bc), R(B, m)
+    V = R(B, plan.d, m) if per_sample else R(plan.d, m)
+    v_stride = plan.d * m if per_sample else 0
+    need = int(lib.gpde_vo_workspace_bytes(plan.handle, B, m))
+
+    def run(ws, after_each):
+        r, q = (torch.empty(B, n, dtype=dtype, device=dev) for n in (m, plan.d))
+        ga, gg = (torch.empty(B, n, dtype=dtype, device=dev) for n in (plan.n_inputs, plan.n_bc))
+        calls = [lambda: getattr(lib, "gpde_vo_residual_" + sfx)(plan.handle, P(x), plan.n_inputs, 1, P(y), P(g), plan.n_bc,
+                                                                 P(V), v_stride, m, P(r), None, P(ws), 0, B, st),
+                 lambda: getattr(lib, "gpde_vo_residual_T_" + sfx)(plan.handle, P(x), plan.n_inputs, 1, P(V), v_stride, m,
+                                                                   P(s), P(q), P(ws), B, st),
+                 lambda: getattr(lib, "gpde_vo_residual_grad_" + sfx)(plan.handle, P(x), plan.n_inputs, 1, P(y), P(g),
+                                                                      plan.n_bc, P(V), v_stride, m, P(s), P(ga), P(gg),
+                                                                      P(ws), B, st)]
+        for name, call in zip(("residual", "residual_T", "residual_grad"), calls):
+            assert call() == 0, name
+            after_each(name)
+        return r, q, ga, gg
+
+    buf = torch.full((need + (1 << 16),), 0xA5, dtype=torch.uint8, device=dev)
+
+    def tail_intact(name):
+        torch.cuda.synchronize()
+        assert bool((buf[need:] == 0xA5).all()), "%s wrote past gpde_vo_workspace_bytes = %d" % (name, need)
+
+    exact = run(buf[:need], tail_intact)
+    generous = run(torch.empty(2 * need + (1 << 20), dtype=torch.uint8, device=dev), lambda name: None)
+    for got, want in zip(exact, generous):
+        assert torch.equal(got, want)

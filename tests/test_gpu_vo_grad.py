@@ -81,17 +81,18 @@ def _per_sample_rel(got, want):
 
 
 def _grad_kernels(fn):
-    """Names of the vo_grad_* kernels fn launches (torch.profiler)."""
+    """Names of the vo_grad_* kernels fn launches (torch.profiler).  fn launches at least the expansion kernel, so a capture
+    without any of the project's kernels has lost its device records (in a long test process the profiler sometimes returns
+    a short capture empty) and is taken again."""
     from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    names = set()
-    for e in prof.events():
-        for k in ("vo_grad_grid_kernel", "vo_grad_cells_kernel", "vo_grad_g_kernel"):
-            if k in e.name:
-                names.add(k)
-    return names
+    for _ in range(3):
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            fn()
+            torch.cuda.synchronize()
+        seen = [e.name for e in prof.events()]
+        if any("gpde::" in s for s in seen):
+            break
+    return {k for k in ("vo_grad_grid_kernel", "vo_grad_cells_kernel", "vo_grad_g_kernel") if any(k in s for s in seen)}
 
 
 def _call(plan, inp, y, g, V, gbar, dev, a_is_log, dtype=torch.float64, **kw):
@@ -213,7 +214,7 @@ def test_fp32_io_matches_fp64_on_rounded_inputs(pixel, m, dev):
             assert _per_sample_rel(lo, hi) < 2e-6
 
 
-def test_edge_cases(dev):
+def test_edge_cases_with_one_workspace_query(dev):
     from gpde_b200 import _lib
     plan, ref = _problem(16, 16, "right", True, dev)
     x, y, g, V, gbar = (t.to(dev) for t in _inputs(plan, ref, 8, 25, "NDP", seed=9))
@@ -250,7 +251,7 @@ def test_edge_cases(dev):
             plan.residual_grad(*bad_args, V, gbar)
     # argument errors: GpdeLibraryError, no device fault
     lib = _lib.load()
-    ws = torch.empty(int(lib.gpde_vo_grad_workspace_bytes(plan.handle, 8, 25)) + 64, dtype=torch.uint8, device=dev)
+    ws = torch.empty(int(lib.gpde_vo_workspace_bytes(plan.handle, 8, 25)) + 64, dtype=torch.uint8, device=dev)
     P = lambda t: _lib.ptr(t, dev)
     st = _lib.stream_of(dev)
     Vc, gbc = V.contiguous(), gbar.contiguous()
@@ -260,11 +261,10 @@ def test_edge_cases(dev):
            dict(ws=ctypes.c_void_p(ws.data_ptr() + 8)), dict(ws=None)]
     for change in bad:
         k = dict(base, **change)
-        rc = lib.gpde_vo_residual_grad_f64(plan.handle, k["a"], k["a_stride"], 1, P(y), P(g), plan.n_bc, k["V"], k["m"],
+        rc = lib.gpde_vo_residual_grad_f64(plan.handle, k["a"], k["a_stride"], 1, P(y), P(g), plan.n_bc, k["V"], 0, k["m"],
                                            k["gbar"], P(out_a), None, k["ws"], 8, st)
         with pytest.raises(_lib.GpdeLibraryError):
             _lib.check(rc, "gpde_vo_residual_grad_f64")
-    assert int(lib.gpde_vo_grad_workspace_bytes(plan.handle, 8, 0)) == 0
     torch.cuda.synchronize()
     assert torch.equal(plan.residual_grad(x, y, g, V, gbar)[0], full_a)
 
