@@ -595,8 +595,11 @@ static int launch_grid2(const gpde_vo_plan *pl, const TA *a, long long a_stride,
     }
     const unsigned grid = blocks * (unsigned)csize;
     // the residual kernel is launched as a programmatic dependent of the packing kernel (its prologue and first
-    // a / y stages overlap the packing)
-    const bool pdl = !rho && !prepacked && csize == 1;
+    // a / y stages overlap the packing); with prepacked weights (the packing, if any, was a call of its own) as a
+    // dependent of whatever the stream ran before, which it waits for before its first global read: only the launch
+    // overlaps
+    const bool pdl = !rho && csize == 1;
+    G.wait_first = prepacked ? 1 : 0;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3(grid);

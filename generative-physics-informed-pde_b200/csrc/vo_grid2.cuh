@@ -53,6 +53,7 @@ struct Grid2Dev {
     int stage_bytes, v_row_bytes;   // one a/y stage (all samples of the CTA); one packed V row
     int nvs;                        // V stages in the ring (2 or 3)
     int spc;                        // samples a CTA takes (<= 8 groups): group i gets [i spc / groups, (i + 1) spc / groups)
+    int wait_first;                 // programmatic dependent of a kernel this one does not know: griddepcontrol.wait first
 };
 
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -163,8 +164,10 @@ __global__ void vo_grid2_pack_kernel(Grid2Dev G, const TV *__restrict__ V, int m
     // programmatic dependent launch: the residual kernel may start its prologue (shared-memory setup, first a / y
     // stages) now; it waits for this grid (griddepcontrol.wait) before it touches the packed rows
     asm volatile("griddepcontrol.launch_dependents;");
-    // one warp per (node row t, strip q): it writes the strip's NT tiles (128 doubles each, 4 per lane, all loads
-    // independent), the extra column and -- from the values it has just seen -- the strip's mask word
+    // one warp per (node row t, strip q): it writes the strip's NT tiles (128 doubles each, 4 per lane), the extra column
+    // and -- from the values it has just seen -- the strip's mask word.  All loads of a warp are issued before its first
+    // store (NT <= 4 tiles unrolled): the launch sits on the critical path of a residual call, and a loop over the tiles
+    // with its stores in between waits out one load round trip per tile.
     const int per_strip = 4 * NT * 32, per_row = G.v_row_bytes / 8, main = G.nstrips * per_strip;
     const int data = main + (NX ? G.nstrips * 16 : 0);     // doubles of a row before the masks
     const int lane = threadIdx.x & 31;
@@ -175,28 +178,34 @@ __global__ void vo_grid2_pack_kernel(Grid2Dev G, const TV *__restrict__ V, int m
         unsigned bits = 0;
         if (q < G.nstrips) {
             const TV *Vt = V + (long long)t * G.ncol * m;
-            for (int tt = 0; tt < NT; ++tt) {
-                double v[4];
+            double v[4][4], vx = 0.0;
+#pragma unroll
+            for (int tt = 0; tt < 4; ++tt)
 #pragma unroll
                 for (int it = 0; it < 4; ++it) {
                     const int e = it * 32 + lane;                       // [half ph][lane ln][h]
                     const int h = e & 1, ln = (e >> 1) & 31, ph = e >> 6;
                     const int c = 16 * q + 4 * (ln & 3) + 2 * ph + h, col = 8 * tt + (ln >> 2);
-                    v[it] = (c < G.ncol && col < m) ? (double)Vt[(long long)c * m + col] : 0.0;
+                    v[tt][it] = (tt < NT && c < G.ncol && col < m) ? (double)Vt[(long long)c * m + col] : 0.0;
                 }
-                bool nz = false;
-#pragma unroll
-                for (int it = 0; it < 4; ++it) {
-                    row[q * per_strip + tt * 128 + it * 32 + lane] = v[it];
-                    nz |= v[it] != 0.0;
-                }
-                if (__any_sync(0xffffffffu, nz)) bits |= 1u << tt;
-            }
             if (NX) {
                 const int c = 16 * q + lane, col = 8 * NT;               // [k][j] = column 16 q + 4 k + j: lanes 0..15
-                const double v = (lane < 16 && c < G.ncol && col < m) ? (double)Vt[(long long)c * m + col] : 0.0;
-                if (lane < 16) row[main + q * 16 + lane] = v;
-                if (__any_sync(0xffffffffu, v != 0.0)) bits |= 0x80u;
+                vx = (lane < 16 && c < G.ncol && col < m) ? (double)Vt[(long long)c * m + col] : 0.0;
+            }
+#pragma unroll
+            for (int tt = 0; tt < 4; ++tt)
+                if (tt < NT) {
+                    bool nz = false;
+#pragma unroll
+                    for (int it = 0; it < 4; ++it) {
+                        row[q * per_strip + tt * 128 + it * 32 + lane] = v[tt][it];
+                        nz |= v[tt][it] != 0.0;
+                    }
+                    if (__any_sync(0xffffffffu, nz)) bits |= 1u << tt;
+                }
+            if (NX) {
+                if (lane < 16) row[main + q * 16 + lane] = vx;
+                if (__any_sync(0xffffffffu, vx != 0.0)) bits |= 0x80u;
             }
         }
         if (lane == 0) reinterpret_cast<unsigned *>(row + data)[q] = bits;
@@ -339,6 +348,10 @@ vo_grid2_kernel(Grid2Dev G, const TA *__restrict__ a, long long a_stride, int a_
     const bool is_left = c0 == 0, is_right = c0 == nx - 4;
     const TY *yb = y + b * y_stride;
     const TA *gp = (!WT && g && (is_left || is_right)) ? g + b * g_stride + (is_right ? 1 : 0) : nullptr;
+    // Launched as a programmatic dependent of whatever the stream ran before (prepacked weights): nothing from global
+    // memory is read before that grid has completed; only the launch overlaps it.  (After the packing kernel of the same
+    // call, its prerequisites completed before it started, and only the packed rows wait for it: see below.)
+    if (G.wait_first) asm volatile("griddepcontrol.wait;" ::: "memory");
     // node row 0 of this lane comes straight from global memory: requested here, consumed after the set-up below (one
     // exposed DRAM round trip less per CTA: in the profile of a one-wave launch 3.5 % of the warp samples sat behind it)
     double r0[4] = {0.0, 0.0, 0.0, 0.0}, r0l = 0.0, r0r = 0.0, r0g = 0.0;
